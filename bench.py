@@ -29,6 +29,10 @@ way (their lines are committed under profiles/).
   parity    asserted inside this run: e2e text == host-formatted records of the
             resident pass == CLI output file, and its head == the CPU checker's output
 
+`--dump-outputs DIR` writes, after the timed steps, the output text of the last timed e2e
+step (rank 0's reads) for a fixed, seeded sample of reads, so that two builds can be compared
+output for output on identical inputs (see dump_outputs).
+
 Multi-GPU (torchrun, one rank per GPU): reads sharded, CTR replicated, no collective on the
 data path; weak scaling.  `single_process` additionally times ONE utb_searcher over all
 N devices on one FASTA of N x the reads (one upload + NVLink fan-out of the tables, one
@@ -76,6 +80,7 @@ CONFIGS = {
 SEED = 20260101
 ALL_CPUS = os.sched_getaffinity(0)
 CHUNK_BYTES = 1_900_000_000          # raw bytes of one resident batch (positions x 2 strands must fit 32 bits)
+DUMP_READS = 1 << 15                 # reads whose output lines --dump-outputs writes (< 64 MB at any label length in CONFIGS)
 
 
 def log(*a):
@@ -329,6 +334,44 @@ def cli_run(exe, ctr_path, fasta, out, threads):
     return dt, (float(m.group(1)) if m else None)
 
 
+def search_mem_unread(capi, searcher, ptr, n):
+    """Searcher.search_mem(copy=False) that also returns where the text is: it stays in the searcher's arena until the
+    next search, so it can be copied once the clock has stopped.  -> (rc, text address, text length, stats)."""
+    import ctypes as C
+    st, ex = capi.Stats(), C.c_int()
+    out, out_len = C.c_void_p(), C.c_size_t()
+    rc = capi.lib().utb_search_mem(searcher.h, ptr, n, 1, C.byref(out), C.byref(out_len), C.byref(st), C.byref(ex))
+    return rc, out.value, out_len.value, st.as_dict()
+
+
+def dump_outputs(d, text, first_read, n_reads):
+    """The output lines of DUMP_READS reads drawn with a fixed seed from reads [first_read, first_read + n_reads) (all
+    of them when there are fewer), as d/read_index.npy (float64, the sampled read numbers, ascending),
+    d/line_offsets.npy (float64, n + 1: read i's line is line_bytes[off[i]:off[i + 1]] without its newline, empty when
+    the read has no line) and d/line_bytes.npy (float32, the bytes of those lines).  Reads are named r%09u after their
+    number and their lines come in input order."""
+    t = np.frombuffer(text, dtype=np.uint8)
+    ends = np.flatnonzero(t == 10)
+    starts = np.concatenate([[0], ends + 1])[:ends.size].astype(np.int64)
+    num = np.zeros(starts.size, dtype=np.int64)
+    for k in range(1, 10):
+        num = num * 10 + t[starts + k].astype(np.int64) - 48
+    rng = np.random.default_rng(SEED)
+    reads = first_read + np.sort(rng.choice(n_reads, min(n_reads, DUMP_READS), replace=False)).astype(np.int64)
+    pos = np.minimum(np.searchsorted(num, reads), max(num.size - 1, 0))
+    has = num[pos] == reads if num.size else np.zeros(reads.size, dtype=bool)
+    lens = np.zeros(reads.size, dtype=np.int64)
+    lens[has] = ends[pos[has]] - starts[pos[has]]
+    off = np.concatenate([[0], np.cumsum(lens)]).astype(np.int64)
+    line_bytes = t[np.repeat(starts[pos[has]] - off[:-1][has], lens[has]) + np.arange(off[-1])].astype(np.float32)
+    assert line_bytes.nbytes + 16 * (reads.size + 1) <= 64 << 20, "dump over 64 MB"
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "read_index.npy"), reads.astype(np.float64))
+    np.save(os.path.join(d, "line_offsets.npy"), off.astype(np.float64))
+    np.save(os.path.join(d, "line_bytes.npy"), line_bytes)
+    log(f"dumped the lines of {int(has.sum())} of {reads.size} sampled reads ({line_bytes.size} bytes) to {d}")
+
+
 def main():
     global _REAL_STDOUT
     sys.stdout.flush()
@@ -343,7 +386,10 @@ def main():
     ap.add_argument("--reads", type=int, default=0, help="reads per GPU (default: the config's)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the e2e_file / e2e_cli / e2e_pageable / single_process legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed e2e step there (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     if args.reads:
         cfg["reads"] = args.reads
@@ -454,14 +500,20 @@ def main():
     out_len = len(out_text) if rank == 0 else out_text
     barrier()
     t0 = time.time()
-    e2e_stats = []
-    for _ in range(args.steps):
-        rc_, ex, nbytes, st = searcher.search_mem(None, do_rc=True, ptr=ptr, n=reads_np.size, copy=False)
+    e2e_stats, last_text = [], None
+    for i in range(args.steps):
+        if args.dump_outputs and rank == 0 and i == args.steps - 1:
+            rc_, last_text, nbytes, st = search_mem_unread(capi, searcher, ptr, reads_np.size)
+        else:
+            rc_, ex, nbytes, st = searcher.search_mem(None, do_rc=True, ptr=ptr, n=reads_np.size, copy=False)
         assert rc_ == 0 and nbytes == out_len
         e2e_stats.append(st)
     own_e2e_s = time.time() - t0                                   # this rank alone; the figure uses the time up to the barrier, i.e. the slowest rank
     barrier()
     e2e_s = time.time() - t0
+    if last_text is not None:
+        import ctypes
+        dump_outputs(args.dump_outputs, ctypes.string_at(last_text, nbytes) if nbytes else b"", lo_read, n_reads)
     clocks = sampler.summary()
     log(f"rank {rank}: e2e {own_e2e_s * 1e3 / args.steps:.1f} ms per step on its own ({ncpu} cores visible, {host_threads} host threads)")
 

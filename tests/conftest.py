@@ -1,13 +1,46 @@
+import hashlib
 import json
 import os
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 GOLD = os.path.join(ROOT, "tests", "golden")
 REFDIR = os.path.join(ROOT, "oracle", "_ref")
+REFERENCE_RUNS = os.path.join(GOLD, "reference_runs.json")
+
+
+def _digest(data, text):
+    e = {"bytes": len(data), "sha256": hashlib.sha256(data).hexdigest()}
+    if text:
+        lines = data.split(b"\n")
+        idx = np.random.default_rng(len(lines)).choice(len(lines), min(40, len(lines)), replace=False)
+        e["lines"] = len(lines)
+        e["sample"] = {str(i): lines[i].decode("latin-1") for i in sorted(idx.tolist())}
+    return e
+
+
+def check_reference_run(name, got, text=True):
+    """`got` == the bytes the reference wrote for case `name`.  tests/golden/reference_runs.json keeps their size and
+    sha256 and, for text, the line count and a seeded sample of lines, compared first so that a mismatch names a line.
+    UTB_RECORD_REFERENCE_RUNS=1 writes the entry instead of comparing (see "_about" in that file)."""
+    runs = json.load(open(REFERENCE_RUNS)) if os.path.exists(REFERENCE_RUNS) else {}
+    if os.environ.get("UTB_RECORD_REFERENCE_RUNS") == "1":
+        runs[name] = _digest(got, text)
+        with open(REFERENCE_RUNS, "w") as f:
+            json.dump(runs, f, indent=1, sort_keys=True)
+        return
+    assert name in runs, f"no recorded reference output for {name}"
+    want = runs[name]
+    if text:
+        lines = got.split(b"\n")
+        assert len(lines) == want["lines"], name
+        for i, line in want["sample"].items():
+            assert lines[int(i)].decode("latin-1") == line, (name, int(i))
+    assert (len(got), hashlib.sha256(got).hexdigest()) == (want["bytes"], want["sha256"]), name
 
 
 def pytest_configure(config):

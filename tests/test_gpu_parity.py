@@ -8,7 +8,7 @@ import pytest
 
 import conftest  # noqa: F401  (puts the repo root on sys.path)
 from oracle import oracle_api
-from conftest import BAD_CASES, CASES, ROOT, gold, read_fasta
+from conftest import BAD_CASES, CASES, ROOT, check_reference_run, gold, read_fasta
 
 pytestmark = pytest.mark.gpu
 
@@ -314,13 +314,15 @@ def test_cli_sieve_kernel_variants_agree(ctrs, tmp_path, variant):
         assert open(o, "rb").read() == open(gold(out), "rb").read(), (variant, reads)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "utree-build_gg")), reason="oracle/_ref not built")
 @pytest.mark.parametrize("complevel", [0, 2])
 def test_synthetic_ctr_equals_reference_built_tree(built, tmp_path, complevel):
     """The GPU CTR synthesiser (bench input generator) against the REAL builder:
     same universe through utree-build_gg + utree-compress and through
-    uts_build_ctr must classify identically (reference search on both trees),
-    and the product must match the reference on the synthesised tree."""
+    uts_build_ctr must classify identically, and the product must write on the
+    synthesised tree what the reference search wrote (reference_runs.json; live
+    when oracle/_ref is built).  The built tree comes from the product's builder
+    and compressor, byte-identical to the reference's, and from the reference
+    binaries too when they are there."""
     from utree_b200 import build, capi
     from tools import synthgpu
     build.build_synth()
@@ -331,26 +333,37 @@ def test_synthetic_ctr_equals_reference_built_tree(built, tmp_path, complevel):
         for g in range(uni.n_genomes):
             f.write(b">gen%d\n" % g + uni.genome_ascii(g) + b"\n")
             m.write(b"gen%d\t" % g + uni.genome_tax(g) + b"\n")
-    ubt, ctr_ref, ctr_syn = str(tmp_path / "t.ubt"), str(tmp_path / "ref.ctr"), str(tmp_path / "syn.ctr")
-    subprocess.run([os.path.join(ref, "utree-build_gg"), fa, mp, ubt, "1", str(complevel)], check=True, stdout=subprocess.DEVNULL)
-    subprocess.run([os.path.join(ref, "utree-compress"), ubt, ctr_ref], check=True, stdout=subprocess.DEVNULL)
+    ubt, ctr_built, ctr_syn = str(tmp_path / "t.ubt"), str(tmp_path / "built.ctr"), str(tmp_path / "syn.ctr")
+    rc, _, _ = capi.build_ubt(fa, mp, ubt, complevel=complevel, gg=True, ix_bytes=2)
+    assert rc == 0, capi.lib().utb_last_error()
+    capi.compress_ubt(ubt, ctr_built)
+    trees = [ctr_built]
+    if os.path.exists(os.path.join(ref, "utree-build_gg")):
+        ctr_ref, ubt_ref = str(tmp_path / "ref.ctr"), str(tmp_path / "ref.ubt")
+        subprocess.run([os.path.join(ref, "utree-build_gg"), fa, mp, ubt_ref, "1", str(complevel)], check=True, stdout=subprocess.DEVNULL)
+        subprocess.run([os.path.join(ref, "utree-compress"), ubt_ref, ctr_ref], check=True, stdout=subprocess.DEVNULL)
+        assert open(ctr_ref, "rb").read() == open(ctr_built, "rb").read()
+        trees.append(ctr_ref)
     n, nl = uni.build_ctr(ctr_syn, complevel=complevel)
-    assert n == np.frombuffer(open(ctr_ref, "rb").read(32), dtype="<u8")[3]
+    assert n == np.frombuffer(open(ctr_built, "rb").read(32), dtype="<u8")[3]
     reads = str(tmp_path / "r.fa")
     uni.make_reads(20000, read_len=150).tofile(reads)
     outs = []
-    for c in (ctr_ref, ctr_syn):
-        o = c + ".out"
-        subprocess.run([os.path.join(ref, "utree-search_gg"), c, reads, o, "1", "RC"], check=True, stdout=subprocess.DEVNULL)
-        outs.append(open(o, "rb").read())
-    assert outs[0] == outs[1] and outs[0].count(b"\n") > 15000
-    ctr = capi.Ctr(ctr_syn)
-    s = capi.Searcher(ctr, devices=(0,), host_threads=2)
-    try:
-        code, _, text, st = s.search_mem(open(reads, "rb").read(), do_rc=True)
-        assert code == 0 and text == outs[1]
-    finally:
-        s.destroy(); ctr.close()
+    for c in trees + [ctr_syn]:
+        ctr = capi.Ctr(c)
+        s = capi.Searcher(ctr, devices=(0,), host_threads=2)
+        try:
+            code, _, text, st = s.search_mem(open(reads, "rb").read(), do_rc=True)
+            assert code == 0
+            outs.append(text)
+        finally:
+            s.destroy(); ctr.close()
+        if c != ctr_syn and os.path.exists(os.path.join(ref, "utree-search_gg")):
+            o = c + ".out"
+            subprocess.run([os.path.join(ref, "utree-search_gg"), c, reads, o, "1", "RC"], check=True, stdout=subprocess.DEVNULL)
+            outs.append(open(o, "rb").read())
+    assert all(o == outs[-1] for o in outs) and outs[-1].count(b"\n") > 15000
+    check_reference_run(f"synthetic_ctr_complevel{complevel}", outs[-1])
 
 
 def _lookup_probe_words(words, rng):
@@ -695,7 +708,8 @@ def test_shallow_cli_binary(ctrs, tmp_path):
 
 # ---- utree-build_gg on the GPU (SURVEY 8f-4) ---------------------------------------------------------------------
 BUILD_CASES = [
-    # name, make_genomes kwargs, complevel, ix_bytes, golden .ubt made by the reference builder (scripts/make_golden.py)
+    # name, make_genomes kwargs, complevel, ix_bytes, golden .ubt made by the reference builder (scripts/make_golden.py);
+    # None: compared with the digests of the reference's output in reference_runs.json
     ("toyA", dict(seed=11, n_phyla=2, n_genera=2, n_species=2, n_strains=2, length=4000), 0, 2, "toyA.ubt"),
     ("toyB", dict(seed=21, n_phyla=3, n_genera=2, n_species=2, n_strains=2, length=6000, quirky_tax=True), 1, 4, "toyB_u32.ubt"),
     ("mid2", dict(seed=5, n_phyla=3, n_genera=3, n_species=3, n_strains=2, length=30000), 2, 2, None),
@@ -707,7 +721,8 @@ BUILD_CASES = [
 def test_gpu_builder_is_byte_identical_to_the_reference_builder(built, tmp_path, name, kw, complevel, ix_bytes, golden):
     """FASTA + map -> .ubt on the GPU: the bytes the reference's serial builder writes (words, label ids in its
     order of registration incl. superseded derived labels, counts, .gg.log), against the committed .ubt fixtures
-    and, where oracle/_ref is present, against the reference builder run live on the same input."""
+    or the digests of the reference's files and stdout, and, where oracle/_ref is present, against the reference
+    builder run live on the same input."""
     from tools import synth
     from utree_b200 import capi
     genomes = synth.make_genomes(**kw)
@@ -719,6 +734,12 @@ def test_gpu_builder_is_byte_identical_to_the_reference_builder(built, tmp_path,
     assert st["records"] == int.from_bytes(got[24:32], "little") > 0
     if golden:
         assert got == open(gold(golden), "rb").read()
+    else:
+        check_reference_run(f"build_{name}.ubt", got, text=False)
+        check_reference_run(f"build_{name}.ubt.gg.log", open(out + ".gg.log", "rb").read())
+        p = subprocess.run([os.path.join(ROOT, "bin", "utree-build_gg"), fa, mp, out + "2", "1", str(complevel)], capture_output=True)
+        assert p.returncode == 0 and open(out + "2", "rb").read() == got
+        check_reference_run(f"build_{name}.stdout", p.stdout)
     ref = os.path.join(ROOT, "oracle", "_ref", "utree-build_gg" + ("_u32" if ix_bytes == 4 else ""))
     if os.path.exists(ref):
         rout = str(tmp_path / "ref.ubt")
@@ -731,5 +752,3 @@ def test_gpu_builder_is_byte_identical_to_the_reference_builder(built, tmp_path,
             p = subprocess.run([os.path.join(ROOT, "bin", "utree-build_gg"), fa, mp, out + "2", "1", str(complevel)], capture_output=True, text=True, env=env)
             assert p.returncode == 0 and open(out + "2", "rb").read() == got
             assert p.stdout == q.stdout
-    else:
-        assert golden, "neither a golden .ubt nor oracle/_ref to compare with"

@@ -1,8 +1,10 @@
 """Parity at the scales BASELINE.json names, against the UNMODIFIED reference
-binary (oracle/_ref, threads=1 = input order) on the GPU box: the L2-scale CTR,
-the L4 CTR, a uint32_t-label CTR with > 65,536 labels at complevel 0, and long /
-whole-genome queries up to the 16,777,214-base limit.  Inputs come from the GPU
-synthesiser (itself checked against the real builder in test_gpu_parity.py)."""
+binary (threads=1 = input order): the L2-scale CTR, the L4 CTR, a uint32_t-label
+CTR with > 65,536 labels at complevel 0, and long / whole-genome queries up to the
+16,777,214-base limit.  Inputs come from the seeded GPU synthesiser (itself checked
+against the real builder in test_gpu_parity.py); what the reference wrote for them
+is kept in tests/golden/reference_runs.json, and the reference also runs live when
+oracle/_ref is built."""
 import os
 import subprocess
 import sys
@@ -11,15 +13,17 @@ import time
 import numpy as np
 import pytest
 
-from conftest import ROOT
+from conftest import ROOT, check_reference_run
 
 pytestmark = pytest.mark.gpu
 REF = os.path.join(ROOT, "oracle", "_ref")
-need_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "utree-search_gg")), reason="oracle/_ref not built")
 
 
 def _ref_search(ctr, fasta, out, u32=False):
+    """The reference binary's output, or None when oracle/_ref is not built."""
     exe = os.path.join(REF, "utree-search_gg" + ("_u32" if u32 else ""))
+    if not os.path.exists(exe):
+        return None
     p = subprocess.run([exe, ctr, fasta, out, "1", "RC"], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
     assert p.returncode == 0, p.stderr[-500:]
     return open(out, "rb").read()
@@ -46,7 +50,6 @@ def bench_mod(built):
     return bench
 
 
-@need_ref
 @pytest.mark.parametrize("config,n_reads", [("l2s", 150_000), ("l4", 300_000)])
 def test_l2_scale_and_l4_match_reference(bench_mod, tmp_path, config, n_reads):
     cfg = dict(bench_mod.CONFIGS[config])
@@ -55,33 +58,36 @@ def test_l2_scale_and_l4_match_reference(bench_mod, tmp_path, config, n_reads):
     reads, _ = bench_mod.make_reads(cfg, 60_000_000, n_reads, 0)          # a window of the read stream the bench never uses
     fa = str(tmp_path / "r.fa")
     reads.tofile(fa)
-    want = _ref_search(ctr_path, fa, str(tmp_path / "ref.out"))
     got, st = _ours(ctr_path, reads.tobytes())
-    assert got == want
-    assert want.count(b"\n") > 0.9 * n_reads * (0.5 if config == "l4" else 1) * 0.5
+    check_reference_run(f"scale_{config}_{n_reads}", got)
+    want = _ref_search(ctr_path, fa, str(tmp_path / "ref.out"))
+    assert want is None or got == want
+    assert got.count(b"\n") > 0.9 * n_reads * (0.5 if config == "l4" else 1) * 0.5
     assert st["lookups"] > 200 * n_reads
 
 
-@need_ref
 def test_l2_scale_two_million_reads_every_batch_size(bench_mod, tmp_path):
     """2 M reads against the L2-scale tree: full-size 128 MiB batches (the shape the bench's e2e leg runs) and the
     ramp batches at both ends.  The reference runs with all host threads, so its lines come in any order
-    (SURVEY 0 #3): the two outputs must hold the same lines, ours in input order."""
+    (SURVEY 0 #3): the two outputs must hold the same lines, ours in input order.  The recorded output is those
+    lines in input order."""
     cfg = dict(bench_mod.CONFIGS["l2s"])
     ctr_path, _ = bench_mod.ensure_ctr("l2s", cfg, 0)
     n_reads = 2_000_000
     reads, _ = bench_mod.make_reads(cfg, 70_000_000, n_reads, 0)
     fa = str(tmp_path / "r.fa")
-    reads.tofile(fa)
-    exe = os.path.join(REF, "utree-search_gg")
-    p = subprocess.run([exe, ctr_path, fa, str(tmp_path / "ref.out"), str(os.cpu_count() or 4), "RC"],
-                       stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
-    assert p.returncode == 0, p.stderr[-500:]
-    want = open(str(tmp_path / "ref.out"), "rb").read().split(b"\n")
     got, st = _ours(ctr_path, reads.tobytes())
     assert st["batches"] >= 4 and st["reads"] == n_reads
+    check_reference_run("scale_l2s_2M_every_batch_size", got)
     lines = got.split(b"\n")
-    assert sorted(lines) == sorted(want)
+    exe = os.path.join(REF, "utree-search_gg")
+    if os.path.exists(exe):
+        reads.tofile(fa)
+        p = subprocess.run([exe, ctr_path, fa, str(tmp_path / "ref.out"), str(os.cpu_count() or 4), "RC"],
+                           stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
+        assert p.returncode == 0, p.stderr[-500:]
+        want = open(str(tmp_path / "ref.out"), "rb").read().split(b"\n")
+        assert sorted(lines) == sorted(want)
     names = [ln.split(b"\t", 1)[0] for ln in lines if ln]
     assert names == sorted(names) and len(names) > 0.9 * n_reads      # names are r%09u: input order = sorted
 
@@ -106,7 +112,6 @@ def test_two_physical_gpus_one_searcher(bench_mod, tmp_path):
         s.destroy(); ctr.close()
 
 
-@need_ref
 def test_uint32_labels_over_64k_match_reference(bench_mod, tmp_path):
     """IXTYPE=uint32_t (SZ=9), complevel 0, 73,260 labels, 250 bp reads."""
     from tools import synthgpu
@@ -118,15 +123,15 @@ def test_uint32_labels_over_64k_match_reference(bench_mod, tmp_path):
         reads = uni.make_reads(100_000, read_len=250, read_seed=5)
         fa = str(tmp_path / "r.fa")
         reads.tofile(fa)
-        want = _ref_search(ctr_path, fa, str(tmp_path / "ref.out"), u32=True)
         got, st = _ours(ctr_path, reads.tobytes())
-        assert got == want
+        check_reference_run("scale_u32_100k", got)
+        want = _ref_search(ctr_path, fa, str(tmp_path / "ref.out"), u32=True)
+        assert want is None or got == want
         assert st["hits"] > 10 * 100_000                              # dense tree: most k-mers of a read hit
     finally:
         os.remove(ctr_path)
 
 
-@need_ref
 def test_long_and_whole_genome_queries_match_reference(bench_mod, tmp_path):
     """10 kb - 1 Mb reads, whole genomes, and one query at the 16,777,214-base limit vs the L2-scale CTR."""
     from tools import synthgpu
@@ -152,13 +157,15 @@ def test_long_and_whole_genome_queries_match_reference(bench_mod, tmp_path):
     fasta = b"".join(b">" + n + b"\n" + s + b"\n" for n, s in recs)
     fa = str(tmp_path / "long.fa")
     open(fa, "wb").write(fasta)
+    got, st = _ours(ctr_path, fasta)
+    check_reference_run("scale_long_queries", got)
+    assert got.count(b"\n") == len(recs)
     t = time.time()
     want = _ref_search(ctr_path, fa, str(tmp_path / "ref.out"))
-    t_ref = time.time() - t
-    got, st = _ours(ctr_path, fasta)
-    assert got == want
-    assert want.count(b"\n") == len(recs)
-    print(f"long queries: {sum(len(s) for _, s in recs) / 1e6:.1f} Mb, reference {t_ref:.1f} s (incl. load), ours {st['seconds_total']:.2f} s")
+    assert want is None or got == want
+    if want is not None:
+        print(f"long queries: {sum(len(s) for _, s in recs) / 1e6:.1f} Mb, reference {time.time() - t:.1f} s (incl. load), "
+              f"ours {st['seconds_total']:.2f} s")
 
 
 def test_tree_with_more_than_2_32_records(bench_mod):
