@@ -2040,6 +2040,7 @@ extern "C" int utb_db_upload(const utb_ctr *ctr, int device, utb_db **out) {
     utb_db *db = (utb_db *)calloc(1, sizeof(utb_db));
     if (!db) { utb_set_error("out of memory"); return UTB_ERR_NOMEM; }
     db->device = device;
+    db->ema_hit_rate = -1.0;                                       // no batch seen yet: the first one sets it
     rc = db_upload_impl(ctr, device, db);
     if (rc) { utb_db_free(db); return rc; }                        // device buffers allocated so far are released
     *out = db;
@@ -2126,12 +2127,13 @@ static int db_build_tables(utb_db *db, size_t nb_binix, size_t nb_recs) {
         const char *lk = getenv("UTB_LOOKUP");                      // "exact" forces the reference probe sequence
         db->use_table = db->regular && !(lk && !strcmp(lk, "exact"));
     }
+    // sector hash table at load <= 0.5 (4 entries per sector, 3 with uint32_t labels); grown if a record cannot be placed within KT_MAXD sectors
+    const uint64_t n = db->d.num_nodes;
+    const uint32_t wide = db->d.ix_bytes == 4;
+    uint64_t sectors = wide ? n / 3 * 2 + 1 : n / 2 + 1;
+    if (sectors < KT_MIN_SECTORS) sectors = KT_MIN_SECTORS;
+    uint32_t table_failed = 0;                                      // records the table could not place at its largest size
     if (db->use_table) {
-        const uint64_t n = db->d.num_nodes;
-        // sector hash table at load <= 0.5 (4 entries per sector, 3 with uint32_t labels); grown if a record cannot be placed within KT_MAXD sectors
-        const uint32_t wide = db->d.ix_bytes == 4;
-        uint64_t sectors = wide ? n / 3 * 2 + 1 : n / 2 + 1;
-        if (sectors < KT_MIN_SECTORS) sectors = KT_MIN_SECTORS;
         uint32_t *d_ovf;
         CK(cudaMalloc(&d_ovf, 4));
         for (int attempt = 0;; ++attempt) {
@@ -2157,10 +2159,16 @@ static int db_build_tables(utb_db *db, size_t nb_binix, size_t nb_recs) {
             if (e != cudaSuccess) { cudaFree(d_ovf); CK(e); }
             if (!ovf) break;
             cudaFree(db->ktab); db->ktab = nullptr;
-            if (attempt == 3) { cudaFree(d_ovf); utb_set_error("cannot build the lookup table (%u records unplaced)", ovf); return UTB_ERR_LIMIT; }
+            if (attempt == 3) { table_failed = ovf; break; }
             sectors += sectors / 2;
         }
         cudaFree(d_ovf);
+        // Records whose hashes crowd one stretch of sectors more than 1.5^3 growth spreads them: the CTR is
+        // still valid, so search it with the reference probe sequence on the on-disk image (still resident
+        // here) instead of refusing it.  It gets the same L2 set-up as an irregular CTR below.
+        if (table_failed) db->use_table = 0;
+    }
+    if (db->use_table) {
         db->d.ktab = (const uint64_t *)db->ktab; db->d.kt_wide = wide; db->d.kt_sectors = sectors;
         db->nb_ktab = sectors * 32;
         const char *bm = getenv("UTB_SIEVE");                      // 0 off, 1 always, default auto
@@ -2210,10 +2218,13 @@ static int db_build_tables(utb_db *db, size_t nb_binix, size_t nb_recs) {
             } else cudaGetLastError();
         }
     }
-    if (getenv("UTB_STATS"))
-        fprintf(stderr, "utree-b200: device %d: %s, %.2f GB resident (table %.2f GB, sieve %.2f GB)\n", db->device,
-                db->use_table ? "sector hash table" : "reference probe sequence", db->hbm_bytes / 1e9,
+    if (getenv("UTB_STATS")) {
+        char why[96] = "";
+        if (table_failed) snprintf(why, sizeof why, " (sector hash table not built: %u records unplaced)", table_failed);
+        fprintf(stderr, "utree-b200: device %d: %s%s, %.2f GB resident (table %.2f GB, sieve %.2f GB)\n", db->device,
+                db->use_table ? "sector hash table" : "reference probe sequence", why, db->hbm_bytes / 1e9,
                 db->nb_ktab / 1e9, db->nb_sieve / 1e9);
+    }
     return UTB_OK;
 }
 
