@@ -17,7 +17,7 @@
  *     XT_WORD_SEARCH       itree.c:903-933     pack + sieve kernels
  *     XT_getIX32/xtSuffixBS itree.c:699-730    table lookup kernel (or the probe sequence verbatim)
  *     full aufbau vote     itree.c:1028-1098   vote kernels
- *     fprintf lines        itree.c:1032-1096   format kernels (host formatter behind them)
+ *     fprintf lines        itree.c:1032-1096   format kernels
  *   main() search branch   itree.c:1357-1377 utb_main
  */
 #ifndef UTREE_B200_H
@@ -112,15 +112,11 @@ int utb_batch_submit(utb_batch *b, size_t n_bytes, size_t n_reads, int do_rc);
 /* Blocks until the batch is done; *results points at n_reads records in
  * pinned memory, valid until the next submit on this batch. */
 int utb_batch_wait(utb_batch *b, const utb_result **results);
-/* Same pipeline, but the output LINES (itree.c:1032, 1040, 1096) are built on
- * the device too.  The caller additionally fills, per read, where its name
- * sits in the raw bytes (utb_batch_name_off/_len, pinned).  wait_text returns
- * the finished text of the batch (pinned, valid until the next submit) and the
- * number of reads with >= 1 hit. */
+/* Pinned, per read: where its name sits in the raw bytes.  The search
+ * pipeline fills them for the format kernels, which build the output LINES
+ * (itree.c:1032, 1040, 1096) on the device. */
 uint32_t *utb_batch_name_off(utb_batch *b);
 uint32_t *utb_batch_name_len(utb_batch *b);
-int utb_batch_submit_text(utb_batch *b, size_t n_bytes, size_t n_reads, int do_rc);
-int utb_batch_wait_text(utb_batch *b, const char **text, size_t *len, uint64_t *good_finds);
 /* Re-runs only the device stages on the inputs already resident from the last
  * submit (no PCIe traffic) `iters` times and reports CUDA-event milliseconds
  * per stage, summed over iters: ms[0]=pack ms[1]=lookup ms[2]=vote ms[3]=total.
@@ -165,11 +161,6 @@ int utb_vote_hits_sparse(utb_db *db, const uint32_t *hits, const uint64_t *off,
 int utb_frame_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
                       uint64_t *seq_off, uint32_t *seq_len, uint32_t *name_off, uint32_t *name_len,
                       size_t *n_reads, size_t *used, int *ref_exit);
-/* Newline count and NUL detection of a buffer on the host threads (AVX2).  The
- * search pipeline no longer needs it -- records are framed on the GPU, the
- * host only cuts chunks before a line that begins with '>' -- it is kept as a
- * host stage the CPU tests check the device-side count against. */
-int utb_count_newlines(const char *buf, size_t n, int threads, size_t *n_newlines, int *has_nul);
 /* The reference's output lines (itree.c:1032, 1040, 1096) for n_reads result
  * records; names are taken from bytes[name_off[r] .. +name_len[r]). */
 int utb_format_results(const utb_ctr *ctr, const char *bytes, const uint32_t *name_off, const uint32_t *name_len,

@@ -213,24 +213,6 @@ def test_framer_odd_inputs(built):
             assert (rc != 0) == bad, (data, t)
 
 
-def test_newline_counter_of_the_device_framing_path(built):
-    """utb_count_newlines: all the host looks at when the GPU frames the records."""
-    from utree_b200 import capi
-    rng = np.random.default_rng(5)
-    for n in (0, 1, 31, 32, 33, 255 * 32, 255 * 32 + 7, 100_003):
-        raw = rng.integers(1, 256, size=n, dtype=np.uint8)
-        raw[rng.random(n) < 0.02] = 10
-        data = raw.tobytes()
-        for t in (1, 3, 16):
-            assert capi.count_newlines(data, t) == (data.count(b"\n"), False), (n, t)
-        if n:
-            raw[n // 2] = 0
-            assert capi.count_newlines(raw.tobytes(), 4) == (raw.tobytes().count(b"\n"), True)
-    for fa in ("toyA_reads.fa", "edge_reads.fa", "long_reads.fa"):
-        data = open(gold(fa), "rb").read()
-        assert capi.count_newlines(data, 5) == (data.count(b"\n"), b"\0" in data)
-
-
 def test_framer_partial_buffer_carries_the_tail(built):
     """Without EOF an incomplete last record is left for the next buffer."""
     from utree_b200 import capi

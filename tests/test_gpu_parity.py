@@ -301,17 +301,16 @@ def test_cli_binary_matches_reference(ctrs, tmp_path, db_name, reads, out, rc):
     assert lines[-2] == f"Good finds: {n_out}"
 
 
-@pytest.mark.parametrize("variant", ["1", "2", "3", "4"])
-def test_cli_sieve_kernel_variants_agree(ctrs, tmp_path, variant):
-    """UTB_SV_VARIANT picks another (steps per tile, CTAs per SM) instantiation of the sieve kernel once per process;
-    every one must write the golden bytes (reads of 150 bp and the 64 kb queries, whose tiles run into the guard groups)."""
+@pytest.mark.parametrize("reads,out,rc", [c[1:] for c in (CASES[0], CASES[1], CASES[7], CASES[8])])
+def test_cli_with_sieve_forced_on_matches_reference(ctrs, tmp_path, reads, out, rc):
+    """The CLI with the sieve kernel forced on writes the golden bytes: reads of 150 bp (both strands and forward
+    only), the edge cases, and the 64 kb queries, whose tiles run into the guard groups."""
     exe = os.path.join(ROOT, "bin", "utree-search_gg")
     o = str(tmp_path / "cli.out")
-    for reads, out in (("toyA_reads.fa", "toyA_rc.out"), ("long_reads.fa", "long_rc.out"), ("edge_reads.fa", "edge_rc.out")):
-        p = subprocess.run([exe, ctrs["toyA"], gold(reads), o, "2", "RC"], capture_output=True, text=True, timeout=600,
-                           env=dict(os.environ, UTB_SV_VARIANT=variant, UTB_SIEVE="1"))
-        assert p.returncode == 0, p.stderr
-        assert open(o, "rb").read() == open(gold(out), "rb").read(), (variant, reads)
+    p = subprocess.run([exe, ctrs["toyA"], gold(reads), o, "2"] + (["RC"] if rc else []), capture_output=True, text=True,
+                       timeout=600, env=dict(os.environ, UTB_SIEVE="1"))
+    assert p.returncode == 0, p.stderr
+    assert open(o, "rb").read() == open(gold(out), "rb").read()
 
 
 @pytest.mark.parametrize("complevel", [0, 2])
@@ -432,39 +431,46 @@ def test_irregular_ctr_takes_the_exact_probe_path(built, tmp_path):
 
 
 @pytest.mark.parametrize("db_name,reads,out,rc", [CASES[0], CASES[2], CASES[7], CASES[8]])
-def test_host_formatter_path_matches_reference(gpu, tmp_path, db_name, reads, out, rc):
-    """UTB_HOST_FORMAT=1: result records come back and the host formatter team writes the lines
-    (default: the lines are built on the device)."""
+def test_host_formatter_path_matches_reference(gpu, db_name, reads, out, rc):
+    """utb_batch_submit hands back one result record per read and utb_format_results writes the lines on the host
+    (the search pipeline builds them on the device): the reference's output."""
     from utree_b200 import capi
-    os.environ["UTB_HOST_FORMAT"] = "1"
+    ctr, db, _ = gpu[db_name]
+    data = open(gold(reads), "rb").read()
+    code, _, used, recs, (name_off, name_len) = capi.frame_records(data, threads=2)
+    assert code == 0 and used == len(data)
+    lens = np.array([len(seq) for _, seq in recs], dtype=np.uint32)
+    n, total = len(recs), int(lens.sum())
+    b = capi.Batch(db, total + 64, n)
     try:
-        s = capi.Searcher(gpu[db_name][0], devices=(0,), host_threads=4)
+        b.bytes[:total] = np.frombuffer(b"".join(seq for _, seq in recs), dtype=np.uint8)
+        b.seq_off[0] = 0
+        b.seq_off[1:n] = np.cumsum(lens[:-1], dtype=np.uint64)
+        b.seq_len[:n] = lens
+        b.submit(total, n, rc)
+        text = capi.format_results(ctr, data, name_off, name_len, b.wait())
     finally:
-        del os.environ["UTB_HOST_FORMAT"]
-    try:
-        o = str(tmp_path / "out.txt")
-        code, ref_exit, st = s.search_file(gold(reads), o, do_rc=bool(rc))
-        assert code == 0 and open(o, "rb").read() == open(gold(out), "rb").read()
-    finally:
-        s.destroy()
+        b.destroy()
+    assert text == open(gold(out), "rb").read()
 
 
-@pytest.mark.parametrize("host_format", [0, 1])
-def test_zero_copy_from_pinned_caller_buffer(gpu, host_format):
-    """utb_search_mem on a page-locked caller buffer: framed in place, copied to the device from where it lies."""
+@pytest.mark.parametrize("host_frame", [0, 1])
+def test_zero_copy_from_pinned_caller_buffer(gpu, host_frame):
+    """utb_search_mem on a page-locked caller buffer: framed in place (on the device, or by the host framer with
+    UTB_HOST_FRAME=1), copied to the device from where it lies."""
     import torch
     from utree_b200 import capi
     data = open(gold("toyB_reads.fa"), "rb").read() + open(gold("edge_reads.fa"), "rb").read()
     want_b = open(gold("toyB_u32_rc.out"), "rb").read()
     pinned = torch.empty(len(data), dtype=torch.uint8, pin_memory=True)
     pinned.numpy()[:] = np.frombuffer(data, dtype=np.uint8)
-    if host_format:
-        os.environ["UTB_HOST_FORMAT"] = "1"
+    if host_frame:
+        os.environ["UTB_HOST_FRAME"] = "1"
     os.environ["UTB_BATCH_MB"] = "33"
     try:
         s = capi.Searcher(gpu["toyB_u32"][0], devices=(0, 0), host_threads=6)
     finally:
-        os.environ.pop("UTB_HOST_FORMAT", None); os.environ.pop("UTB_BATCH_MB", None)
+        os.environ.pop("UTB_HOST_FRAME", None); os.environ.pop("UTB_BATCH_MB", None)
     try:
         rc, ex, text, st = s.search_mem(None, do_rc=True, ptr=pinned.data_ptr(), n=len(data))
         rc2, ex2, text2, st2 = s.search_mem(data, do_rc=True)            # pageable copy of the same bytes
@@ -472,6 +478,49 @@ def test_zero_copy_from_pinned_caller_buffer(gpu, host_format):
         assert text.startswith(want_b) and st["reads"] == st2["reads"]
     finally:
         s.destroy()
+
+
+def test_tree_with_a_long_label_is_searched_in_smaller_batches(built, tmp_path):
+    """A batch's output lines are built on the device in a buffer sized for every read printing the longest label,
+    addressed with 32 bits.  toyA with one label 32 KB longer would need far more than that at the default
+    reads per batch, so the searcher takes fewer reads per batch (about 130 thousand here).  Its reads, twice,
+    around 200 thousand random 40-mers that hit nothing: two batches at least, with lines in the first and
+    the last, 132 of them ending in the long label.  The output equals the checker's."""
+    import collections
+    from tools import synth
+    from utree_b200 import capi
+    words, ixs, tail, ix_bytes = synth.ubt_read(gold("toyA.ubt"))
+    labels = [l.rsplit(b"\t", 1)[0] for l in tail.split(b"\n") if l]
+    printed = collections.Counter(l.split(b"\t")[1] for l in open(gold("toyA_rc.out"), "rb").read().splitlines())
+    longest = max(range(len(labels)), key=lambda i: printed[labels[i]])
+    labels[longest] += b"x" * 32768
+    path = str(tmp_path / "long.ctr")
+    synth.ctr_write(path, words, ixs, synth._label_tail(labels, np.bincount(ixs.astype(np.int64), minlength=len(labels))),
+                    ix_bytes=ix_bytes)
+    rng = np.random.default_rng(3)
+    pad = np.frombuffer(b"ACGT", np.uint8)[rng.integers(0, 4, (200_000, 40))]
+    toy = open(gold("toyA_reads.fa"), "rb").read()
+    fa = str(tmp_path / "reads.fa")
+    open(fa, "wb").write(toy + b"".join(b">p%d\n%s\n" % (k, pad[k].tobytes()) for k in range(len(pad))) + toy)
+    orc = oracle_api.OracleDb(path)
+    want = str(tmp_path / "want.out")
+    code, ost, err = orc.search_file(fa, want, do_rc=True)
+    orc.free()
+    assert code == 0, err
+    want = open(want, "rb").read()
+    assert sum(1 for l in want.splitlines() if l.split(b"\t")[1] == labels[longest]) == 132
+    ctr = capi.Ctr(path)
+    s = capi.Searcher(ctr, devices=(0,), host_threads=4)
+    try:
+        o = str(tmp_path / "out.txt")
+        code, _, st = s.search_file(fa, o, do_rc=True)
+        assert code == 0 and open(o, "rb").read() == want
+        code, _, text, st2 = s.search_mem(open(fa, "rb").read(), do_rc=True)
+        assert code == 0 and text == want
+        for x in (st, st2):
+            assert x["batches"] >= 2 and (x["reads"], x["good_finds"]) == (ost["reads"], ost["good_finds"])
+    finally:
+        s.destroy(); ctr.close()
 
 
 @pytest.mark.parametrize("env", [{"UTB_SIEVE": "0"}, {"UTB_SIEVE": "1"}, {"UTB_LOOKUP": "exact"}])

@@ -7,16 +7,12 @@ constructed: mix64 is invertible, so a record with any chosen hash, hence any ch
 unmix64(hash).  Every answer is compared with the CPU checker (oracle/), which the golden tests pin to the
 reference.  The CPU tests check the construction itself with a model of the table."""
 import contextlib
-import json
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 import conftest  # noqa: F401  (puts the repo root on sys.path)
-from conftest import ROOT
 
 MISS = 0xFFFFFFFF
 M64 = (1 << 64) - 1
@@ -627,46 +623,35 @@ def dense(request, gpu_built, tmp_path_factory):
     orc.free()
 
 
-def _dense_expect(dense, rc):
+def _dense_expect(dense, rc, reps=DENSE_REPS):
     text, st = dense["want"][rc]
     assert st["hits"] > st["lookups"] // (2 if rc else 1) * 8 // 10     # nearly every forward window is a member
-    return text * DENSE_REPS, tuple(st[k] * DENSE_REPS for k in ("lookups", "hits", "good_finds"))
-
-
-_VARIANT_RUN = r"""
-import json, sys
-sys.path.insert(0, sys.argv[1])
-from utree_b200 import capi
-ctr = capi.Ctr(sys.argv[2])
-s = capi.Searcher(ctr, devices=(0,), host_threads=3)
-data = open(sys.argv[3], "rb").read()
-res = {}
-for rc in (1, 0):
-    code, _, text, st = s.search_mem(data, do_rc=bool(rc))
-    open(sys.argv[4] + str(rc), "wb").write(text)
-    res[rc] = [code, st["lookups"], st["hits"], st["good_finds"]]
-s.destroy(); ctr.close()
-print(json.dumps(res))
-"""
+    return text * reps, tuple(st[k] * reps for k in ("lookups", "hits", "good_finds"))
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("variant", ["0", "1", "2", "3", "4"])
-def test_dense_tree_sieve_has_no_false_negatives_in_any_kernel_variant(dense, variant):
-    """Sieve forced on; UTB_SV_VARIANT is read once per process, so each variant runs in a process of its own.
-    Both strands and forward only: the bytes and the lookups and hits counts equal the checker's."""
-    d = dense["dir"]
-    out = str(d / ("var%s_" % variant))
-    p = subprocess.run([sys.executable, "-c", _VARIANT_RUN, ROOT, dense["path"], str(d / "all.fa"), out],
-                       capture_output=True, text=True, timeout=900,
-                       env=dict(os.environ, UTB_SIEVE="1", UTB_SV_VARIANT=variant))
-    assert p.returncode == 0, p.stderr
-    res = json.loads(p.stdout.strip().splitlines()[-1])
-    for rc in (1, 0):
-        text, counts = _dense_expect(dense, rc)
-        code, *got = res[str(rc)]
-        assert code == 0 and tuple(got) == counts, (rc, got, counts)
-        assert open(out + str(rc), "rb").read() == text, rc
+@pytest.mark.parametrize("env,reps", [({}, DENSE_REPS), ({"UTB_HOST_FRAME": "1"}, DENSE_REPS), ({}, 1),
+                                      ({"UTB_HOST_FRAME": "1"}, 1), ({"UTB_BATCH_MB": "33"}, 0)],
+                         ids=["device_frame", "host_frame", "device_frame_one_copy", "host_frame_one_copy", "batches"])
+def test_dense_tree_sieve_has_no_false_negatives(dense, env, reps):
+    """Sieve forced on.  The sieve kernel's grid follows the batch: persistent warps over several tiles each
+    (DENSE_REPS copies of the reads), one tile per warp (one copy), and several batches of 33 MiB (reps 0: over
+    100 MiB).  The group count it stops at comes from the device framer, or with UTB_HOST_FRAME=1 from the host.
+    Both strands and forward only: the bytes and the lookups, hits and good finds counts equal the checker's."""
+    from utree_b200 import capi
+    reps = reps or 110 * 1024 * 1024 // len(dense["one"]) + 1
+    ctr = capi.Ctr(dense["path"])
+    with _env({"UTB_SIEVE": "1", **env}):
+        s = capi.Searcher(ctr, devices=(0,), host_threads=3)
+    try:
+        for rc in (1, 0):
+            text, counts = _dense_expect(dense, rc, reps)
+            code, _, got, st = s.search_mem(dense["one"] * reps, do_rc=bool(rc))
+            assert code == 0 and (st["lookups"], st["hits"], st["good_finds"]) == counts, rc
+            assert got == text, rc
+            assert st["batches"] >= (3 if "UTB_BATCH_MB" in env else 1)
+    finally:
+        s.destroy(); ctr.close()
 
 
 @pytest.mark.gpu

@@ -47,8 +47,8 @@ EXPORTS = [
     "utb_device_count", "utb_db_upload", "utb_db_free", "utb_db_hbm_bytes", "utb_db_lookup_mode",
     "utb_batch_create", "utb_batch_destroy", "utb_batch_bytes", "utb_batch_seq_off", "utb_batch_seq_len",
     "utb_batch_max_bytes", "utb_batch_max_reads", "utb_read_slots", "utb_batch_max_slots",
-    "utb_batch_submit", "utb_batch_wait", "utb_batch_name_off", "utb_batch_name_len", "utb_batch_submit_text", "utb_batch_wait_text", "utb_batch_rerun_device", "utb_batch_counts", "utb_batch_lookup_detail", "utb_db_clone", "utb_db_device",
-    "utb_lookup_words", "utb_pack_sequence", "utb_vote_hits", "utb_vote_hits_sparse", "utb_frame_records", "utb_count_newlines", "utb_format_results",
+    "utb_batch_submit", "utb_batch_wait", "utb_batch_name_off", "utb_batch_name_len", "utb_batch_rerun_device", "utb_batch_counts", "utb_batch_lookup_detail", "utb_db_clone", "utb_db_device",
+    "utb_lookup_words", "utb_pack_sequence", "utb_vote_hits", "utb_vote_hits_sparse", "utb_frame_records", "utb_format_results",
     "utb_searcher_create", "utb_searcher_destroy", "utb_search_file", "utb_search_mem", "utb_free",
     "utb_main", "utb_main_shallow", "utb_build_ubt", "utb_build_main", "utb_searcher_set_shallow", "utb_measure_rand32", "utb_compress_ubt", "utb_compress_main",
 ]
@@ -149,14 +149,6 @@ def frame_records(buf: bytes, eof=True, threads=1, max_reads=None):
                                  name_off.ctypes.data, name_len.ctypes.data, C.byref(n), C.byref(used), C.byref(ex))
     recs = [(buf[name_off[i]:name_off[i] + name_len[i]], buf[seq_off[i]:seq_off[i] + seq_len[i]]) for i in range(n.value)]
     return rc, ex.value, used.value, recs, (name_off[:n.value].copy(), name_len[:n.value].copy())
-
-
-def count_newlines(buf: bytes, threads=1):
-    """Host stage of the device-side framing (utb_count_newlines) -> (n_newlines, has_nul)."""
-    n, z = C.c_size_t(), C.c_int()
-    lib().utb_count_newlines.argtypes = [C.c_char_p, C.c_size_t, C.c_int, C.POINTER(C.c_size_t), C.POINTER(C.c_int)]
-    _ck(lib().utb_count_newlines(buf, len(buf), threads, C.byref(n), C.byref(z)))
-    return n.value, bool(z.value)
 
 
 def format_results(ctr, buf, name_off, name_len, results):

@@ -85,7 +85,6 @@ struct utb_db {
     int sieve_mode;            // 0 off, 1 always, 2 auto (on while the observed hit rate is low)
     volatile double ema_hit_rate;   // of the batches seen so far (written by the formatter thread, read at submit)
     size_t max_label;          // longest label, bytes
-    volatile double text_per_byte;  // running estimate of output bytes per input byte (sizes the speculative text D2H)
     uint64_t hbm_bytes;
     int sm_count;              // multiprocessors of the device (grid sizing)
     size_t nb_binix, nb_recs, nb_blob, nb_lab, nb_ktab, nb_sieve;   // bytes behind the device pointers (utb_db_clone)
@@ -636,7 +635,7 @@ __device__ __forceinline__ uint32_t emit_survivors(const DevDB &db, WarpQueue &w
 // where positions beyond lane 31 belong to the next step -- which is computed one tile ahead and
 // carried over, so nothing is computed twice.
 // template parameters of sieve_kernel: SV_U steps per tile (= filter loads in flight per lane), SV_MINB CTAs per SM
-// the register budget is sized for; the pair in use is picked at run time (sv_variant: measured on B200, UTB_SV_VARIANT)
+// the register budget is sized for (launch_stages uses U = 6 at 3 CTAs per SM; the measurements are at the launch)
 #define SV_DEAD 0xFFFFFFFFu       // SvStep.blk of a position without a valid window
 struct SvStep { uint32_t wh, wl, rh, rl, h, blk; };              // window, its reverse complement (halves), 16-mer hash, block in the line
 struct SvWords { uint64_t hi, lo, rhi, rlo; uint32_t bh, bl; };   // groups s and s + 1 of pk / pkr / bad
@@ -1676,8 +1675,8 @@ shallow_compact_kernel(VoteIn in, uint32_t n_reads, const uint32_t *__restrict__
 // ---------------------------------------------------------------------------
 // output text on the device (the fprintf lines of itree.c:1032, 1040, 1096)
 // ---------------------------------------------------------------------------
-// The host formatter competes with the framer for a handful of cores (16 for
-// 8 GPUs on the test box), so the lines are produced here: per-read length,
+// Formatting on the host would compete with the framer for a handful of cores
+// (16 for 8 GPUs on the test box), so the lines are produced here: per-read length,
 // exclusive scan, then one warp per read copies name, label prefix and the
 // numeric tail.  The host only moves the finished text to the sink.
 __device__ __forceinline__ uint32_t dec_digits(uint32_t v) {
@@ -2207,8 +2206,7 @@ static int db_build_tables(utb_db *db, size_t nb_binix, size_t nb_recs) {
         // index so the record traffic does not evict it (applied per stream in utb_batch_create).
         cudaDeviceProp p;
         CK(cudaGetDeviceProperties(&p, db->device));
-        const char *env = getenv("UTB_L2_PERSIST");
-        if ((!env || atoi(env) != 0) && p.persistingL2CacheMaxSize > 0 && p.accessPolicyMaxWindowSize > 0) {
+        if (p.persistingL2CacheMaxSize > 0 && p.accessPolicyMaxWindowSize > 0) {
             size_t want = nb_binix < (size_t)p.persistingL2CacheMaxSize ? nb_binix : (size_t)p.persistingL2CacheMaxSize;
             if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
                 db->l2_window = 1;
@@ -2356,10 +2354,10 @@ struct utb_batch {
     uint64_t *d_pk; uint32_t *d_bad; uint32_t *d_hits; uint64_t *d_pkr;
     utb_result *d_results; uint32_t *d_gen_list; uint32_t *d_gen_count; uint32_t *d_warp_list; uint32_t *d_warp_count;
     uint32_t *d_name_off, *d_name_len, *d_line_len, *d_line_off, *d_scan_sums, *d_text_len; char *d_text;
-    int want_text; cudaEvent_t text_len_ready; size_t text_prefetched;
+    utb_batch_out out;
     unsigned long long *d_counters;   // [4][COUNTER_SLOTS]: lookups, hits, good finds, exact-path sectors (summed on the host)
     vote_scratch vs;
-    uint32_t *d_sel_cnt, *d_sel_off, *d_sel, *d_sel_gap, *d_sel_total, *h_sel_cnt, *h_sel, *h_sel_total; size_t sel_cap;   // non-GG mode (want_text == 3)
+    uint32_t *d_sel_cnt, *d_sel_off, *d_sel, *d_sel_gap, *d_sel_total, *h_sel_cnt, *h_sel, *h_sel_total; size_t sel_cap;   // non-GG mode (UTB_OUT_SELECTIONS)
     uint64_t *d_qwords; uint32_t *d_qslots; unsigned long long *d_qcount; uint64_t q_cap;   // filter survivors
     uint32_t *d_hitmap;
     uint32_t *d_rid, *d_hcnt;     // group -> read, hits per read (list mode of the survivor kernel)
@@ -2370,7 +2368,6 @@ struct utb_batch {
     uint32_t *d_nl, *d_blk, *d_frame_err, *h_frame_err; int framed_on_device;
     uint32_t *d_frame_info;                                        // [0] newlines of the chunk, [1] NUL seen
     uint32_t *d_dims, *h_dims; const uint32_t *dims_dev;           // [0] records, [1] position groups of the batch as the device derived them
-    size_t in_bytes;                                               // raw bytes of the last submit
 };
 
 extern "C" uint64_t utb_read_slots(uint32_t len) { return ((uint64_t)len + 1 + 31) / 32; }
@@ -2390,7 +2387,6 @@ extern "C" void utb_batch_destroy(utb_batch *b) {
     cudaFreeHost(b->h_name_off); cudaFreeHost(b->h_name_len); cudaFreeHost(b->h_text); cudaFreeHost(b->h_text_len);
     cudaFree(b->d_name_off); cudaFree(b->d_name_len); cudaFree(b->d_line_len); cudaFree(b->d_line_off); cudaFree(b->d_scan_sums);
     cudaFree(b->d_text_len); cudaFree(b->d_text);
-    if (b->text_len_ready) cudaEventDestroy(b->text_len_ready);
     cudaFree(b->d_raw); cudaFree(b->d_seq_off); cudaFree(b->d_seq_len); cudaFree(b->d_grp_off);
     cudaFree(b->d_pk); cudaFree(b->d_bad); cudaFree(b->d_hits); cudaFree(b->d_results); cudaFree(b->d_pkr);
     cudaFree(b->d_gen_list); cudaFree(b->d_gen_count); cudaFree(b->d_warp_list); cudaFree(b->d_warp_count); cudaFree(b->d_counters);
@@ -2432,7 +2428,6 @@ extern "C" int utb_batch_create(utb_db *db, size_t max_bytes, size_t max_reads, 
     BK(cudaMallocHost(&b->h_name_off, (max_reads + 1) * 4));
     BK(cudaMallocHost(&b->h_name_len, (max_reads + 1) * 4));
     BK(cudaMallocHost(&b->h_text_len, 4));
-    BK(cudaEventCreateWithFlags(&b->text_len_ready, cudaEventDisableTiming));
     BK(cudaMalloc(&b->d_name_off, (max_reads + 1) * 4));
     BK(cudaMalloc(&b->d_name_len, (max_reads + 1) * 4));
     BK(cudaMalloc(&b->d_line_len, (max_reads + 1) * 4));
@@ -2518,7 +2513,7 @@ static int launch_stages(utb_batch *b, bool timed) {
             // under its read (list mode, see HitSink); non-GG path: by slot, flagged in a 1-bit-per-slot map
             HitSink sink;
             sink.hits = b->d_hits; sink.sh = nstr == 2 ? 6u : 5u;
-            const bool lists = b->want_text != 3;
+            const bool lists = b->out != UTB_OUT_SELECTIONS;
             if (lists) { sink.hitmap = nullptr; sink.rid = b->d_rid; sink.grp_off = b->d_grp_off; sink.cnt = b->d_hcnt;
                          CK(cudaMemsetAsync(b->d_hcnt, 0, ((size_t)n_reads + 1) * 4, b->st)); }
             else { sink.hitmap = b->d_hitmap; sink.rid = nullptr; sink.grp_off = nullptr; sink.cnt = nullptr;
@@ -2526,23 +2521,15 @@ static int launch_stages(utb_batch *b, bool timed) {
             b->used_lists = lists;
             if (timed) CK(cudaEventRecord(b->ev[4], b->st));
             // persistent: MINB CTAs per SM, every warp a contiguous range of steps (small batches: one tile per warp)
-            static const int sv_variant = [] { const char *e = getenv("UTB_SV_VARIANT"); return e ? atoi(e) : 0; }();
-#define SV_LAUNCH(U, MINB) do { \
-                const unsigned wb = (n_groups + 8u * U - 1) / (8u * U); \
-                const unsigned pb = wb < sms * MINB ? (wb ? wb : 1u) : sms * MINB; \
-                if (nstr == 2) sieve_kernel<2, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pk, b->d_bad, b->d_pkr, n_pos, b->dims_dev ? b->dims_dev + 1 : nullptr, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink); \
-                else sieve_kernel<1, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pk, b->d_bad, b->d_pkr, n_pos, b->dims_dev ? b->dims_dev + 1 : nullptr, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink); } while (0)
             // measured on B200, 10 M x 150 bp (profiles/r02_sieve_variants.txt): U = 6 steps per tile at 3 CTAs per SM (80
             // registers) 8.54 ms; (5, 3) 8.60; (4, 3) 8.81; (4, 4) 8.98 (64 registers: 16 of them spilled); (3, 4) 9.22;
             // (4, 5) 9.85; (2, 5) 10.5; (6, 2) 9.66; (8, 2) 9.88 -- instructions per step, not occupancy, decide
-            switch (sv_variant) {
-            case 1: SV_LAUNCH(4, 3); break;
-            case 2: SV_LAUNCH(4, 4); break;
-            case 3: SV_LAUNCH(2, 6); break;
-            case 4: SV_LAUNCH(5, 3); break;
-            default: SV_LAUNCH(6, 3); break;
-            }
-#undef SV_LAUNCH
+            constexpr unsigned U = 6, MINB = 3;
+            const unsigned wb = (n_groups + 8u * U - 1) / (8u * U);
+            const unsigned pb = wb < sms * MINB ? (wb ? wb : 1u) : sms * MINB;
+            const uint32_t *sv_groups = b->dims_dev ? b->dims_dev + 1 : nullptr;
+            if (nstr == 2) sieve_kernel<2, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pk, b->d_bad, b->d_pkr, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
+            else sieve_kernel<1, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pk, b->d_bad, b->d_pkr, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
             if (timed) CK(cudaEventRecord(b->ev[5], b->st));
             if (lists) queue_lookup_kernel<true><<<sms * 6, 256, 0, b->st>>>(d, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink, b->d_counters);
             else queue_lookup_kernel<false><<<sms * 6, 256, 0, b->st>>>(d, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink, b->d_counters);
@@ -2557,7 +2544,7 @@ static int launch_stages(utb_batch *b, bool timed) {
         b->launches++;
     }
     if (timed) CK(cudaEventRecord(b->ev[2], b->st));
-    if (n_reads && b->want_text == 3) {
+    if (n_reads && b->out == UTB_OUT_SELECTIONS) {
         // non-GG mode: no vote on the device (it depends on the order of the reads, itree.c:982); the ids the
         // reference's skipping slide would have collected, per read, compacted: count -> scan -> fill
         VoteIn in;
@@ -2596,45 +2583,41 @@ static int launch_stages(utb_batch *b, bool timed) {
 }
 
 // Text buffers (the device-resident measurement batches never format): d_text holds the worst case (every read
-// prints its name and the longest label); the page-locked staging h_text is sized for the typical output
-// (about half the input) and grown on demand -- page-locking is the slow part (~0.25 s per GB).
+// prints its name and the longest label); the page-locked staging h_text, through which file sinks take the text
+// piece by piece, is sized for the typical output (about half the input) -- page-locking is the slow part.
+static size_t text_bytes(size_t max_bytes, size_t max_reads, size_t max_label) {
+    return max_bytes + max_reads * (max_label + 48) + 64;
+}
+#define TEXT_LIMIT (((size_t)1 << 32) - 1)                         // the format kernels address the text with 32 bits
+extern "C" size_t utb_text_max_reads(size_t max_bytes, size_t max_reads, size_t max_label) {
+    const size_t fixed = text_bytes(max_bytes, 0, max_label);
+    if (fixed > TEXT_LIMIT) return 0;
+    const size_t fit = (TEXT_LIMIT - fixed) / (max_label + 48);
+    return fit < max_reads ? fit : max_reads;
+}
 static int ensure_text_buffers(utb_batch *b) {
     if (b->d_text) return UTB_OK;
-    size_t cap = b->max_bytes + b->max_reads * (b->db->max_label + 48) + 64;
-    if (cap >= ((size_t)1 << 32)) { utb_set_error("batch too large for device-side formatting"); return UTB_ERR_LIMIT; }
+    const size_t cap = text_bytes(b->max_bytes, b->max_reads, b->db->max_label);
+    if (cap > TEXT_LIMIT) { utb_set_error("batch too large for device-side formatting"); return UTB_ERR_LIMIT; }
     const size_t hcap = b->max_bytes / 2 + ((size_t)8 << 20) < cap ? b->max_bytes / 2 + ((size_t)8 << 20) : cap;
     CK(cudaMalloc(&b->d_text, cap));
     CK(cudaMallocHost(&b->h_text, hcap));
     b->text_cap = cap; b->h_text_cap = hcap;
     return UTB_OK;
 }
-static int grow_text_staging(utb_batch *b, size_t need) {
-    if (need <= b->h_text_cap) return UTB_OK;
-    CK(cudaStreamSynchronize(b->st));
-    cudaFreeHost(b->h_text); b->h_text = nullptr; b->h_text_cap = 0;
-    CK(cudaMallocHost(&b->h_text, need));
-    b->h_text_cap = need;
-    return UTB_OK;
-}
-// Everything a searcher's batch will need, allocated up front (utb_searcher_create) instead of inside its first search.
-extern "C" int utb_batch_prepare(utb_batch *b, int want_text, int chunked);
 static int ensure_shallow_buffers(utb_batch *b);
 
-static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, int want_text, uint64_t total_groups);
-static int finish_submit(utb_batch *b, size_t n_bytes);
+static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out, uint64_t total_groups);
+static int finish_submit(utb_batch *b);
 extern "C" int utb_batch_submit(utb_batch *b, size_t n_bytes, size_t n_reads, int do_rc) {
-    return submit_impl(b, nullptr, n_bytes, n_reads, do_rc, 0, 0);
-}
-extern "C" int utb_batch_submit_text(utb_batch *b, size_t n_bytes, size_t n_reads, int do_rc) {
-    return submit_impl(b, nullptr, n_bytes, n_reads, do_rc, 1, 0);
+    return submit_impl(b, nullptr, n_bytes, n_reads, do_rc, UTB_OUT_RESULTS, 0);
 }
 // Pipeline-internal variant: `src` (pinned host memory, or NULL for the batch's own staging) holds the raw
 // bytes; total_groups != 0 means the caller already summed utb_read_slots() over the reads, so the
-// per-read offsets are scanned on the device instead of in a serial host loop.  want_text: 0 result
-// records, 1 text through the batch's pinned staging, 2 text left on the device for utb_batch_text_to().
+// per-read offsets are scanned on the device instead of in a serial host loop.
 extern "C" int utb_batch_submit_ex(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc,
-                                   int want_text, uint64_t total_groups) {
-    return submit_impl(b, src, n_bytes, n_reads, do_rc, want_text, total_groups);
+                                   utb_batch_out out, uint64_t total_groups) {
+    return submit_impl(b, src, n_bytes, n_reads, do_rc, out, total_groups);
 }
 extern "C" int utb_host_ptr_is_pinned(const void *p) {
     cudaPointerAttributes a;
@@ -2653,7 +2636,7 @@ extern "C" void utb_pinned_free(void *p) { if (p) cudaFreeHost(p); }
 extern "C" uint32_t *utb_batch_name_off(utb_batch *b) { return b->h_name_off; }
 extern "C" uint32_t *utb_batch_name_len(utb_batch *b) { return b->h_name_len; }
 
-static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, int want_text, uint64_t total_groups) {
+static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out, uint64_t total_groups) {
     if (!b) { utb_set_error("utb_batch_submit: null batch"); return UTB_ERR_ARG; }
     if (n_bytes > b->max_bytes || n_reads > b->max_reads) { utb_set_error("utb_batch_submit: batch over capacity"); return UTB_ERR_LIMIT; }
     CK(cudaSetDevice(b->db->device));
@@ -2673,11 +2656,11 @@ static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_r
     }
     if (!total_groups) b->h_grp_off[n_reads] = (uint32_t)g;
     b->n_reads = n_reads; b->n_groups = (uint32_t)g; b->do_rc = do_rc ? 1 : 0;
-    b->want_text = want_text; b->dims_dev = nullptr; b->framed_on_device = 0;
-    if (want_text == 3) {                                          // non-GG mode: the names stay with the host framer
+    b->out = out; b->dims_dev = nullptr; b->framed_on_device = 0;
+    if (out == UTB_OUT_SELECTIONS) {                               // non-GG mode: the names stay with the host framer
         int rt = ensure_shallow_buffers(b);
         if (rt) return rt;
-    } else if (want_text) {
+    } else if (out == UTB_OUT_TEXT) {
         int rt = ensure_text_buffers(b);
         if (rt) return rt;
         if (n_reads) {
@@ -2699,16 +2682,15 @@ static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_r
             b->launches += 4;
         }
     }
-    return finish_submit(b, n_bytes);
+    return finish_submit(b);
 }
 
-// device stages + (text | result records) + counters back to the host, all on the batch's stream
-static int finish_submit(utb_batch *b, size_t n_bytes) {
+// device stages + (text | result records | selections) + counters back to the host, all on the batch's stream
+static int finish_submit(utb_batch *b) {
     const size_t n_reads = b->n_reads;                             // device-side framing: an upper bound (the device holds the count)
-    const int want_text = b->want_text;
     int rc = launch_stages(b, true);
     if (rc) return rc;
-    if (want_text == 3) {
+    if (b->out == UTB_OUT_SELECTIONS) {
         // per-read counts, the total, and (device-framed batches) where the names are; the id list follows in the wait
         if (n_reads) {
             CK(cudaMemcpyAsync(b->h_sel_cnt, b->d_sel_cnt, n_reads * 4, cudaMemcpyDeviceToHost, b->st));
@@ -2718,7 +2700,7 @@ static int finish_submit(utb_batch *b, size_t n_bytes) {
             }
         }
         CK(cudaMemcpyAsync(b->h_sel_total, b->d_sel_total, 4, cudaMemcpyDeviceToHost, b->st));
-    } else if (want_text) {
+    } else if (b->out == UTB_OUT_TEXT) {
         // lines built on the device: lengths -> exclusive scan -> one warp per read writes its line
         const uint32_t n = (uint32_t)n_reads, nt = (n + SCAN_TILE - 1) / SCAN_TILE;
         CK(cudaMemsetAsync(b->d_text_len, 0, 4, b->st));
@@ -2733,21 +2715,11 @@ static int finish_submit(utb_batch *b, size_t n_bytes) {
             CK(cudaGetLastError());
         }
         CK(cudaMemcpyAsync(b->h_text_len, b->d_text_len, 4, cudaMemcpyDeviceToHost, b->st));
-        b->text_prefetched = 0;
-        if (want_text == 1) {
-            // the text length is only known on the device: copy an estimate now (no extra round trip in the
-            // common case), wait_text tops it up if it was short
-            size_t est = (size_t)(b->db->text_per_byte * 1.15 * (double)n_bytes) + 4096;
-            if (b->db->text_per_byte <= 0) est = 0;
-            if (est > b->h_text_cap) est = b->h_text_cap;
-            b->text_prefetched = est;
-            if (est) CK(cudaMemcpyAsync(b->h_text, b->d_text, est, cudaMemcpyDeviceToHost, b->st));
-        }
     } else if (n_reads) CK(cudaMemcpyAsync(b->h_results, b->d_results, n_reads * sizeof(utb_result), cudaMemcpyDeviceToHost, b->st));
     if (b->dims_dev) CK(cudaMemcpyAsync(b->h_dims, b->d_dims, 8, cudaMemcpyDeviceToHost, b->st));
     CK(cudaMemcpyAsync(b->h_counters, b->d_counters, 4 * COUNTER_SLOTS * 8, cudaMemcpyDeviceToHost, b->st));
     CK(cudaEventRecord(b->done, b->st));
-    b->in_flight = 1; b->in_bytes = n_bytes;
+    b->in_flight = 1;
     return UTB_OK;
 }
 
@@ -2786,19 +2758,20 @@ static int ensure_shallow_buffers(utb_batch *b) {
     CK(cudaMallocHost(&b->h_sel_total, 4));
     return UTB_OK;
 }
-extern "C" int utb_batch_prepare(utb_batch *b, int want_text, int chunked) {
+// Everything a searcher's batch will need, allocated up front (utb_searcher_create) instead of inside its first search.
+extern "C" int utb_batch_prepare(utb_batch *b, utb_batch_out out, int chunked) {
     if (!b) { utb_set_error("utb_batch_prepare: null batch"); return UTB_ERR_ARG; }
     CK(cudaSetDevice(b->db->device));
-    int rc = want_text == 3 ? ensure_shallow_buffers(b) : want_text ? ensure_text_buffers(b) : UTB_OK;
+    int rc = out == UTB_OUT_SELECTIONS ? ensure_shallow_buffers(b) : out == UTB_OUT_TEXT ? ensure_text_buffers(b) : UTB_OK;
     if (!rc && chunked) rc = ensure_chunk_buffers(b);
     return rc;
 }
-extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, int want_text) {
-    if (!b || !n_bytes || want_text < 1 || want_text > 3) { utb_set_error("utb_batch_submit_chunk: bad argument"); return UTB_ERR_ARG; }
+extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out) {
+    if (!b || !n_bytes || out == UTB_OUT_RESULTS) { utb_set_error("utb_batch_submit_chunk: bad argument"); return UTB_ERR_ARG; }
     if (n_bytes > b->max_bytes || n_reads > b->max_reads || n_bytes >= 0xFFFFFFFFull) { utb_set_error("utb_batch_submit_chunk: batch over capacity"); return UTB_ERR_LIMIT; }
     CK(cudaSetDevice(b->db->device));
     { int ra = ensure_chunk_buffers(b); if (ra) return ra; }
-    int rt = want_text == 3 ? ensure_shallow_buffers(b) : ensure_text_buffers(b);
+    int rt = out == UTB_OUT_SELECTIONS ? ensure_shallow_buffers(b) : ensure_text_buffers(b);
     if (rt) return rt;
     // upper bounds the launches are sized for: every read owns ceil((len+1)/32) <= len/32 + 1 groups
     const size_t n_ub = n_reads ? n_reads : b->max_reads;
@@ -2806,7 +2779,7 @@ extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_by
     if (g_ub > b->max_groups) g_ub = b->max_groups;
     if (g_ub * 32ull * (do_rc ? 2u : 1u) >= 0xFFFFFFFFull) { utb_set_error("utb_batch_submit_chunk: chunk too large for the 32-bit slot space"); return UTB_ERR_LIMIT; }
     b->n_reads = n_ub; b->n_groups = (uint32_t)g_ub; b->do_rc = do_rc ? 1 : 0;
-    b->want_text = want_text; b->dims_dev = b->d_dims; b->framed_on_device = 1;
+    b->out = out; b->dims_dev = b->d_dims; b->framed_on_device = 1;
     *b->h_frame_err = FR_ERR_NONE;
     CK(cudaMemcpyAsync(b->d_raw, src ? src : b->h_bytes, n_bytes, cudaMemcpyHostToDevice, b->st));
     CK(cudaMemsetAsync(b->d_frame_err, 0xFF, 4, b->st));
@@ -2825,7 +2798,7 @@ extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_by
     b->launches += 8;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(b->h_frame_err, b->d_frame_err, 4, cudaMemcpyDeviceToHost, b->st));
-    return finish_submit(b, n_bytes);
+    return finish_submit(b);
 }
 // After the wait of a chunk submit: 0 if the chunk and every record of it were well formed, else 1 with the index
 // of the first malformed record and its code (1 no header '>', 2 sequence begins '>', 4 line too long, 7 the
@@ -2857,36 +2830,10 @@ extern "C" int utb_batch_wait(utb_batch *b, const utb_result **results) {
     return UTB_OK;
 }
 
-// After utb_batch_submit_text: blocks until the batch is done and its output text is in pinned host memory.
-extern "C" int utb_batch_wait_text(utb_batch *b, const char **text, size_t *len, uint64_t *good_finds) {
-    if (!b || !text || !len) { utb_set_error("utb_batch_wait_text: null argument"); return UTB_ERR_ARG; }
-    if (b->want_text != 1) { utb_set_error("utb_batch_wait_text: batch was not submitted for text through the staging buffer"); return UTB_ERR_ARG; }
-    int rc = utb_batch_wait(b, nullptr);
-    if (rc) return rc;
-    const size_t n = *b->h_text_len;
-    if (n > b->text_cap) { utb_set_error("device text overflow"); return UTB_ERR_LIMIT; }
-    if (n > b->h_text_cap) {                                        // more text than the staging holds: grow it, copy afresh
-        rc = grow_text_staging(b, n + n / 8);
-        if (rc) return rc;
-        b->text_prefetched = 0;
-    }
-    if (n > b->text_prefetched) {
-        CK(cudaMemcpyAsync(b->h_text + b->text_prefetched, b->d_text + b->text_prefetched, n - b->text_prefetched,
-                           cudaMemcpyDeviceToHost, b->st));
-        CK(cudaStreamSynchronize(b->st));
-    }
-    if (b->in_bytes >= 4096) {
-        double r = (double)n / (double)b->in_bytes;
-        b->db->text_per_byte = b->db->text_per_byte <= 0 ? r : 0.5 * b->db->text_per_byte + 0.5 * r;
-    }
-    *text = b->h_text; *len = n;
-    if (good_finds) { uint64_t g = 0; for (int i = 0; i < COUNTER_SLOTS; ++i) g += b->h_counters[2 * COUNTER_SLOTS + i]; *good_finds = g; }
-    return UTB_OK;
-}
-// want_text == 2: blocks until the batch is done; its text (*len bytes) is still on the device.
+// UTB_OUT_TEXT: blocks until the batch is done; its text (*len bytes) is still on the device.
 extern "C" int utb_batch_wait_len(utb_batch *b, size_t *len, uint64_t *good_finds) {
     if (!b || !len) { utb_set_error("utb_batch_wait_len: null argument"); return UTB_ERR_ARG; }
-    if (b->want_text != 2) { utb_set_error("utb_batch_wait_len: batch was not submitted with the text left on the device"); return UTB_ERR_ARG; }
+    if (b->out != UTB_OUT_TEXT) { utb_set_error("utb_batch_wait_len: batch was not submitted with the text left on the device"); return UTB_ERR_ARG; }
     int rc = utb_batch_wait(b, nullptr);
     if (rc) return rc;
     *len = *b->h_text_len;
@@ -2894,12 +2841,12 @@ extern "C" int utb_batch_wait_len(utb_batch *b, size_t *len, uint64_t *good_find
     if (good_finds) { uint64_t g = 0; for (int i = 0; i < COUNTER_SLOTS; ++i) g += b->h_counters[2 * COUNTER_SLOTS + i]; *good_finds = g; }
     return UTB_OK;
 }
-// want_text == 3 (non-GG mode): blocks until the batch is done and the ids its reads selected are in page-locked host
+// UTB_OUT_SELECTIONS (non-GG mode): blocks until the batch is done and the ids its reads selected are in page-locked host
 // memory: sel_cnt[r] ids per read, back to back in sel; name_off / name_len: where the read names sit in the raw bytes.
 extern "C" int utb_batch_wait_shallow(utb_batch *b, const uint32_t **sel_cnt, const uint32_t **sel, size_t *sel_total,
                                       const uint32_t **name_off, const uint32_t **name_len) {
     if (!b || !sel_cnt || !sel || !sel_total) { utb_set_error("utb_batch_wait_shallow: null argument"); return UTB_ERR_ARG; }
-    if (b->want_text != 3) { utb_set_error("utb_batch_wait_shallow: batch was not submitted in the non-GG mode"); return UTB_ERR_ARG; }
+    if (b->out != UTB_OUT_SELECTIONS) { utb_set_error("utb_batch_wait_shallow: batch was not submitted in the non-GG mode"); return UTB_ERR_ARG; }
     int rc = utb_batch_wait(b, nullptr);
     if (rc) return rc;
     const size_t n = b->n_reads ? *b->h_sel_total : 0;

@@ -11,9 +11,10 @@
  *                     submits the batch.  No per-read copies: the device gets
  *                     the file bytes as they are plus one (offset, length)
  *                     pair per read.
- *   formatter team -- waits for batches in sequence order, formats the lines
- *                     of a batch in parallel, and emits them in order
- *                     (parallel pwrite / memcpy at prefix-summed offsets).
+ *   formatter team -- waits for batches in sequence order and moves the lines
+ *                     the device built for each to the output, in order
+ *                     (parallel pwrite / memcpy; a page-locked output arena
+ *                     takes them straight from the device).
  * Slots are dealt round-robin over the devices, the database being replicated
  * on each, so multi-GPU needs no collective: the ordered merge is the only
  * cross-device step (SURVEY 8e).
@@ -33,24 +34,6 @@
 #include <sys/vfs.h>
 #include <time.h>
 #include <unistd.h>
-
-int utb_batch_last_ms(utb_batch *b, float ms[4]);
-int utb_ctr_probe(const char *path, uint64_t md[4], uint64_t *binix_read);
-int utb_batch_submit_ex(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, int want_text, uint64_t total_groups);
-int utb_host_ptr_is_pinned(const void *p);
-uint64_t utb_batch_launches(const utb_batch *b);
-int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, int want_text);
-int utb_batch_frame_error(const utb_batch *b, size_t *record, int *code);
-size_t utb_batch_reads(const utb_batch *b);
-int utb_batch_wait_len(utb_batch *b, size_t *len, uint64_t *good_finds);
-int utb_batch_text_to(utb_batch *b, char *dst, size_t len);
-int utb_batch_sync(utb_batch *b);
-int utb_batch_text_piece(utb_batch *b, size_t off, size_t *len, const char **piece);
-int utb_batch_prepare(utb_batch *b, int want_text, int chunked);
-int utb_batch_wait_shallow(utb_batch *b, const uint32_t **sel_cnt, const uint32_t **sel, size_t *sel_total,
-                           const uint32_t **name_off, const uint32_t **name_len);
-int utb_pinned_alloc(size_t n, void **out);
-void utb_pinned_free(void *p);
 
 #define SLOTS_PER_DEVICE 4                         /* measured on B200, ms per 10 M reads (profiles/r02_e2e_sweep.txt): 2 slots 42.9, 3: 36.0, 4: 35.5, 5: 38.0, 6: 37.6 */
 #define DEFAULT_BATCH_BYTES ((size_t)128 << 20)   /* ~2.3 ms of PCIe per batch: launch and sync costs are a few percent of that */
@@ -134,8 +117,7 @@ struct utb_searcher {
     size_t batch_bytes, batch_reads, ramp_bytes;
     size_t max_label;              /* longest label incl. NUL */
     int verbose;                   /* CLI: progress lines on stdout */
-    int device_format;             /* output lines built on the GPU (default) or by the host formatter team */
-    int device_frame;              /* records framed on the GPU (default with device_format): the host only cuts chunks at a "\n>" */
+    int device_frame;              /* records framed on the GPU (default): the host only cuts chunks at a "\n>" */
     int shallow;                   /* the non-GG binary's search (-D SEARCH): SPARSITY-skip slide + shallow vote (utb_searcher_set_shallow) */
     uint32_t *horses; size_t horses_cap;   /* its AllTheKingsHorses (itree.c:970): survives from read to read within a search */
     uint32_t *tally;               /* its Hashes (itree.c:971) */
@@ -186,15 +168,15 @@ int utb_searcher_create(const utb_ctr *ctr, const int *devices, int n_devices,
     const char *e = getenv("UTB_BATCH_MB");
     s->batch_bytes = e && atoi(e) > 0 ? (size_t)atoi(e) << 20 : DEFAULT_BATCH_BYTES;
     if (s->batch_bytes < 2 * (size_t)UTB_LINELEN + 4096) s->batch_bytes = 2 * (size_t)UTB_LINELEN + 4096; /* one max record must fit */
-    s->batch_reads = s->batch_bytes / 64;
-    e = getenv("UTB_HOST_FORMAT");
-    s->device_format = !(e && atoi(e) != 0);
     e = getenv("UTB_HOST_FRAME");
-    s->device_frame = s->device_format && !(e && atoi(e) != 0);
+    s->device_frame = !(e && atoi(e) != 0);
     for (uint32_t i = 0; i < ctr->max_ix; ++i) {
         size_t l = ctr->off[i + 1] - ctr->off[i];
         if (l > s->max_label) s->max_label = l;
     }
+    /* the output lines of a batch are built on the device: long labels take fewer reads per batch */
+    s->batch_reads = utb_text_max_reads(s->batch_bytes, s->batch_bytes / 64, s->max_label);
+    if (!s->batch_reads) { free(s); utb_set_error("batch too large for device-side formatting"); return UTB_ERR_LIMIT; }
     s->devices = (int *)malloc(sizeof(int) * (size_t)n_devices);
     s->dbs = (utb_db **)calloc((size_t)n_devices, sizeof(utb_db *));
     e = getenv("UTB_SLOTS");                                       /* stream slots per device (tuning) */
@@ -222,7 +204,7 @@ int utb_searcher_create(const utb_ctr *ctr, const int *devices, int n_devices,
         sl->dev_index = i % n_devices;
         if (s->spread) mem_interleave(1);
         int rc = utb_batch_create(s->dbs[sl->dev_index], s->batch_bytes, s->batch_reads, &sl->b);
-        if (!rc) rc = utb_batch_prepare(sl->b, s->device_format, s->device_frame);   /* nothing is allocated inside a search */
+        if (!rc) rc = utb_batch_prepare(sl->b, UTB_OUT_TEXT, s->device_frame);   /* nothing is allocated inside a search */
         if (s->spread) mem_interleave(0);
         if (rc) { utb_searcher_destroy(s); return rc; }
         sl->name_off = utb_batch_name_off(sl->b);                  /* pinned: the device formatter reads them too */
@@ -243,7 +225,7 @@ int utb_searcher_set_shallow(utb_searcher *s, int on) {
     if (!s->tally) s->tally = (uint32_t *)calloc(s->ctr->max_ix ? s->ctr->max_ix : 1, sizeof(uint32_t));
     if (!s->tally) { utb_set_error("out of memory"); return UTB_ERR_NOMEM; }
     for (int i = 0; i < s->n_slots; ++i) {
-        int rc = utb_batch_prepare(s->slots[i].b, 3, s->device_frame);
+        int rc = utb_batch_prepare(s->slots[i].b, UTB_OUT_SELECTIONS, s->device_frame);
         if (rc) return rc;
     }
     return UTB_OK;
@@ -427,38 +409,15 @@ static inline char *put_u32(char *p, uint32_t v) {
     return p;
 }
 
-typedef struct {
-    const utb_ctr *c; const slot_t *sl; const utb_result *res; const char *bytes;
-    size_t max_label;
-    char *buf[MAX_TEAM]; size_t cap[MAX_TEAM], len[MAX_TEAM], off[MAX_TEAM];
-    uint64_t good[MAX_TEAM];
-    int nomem;
-    sink_t *sink;
-} fmt_ctx;
-
-/* One line per read with >= 1 hit; shapes of itree.c:1032, 1040, 1096. */
-static void fmt_part(void *c_, int part, int nparts) {
-    fmt_ctx *f = (fmt_ctx *)c_;
-    const slot_t *sl = f->sl;
-    size_t r0 = sl->n_reads * (size_t)part / (size_t)nparts, r1 = sl->n_reads * (size_t)(part + 1) / (size_t)nparts;
-    size_t need = 0;
-    for (size_t r = r0; r < r1; ++r) need += sl->name_len[r];
-    need += (r1 - r0) * (f->max_label + 64) + 64;   /* name + label + 4 tabs + 4 numbers + newline */
-    if (need > f->cap[part]) {
-        free(f->buf[part]);
-        f->cap[part] = need + (need >> 2);
-        f->buf[part] = (char *)malloc(f->cap[part]);
-        if (!f->buf[part]) { f->cap[part] = 0; f->len[part] = 0; f->nomem = 1; return; }
-    }
-    const utb_ctr *c = f->c;
-    const char *bytes = f->bytes;
-    char *p = f->buf[part];
-    uint64_t g = 0;
-    for (size_t r = r0; r < r1; ++r) {
-        const utb_result *v = &f->res[r];
+/* One line per read with >= 1 hit, reads [0, n); shapes of itree.c:1032, 1040, 1096.  out has room for every
+ * name plus n * (max_label + 64) + 64 bytes.  Returns the length written. */
+static size_t fmt_lines(const utb_ctr *c, const char *bytes, const uint32_t *name_off, const uint32_t *name_len,
+                        const utb_result *res, size_t n, char *out) {
+    char *p = out;
+    for (size_t r = 0; r < n; ++r) {
+        const utb_result *v = &res[r];
         if (v->kind == UTB_NONE) continue;
-        ++g;
-        memcpy(p, bytes + sl->name_off[r], sl->name_len[r]); p += sl->name_len[r];
+        memcpy(p, bytes + name_off[r], name_len[r]); p += name_len[r];
         *p++ = '\t';
         const char *lab = c->blob + c->off[v->label];
         size_t ll = c->off[v->label + 1] - c->off[v->label] - 1;
@@ -474,18 +433,7 @@ static void fmt_part(void *c_, int part, int nparts) {
         else { p = put_u32(p, v->sl); *p++ = ';'; p = put_u32(p, v->ol); }
         *p++ = '\n';
     }
-    f->len[part] = (size_t)(p - f->buf[part]);
-    f->good[part] = g;
-}
-static void emit_part(void *c_, int part, int nparts) {
-    fmt_ctx *f = (fmt_ctx *)c_;
-    (void)nparts;
-    if (f->len[part]) sink_put(f->sink, f->buf[part], f->len[part], f->off[part]);
-}
-/* every part of the host formatter's output; in order by one thread when the sink is a stream */
-static void emit_all(team_t *team, fmt_ctx *f) {
-    if (f->sink->fd >= 0 && f->sink->stream) { for (int p = 0; p < team->n; ++p) emit_part(f, p, team->n); }
-    else team_run(team, emit_part, f);
+    return (size_t)(p - out);
 }
 
 typedef struct { sink_t *sink; const char *text; size_t len, off; } copy_ctx;
@@ -502,19 +450,19 @@ static void copy_all(team_t *team, copy_ctx *c) {
 /* The shallow vote of the non-GG binary, read by read in input order (itree.c:979-1003).  sel_cnt[r] ids per read,
  * back to back in sel, are what its slide appended to AllTheKingsHorses; `if (!kingsMen++)` (itree.c:982) never
  * fires but bumps the count, so the tally runs over ONE MORE entry: whatever an earlier read of this search left
- * at that index (0 if none did).  Lines go to F->buf[0]. */
+ * at that index (0 if none did).  Lines go to *buf (*cap bytes, grown as needed). */
 static int shallow_vote(utb_searcher *s, const slot_t *sl, const uint32_t *sel_cnt, const uint32_t *sel, size_t sel_total,
-                        fmt_ctx *F, size_t *n_out, uint64_t *good_out) {
+                        char **buf, size_t *cap, size_t *n_out, uint64_t *good_out) {
     const utb_ctr *c = s->ctr;
     size_t need = 64;
     for (size_t r = 0; r < sl->n_reads; ++r) if (sel_cnt[r]) need += sl->name_len[r] + s->max_label + 48;
-    if (need > F->cap[0]) {
-        free(F->buf[0]);
-        F->cap[0] = need + (need >> 2);
-        F->buf[0] = (char *)malloc(F->cap[0]);
-        if (!F->buf[0]) { F->cap[0] = 0; utb_set_error("out of memory (formatter)"); return UTB_ERR_NOMEM; }
+    if (need > *cap) {
+        free(*buf);
+        *cap = need + (need >> 2);
+        *buf = (char *)malloc(*cap);
+        if (!*buf) { *cap = 0; utb_set_error("out of memory (formatter)"); return UTB_ERR_NOMEM; }
     }
-    char *p = F->buf[0];
+    char *p = *buf;
     uint64_t good = 0;
     size_t at = 0;
     uint32_t *tally = s->tally;
@@ -551,7 +499,7 @@ static int shallow_vote(utb_searcher *s, const slot_t *sl, const uint32_t *sel_c
         memcpy(p, lab, ll); p += ll;
         p += sprintf(p, "\t%f\t%d\n", (double)1 - (double)second / most, (int)most);   /* itree.c:1002 */
     }
-    *n_out = (size_t)(p - F->buf[0]);
+    *n_out = (size_t)(p - *buf);
     *good_out = good;
     return UTB_OK;
 }
@@ -559,10 +507,8 @@ static int shallow_vote(utb_searcher *s, const slot_t *sl, const uint32_t *sel_c
 static void *formatter_main(void *arg) {
     run_t *R = (run_t *)arg;
     utb_searcher *s = R->s;
-    fmt_ctx F;
-    memset(&F, 0, sizeof F);
-    F.c = s->ctr; F.max_label = s->max_label; F.sink = R->sink;
-    const int direct = s->device_format && R->sink->fd < 0;       /* device text -> its final place in the arena */
+    char *vote_buf = NULL; size_t vote_cap = 0;                    /* the non-GG mode's lines */
+    const int direct = R->sink->fd < 0;                            /* device text -> its final place in the arena */
     for (uint64_t seq = 0;; ++seq) {
         pthread_mutex_lock(&R->mu);
         while (R->submitted <= seq && !R->done_reading) pthread_cond_wait(&R->cv, &R->mu);
@@ -570,12 +516,11 @@ static void *formatter_main(void *arg) {
         pthread_mutex_unlock(&R->mu);
         if (!have) break;
         slot_t *sl = &s->slots[seq % (uint64_t)s->n_slots];
-        const utb_result *res = NULL;
         const char *text = NULL; size_t text_len = 0; uint64_t good = 0;
         double tw = now_s();
         const uint32_t *sel_cnt = NULL, *sel = NULL; size_t sel_total = 0;
         int rc = s->shallow ? utb_batch_wait_shallow(sl->b, &sel_cnt, &sel, &sel_total, NULL, NULL)
-                            : s->device_format ? utb_batch_wait_len(sl->b, &text_len, &good) : utb_batch_wait(sl->b, &res);
+                            : utb_batch_wait_len(sl->b, &text_len, &good);
         R->st.fm_wait_gpu += now_s() - tw;
         if (seq < 64) R->tl_gpu_done[seq] = now_s() - R->t0;
         if (rc && !R->error) { R->error = rc; snprintf(R->errmsg, sizeof R->errmsg, "%s", utb_last_error()); }
@@ -589,21 +534,19 @@ static void *formatter_main(void *arg) {
         if (!rc && s->shallow) {
             double tf = now_s();
             size_t n_out = 0;
-            int r2 = shallow_vote(s, sl, sel_cnt, sel, sel_total, &F, &n_out, &good);
+            int r2 = shallow_vote(s, sl, sel_cnt, sel, sel_total, &vote_buf, &vote_cap, &n_out, &good);
             if (r2 && !R->error) { R->error = r2; snprintf(R->errmsg, sizeof R->errmsg, "%s", utb_last_error()); }
             R->st.fm_format += now_s() - tf;
             tf = now_s();
             if (!r2 && n_out && !sink_reserve(R->sink, R->sink->off + n_out)) {
-                F.len[0] = n_out; F.off[0] = R->sink->off;
-                emit_part(&F, 0, 1);
-                F.len[0] = 0;
+                sink_put(R->sink, vote_buf, n_out, R->sink->off);
                 R->sink->off += n_out;
                 R->st.out_bytes += n_out;
             }
             R->st.good_finds += good;
             R->st.fm_emit += now_s() - tf;
             R->st.d2h_bytes += sl->n_reads * 12 + sel_total * 4 + 4 * 1024 * 8 + 16;
-        } else if (!rc && s->device_format) {
+        } else if (!rc) {
             double tf = now_s();
             if (text_len && !sink_reserve(R->sink, R->sink->off + text_len)) {
                 if (direct) {
@@ -623,23 +566,6 @@ static void *formatter_main(void *arg) {
             R->st.good_finds += good;
             R->st.fm_emit += now_s() - tf;
             R->st.d2h_bytes += text_len + 4 * 1024 * 8 + 16;
-        } else if (!rc) {
-            F.sl = sl; F.res = res; F.bytes = sl->host_bytes;
-            double tf = now_s();
-            team_run(&R->fmt_team, fmt_part, &F);
-            R->st.fm_format += now_s() - tf;
-            tf = now_s();
-            size_t tot = 0;
-            for (int p = 0; p < R->fmt_team.n; ++p) { F.off[p] = R->sink->off + tot; tot += F.len[p]; R->st.good_finds += F.good[p]; F.good[p] = 0; }
-            if (F.nomem) { R->error = UTB_ERR_NOMEM; snprintf(R->errmsg, sizeof R->errmsg, "out of memory (formatter)"); }
-            else if (!sink_reserve(R->sink, R->sink->off + tot)) {
-                emit_all(&R->fmt_team, &F);
-                R->sink->off += tot;
-                R->st.out_bytes += tot;
-            }
-            for (int p = 0; p < R->fmt_team.n; ++p) F.len[p] = 0;
-            R->st.fm_emit += now_s() - tf;
-            R->st.d2h_bytes += sl->n_reads * sizeof(utb_result) + 32;
         }
         if (!rc) {
             uint64_t lk = 0, ht = 0; float ms[4] = {0, 0, 0, 0};
@@ -661,7 +587,7 @@ static void *formatter_main(void *arg) {
         pthread_cond_broadcast(&R->cv);
         pthread_mutex_unlock(&R->mu);
     }
-    for (int p = 0; p < MAX_TEAM; ++p) free(F.buf[p]);
+    free(vote_buf);
     return NULL;
 }
 
@@ -870,45 +796,6 @@ static void frame_indexed_part(void *c_, int part, int nparts) {
     c->groups[part] = groups;
 }
 
-/* Device-side framing: all the host needs is the number of newlines of the chunk (and that it
- * holds no NUL byte, for which the reference's strlen() semantics would differ). */
-typedef struct { const char *buf; size_t fill; size_t cnt[MAX_TEAM]; int has_nul[MAX_TEAM]; } nlc_ctx;
-#if defined(__x86_64__)
-__attribute__((target("avx2")))
-static size_t nlc_avx2(const char *buf, size_t a, size_t b, int *has_nul) {
-    const __m256i nl = _mm256_set1_epi8('\n'), zero = _mm256_setzero_si256();
-    __m256i accz = zero, acc = zero;
-    size_t n = 0, i = a;
-    unsigned it = 0;
-    for (; i + 32 <= b; i += 32) {
-        __m256i v = _mm256_loadu_si256((const __m256i *)(buf + i));
-        acc = _mm256_sub_epi8(acc, _mm256_cmpeq_epi8(v, nl));       /* per-byte counters: +1 per match */
-        accz = _mm256_or_si256(accz, _mm256_cmpeq_epi8(v, zero));
-        if (++it == 255) {
-            __m256i sad = _mm256_sad_epu8(acc, zero);
-            n += (size_t)_mm256_extract_epi64(sad, 0) + (size_t)_mm256_extract_epi64(sad, 1) + (size_t)_mm256_extract_epi64(sad, 2) + (size_t)_mm256_extract_epi64(sad, 3);
-            acc = zero; it = 0;
-        }
-    }
-    __m256i sad = _mm256_sad_epu8(acc, zero);
-    n += (size_t)_mm256_extract_epi64(sad, 0) + (size_t)_mm256_extract_epi64(sad, 1) + (size_t)_mm256_extract_epi64(sad, 2) + (size_t)_mm256_extract_epi64(sad, 3);
-    int z = _mm256_movemask_epi8(accz) != 0;
-    for (; i < b; ++i) { n += buf[i] == '\n'; z |= !buf[i]; }
-    *has_nul = z;
-    return n;
-}
-#endif
-static void nlc_part(void *c_, int part, int nparts) {
-    nlc_ctx *c = (nlc_ctx *)c_;
-    size_t a = c->fill * (size_t)part / (size_t)nparts, b = c->fill * (size_t)(part + 1) / (size_t)nparts;
-#if defined(__x86_64__)
-    if (__builtin_cpu_supports("avx2")) { c->cnt[part] = nlc_avx2(c->buf, a, b, &c->has_nul[part]); return; }
-#endif
-    size_t n = 0; int z = 0;
-    for (size_t i = a; i < b; ++i) { n += c->buf[i] == '\n'; z |= !c->buf[i]; }
-    c->cnt[part] = n; c->has_nul[part] = z;
-}
-
 static const char *fe_text(int code) {
     switch (code) {
     case FE_NOHEADER: return "ERROR: no header '>'";
@@ -971,35 +858,20 @@ int utb_frame_records(const char *buf, size_t n, int eof, int threads, size_t ma
     return UTB_OK;
 }
 
-/* Host stage of the device-side framing: newline count and NUL detection of buf[0..n). */
-int utb_count_newlines(const char *buf, size_t n, int threads, size_t *n_newlines, int *has_nul) {
-    if ((!buf && n) || !n_newlines || !has_nul) { utb_set_error("utb_count_newlines: null argument"); return UTB_ERR_ARG; }
-    team_t team;
-    if (team_init(&team, threads)) { utb_set_error("cannot start worker threads"); return UTB_ERR_NOMEM; }
-    nlc_ctx C;
-    C.buf = buf; C.fill = n;
-    team_run(&team, nlc_part, &C);
-    *n_newlines = 0; *has_nul = 0;
-    for (int p = 0; p < team.n; ++p) { *n_newlines += C.cnt[p]; *has_nul |= C.has_nul[p]; }
-    team_destroy(&team);
-    return UTB_OK;
-}
-
 int utb_format_results(const utb_ctr *ctr, const char *bytes, const uint32_t *name_off, const uint32_t *name_len,
                        const utb_result *results, size_t n_reads, char *out, size_t out_cap, size_t *out_len) {
     if (!ctr || !bytes || !name_off || !name_len || !results || !out || !out_len) { utb_set_error("utb_format_results: null argument"); return UTB_ERR_ARG; }
-    slot_t sl; memset(&sl, 0, sizeof sl);
-    sl.n_reads = n_reads; sl.name_off = (uint32_t *)name_off; sl.name_len = (uint32_t *)name_len;
-    fmt_ctx F; memset(&F, 0, sizeof F);
-    F.c = ctr; F.sl = &sl; F.res = results; F.bytes = bytes;
-    for (uint32_t i = 0; i < ctr->max_ix; ++i) { size_t l = ctr->off[i + 1] - ctr->off[i]; if (l > F.max_label) F.max_label = l; }
-    fmt_part(&F, 0, 1);
-    if (F.nomem) { utb_set_error("out of memory (formatter)"); return UTB_ERR_NOMEM; }
+    size_t max_label = 0, need = n_reads * 64 + 64;                /* name + label + 4 tabs + 4 numbers + newline */
+    for (uint32_t i = 0; i < ctr->max_ix; ++i) { size_t l = ctr->off[i + 1] - ctr->off[i]; if (l > max_label) max_label = l; }
+    for (size_t r = 0; r < n_reads; ++r) need += name_len[r] + max_label;
+    char *buf = (char *)malloc(need);
+    if (!buf) { utb_set_error("out of memory (formatter)"); return UTB_ERR_NOMEM; }
+    const size_t len = fmt_lines(ctr, bytes, name_off, name_len, results, n_reads, buf);
     int rc = UTB_OK;
-    if (F.len[0] > out_cap) { utb_set_error("utb_format_results: output needs %zu bytes", F.len[0]); rc = UTB_ERR_LIMIT; }
-    else memcpy(out, F.buf[0], F.len[0]);
-    *out_len = F.len[0];
-    free(F.buf[0]);
+    if (len > out_cap) { utb_set_error("utb_format_results: output needs %zu bytes", len); rc = UTB_ERR_LIMIT; }
+    else memcpy(out, buf, len);
+    *out_len = len;
+    free(buf);
     return rc;
 }
 
@@ -1091,7 +963,7 @@ read_loop:
         if (!fill) break;                                          /* clean EOF */
 
         sl->src_off = consumed;
-        const int want_text = s->shallow ? 3 : s->device_format ? 2 : 0;   /* 2: the text stays on the device until the formatter knows where it goes; 3: non-GG mode */
+        const utb_batch_out out = s->shallow ? UTB_OUT_SELECTIONS : UTB_OUT_TEXT;   /* the text stays on the device until the formatter knows where it goes */
         if (device_frame && fill >= 2 && fill < 0xFFFFFFFFull) {
             /* Fast path: the host does not look at the bytes.  In a well-formed file exactly the header lines
              * begin with '>' (itree.c:880, 886), so the chunk is cut right before the last line that does (at the
@@ -1116,7 +988,7 @@ read_loop:
                 else if (used < fill) { carry_len = fill - used; memcpy(carry, buf + used, carry_len); }
                 rd_t[2] += now_s() - tp; tp = now_s();
                 if (seq < 64) { R.tl_framed[seq] = now_s() - t0; R.tl_reads[seq] = 0; }
-                int r2 = utb_batch_submit_chunk(sl->b, zero_copy ? buf : NULL, used, 0, do_rc, want_text);
+                int r2 = utb_batch_submit_chunk(sl->b, zero_copy ? buf : NULL, used, 0, do_rc, out);
                 if (r2) { rc = r2; break; }
                 R.st.h2d_bytes += used;
                 chunked = 1;
@@ -1191,10 +1063,10 @@ read_loop:
         if (seq < 64) { R.tl_framed[seq] = now_s() - t0; R.tl_reads[seq] = n; }
         if (n) {
             /* every sequence lies inside the first n_bytes of the buffer */
-            int r2 = utb_batch_submit_ex(sl->b, zero_copy ? buf : NULL, fmt_err ? fill : used, n, do_rc, want_text,
+            int r2 = utb_batch_submit_ex(sl->b, zero_copy ? buf : NULL, fmt_err ? fill : used, n, do_rc, out,
                                          groups_known && !cut ? groups : 0);
             if (r2) { rc = r2; break; }
-            R.st.h2d_bytes += (fmt_err ? fill : used) + n * (s->device_format ? 24 : 16) + 4;
+            R.st.h2d_bytes += (fmt_err ? fill : used) + n * 24 + 4;
             if (seq < 64) R.tl_submit[seq] = now_s() - t0;
             pthread_mutex_lock(&R.mu);
             sl->state = 1;

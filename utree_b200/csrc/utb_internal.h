@@ -35,6 +35,38 @@ struct utb_ctr {
 
 void utb_set_error(const char *fmt, ...);
 
+/* What a batch hands back to the host. */
+typedef enum {
+    UTB_OUT_RESULTS,      /* one utb_result per read (utb_batch_submit / utb_batch_wait) */
+    UTB_OUT_TEXT,         /* the output lines, kept on the device (utb_batch_wait_len, then _text_to / _text_piece) */
+    UTB_OUT_SELECTIONS    /* non-GG mode: the ids each read selected (utb_batch_wait_shallow) */
+} utb_batch_out;
+
+/* What the search pipeline (pipeline.c) uses of kernels.cu beyond the public header. */
+int utb_batch_prepare(utb_batch *b, utb_batch_out out, int chunked);
+int utb_batch_submit_ex(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out, uint64_t total_groups);
+int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out);
+int utb_batch_frame_error(const utb_batch *b, size_t *record, int *code);
+size_t utb_batch_reads(const utb_batch *b);
+uint64_t utb_batch_launches(const utb_batch *b);
+int utb_batch_last_ms(utb_batch *b, float ms[4]);
+int utb_batch_wait_len(utb_batch *b, size_t *len, uint64_t *good_finds);
+int utb_batch_text_to(utb_batch *b, char *dst, size_t len);
+int utb_batch_text_piece(utb_batch *b, size_t off, size_t *len, const char **piece);
+int utb_batch_wait_shallow(utb_batch *b, const uint32_t **sel_cnt, const uint32_t **sel, size_t *sel_total,
+                           const uint32_t **name_off, const uint32_t **name_len);
+int utb_batch_sync(utb_batch *b);
+/* The most reads per batch, at most max_reads, for which the worst-case output text of a batch of max_bytes raw
+ * bytes (every read printing its name and the longest label, max_label bytes with the NUL) fits the 32-bit offsets
+ * of the format kernels; 0 if none does. */
+size_t utb_text_max_reads(size_t max_bytes, size_t max_reads, size_t max_label);
+int utb_host_ptr_is_pinned(const void *p);
+int utb_pinned_alloc(size_t n, void **out);
+void utb_pinned_free(void *p);
+
+/* ctr_loader.c: the header of a CTR that utb_ctr_open refused as truncated, for the CLI's messages. */
+int utb_ctr_probe(const char *path, uint64_t md[4], uint64_t *binix_read);
+
 #ifdef __cplusplus
 }
 #endif
