@@ -19,6 +19,7 @@
 //             k-mer word order of itree.c:924) and a bad-base bit mask.  Every
 //             read is padded to a multiple of 32 positions with >= 1 bad
 //             position, so a 32-mer window can never straddle two reads.
+//   pl      : the same bases as two bit planes per group (sieve on; the sieve kernel's input)
 //   hits    : sieve on (GG path): per read the labels of its hits back to back from the read's first slot, hcnt[read]
 //             of them; otherwise one u32 per (position, strand), with a 1-bit-per-slot hitmap in the non-GG path
 //   results : one utb_result per read;  text : the output lines
@@ -99,6 +100,7 @@ struct utb_db {
 // One thread per 32-base group.  The 32 bytes are fetched with nine aligned
 // 32-bit loads (neighbouring threads share cache lines, so the raw bytes move
 // once from L2), classified four at a time with byte-SIMD compares.
+// returns the 2-bit codes of the four bytes, one per byte (a 0, c 1, g 2, t 3)
 __device__ __forceinline__ uint32_t classify4(uint32_t w, uint32_t &badbits) {
     const uint32_t u = w | 0x20202020u;                            // fold case (itree.c:114-117)
     // bits 1 and 2 of the letter give its code: a 0x61 -> 0, c 0x63 -> 1, g 0x67 -> 2, t 0x74 -> 3 (C2Xb, itree.c:110-121)
@@ -110,7 +112,7 @@ __device__ __forceinline__ uint32_t classify4(uint32_t w, uint32_t &badbits) {
     const uint32_t x = u ^ expect;                                  // nonzero byte = not ACGTacgt
     const uint32_t inval = ((((x & 0x7F7F7F7Fu) + 0x7F7F7F7Fu) | x) >> 7) & 0x01010101u;
     badbits = (inval * 0x01020408u) >> 24;                          // bit j = byte j is not a base
-    return (code * 0x40100401u) >> 24;                              // first base most significant: b0 << 6 | b1 << 4 | b2 << 2 | b3
+    return code;
 }
 
 // reverse complement of a 32-mer word: reverse the 2-bit fields of ~w
@@ -118,15 +120,36 @@ __device__ __forceinline__ uint64_t revcomp_word(uint64_t w) {
     uint64_t x = __brevll(~w);
     return ((x >> 1) & 0x5555555555555555ull) | ((x & 0x5555555555555555ull) << 1);
 }
+// The bit planes of a 32-mer: one u64, code bit 1 of every base in the upper 32 bits, code bit 0 in the lower 32,
+// base 0 the most significant bit of both.  A window at any offset is then one funnel shift per plane, and the
+// reverse complement of a plane is ~__brev(plane).  The word is the planes' bit interleave (bit 1 of a code odd).
+__device__ __forceinline__ uint64_t word_to_planes(uint64_t w) {   // perfect unshuffle: odd bits up, even bits down
+    uint64_t t;
+    t = (w ^ (w >> 1)) & 0x2222222222222222ull; w ^= t ^ (t << 1);
+    t = (w ^ (w >> 2)) & 0x0C0C0C0C0C0C0C0Cull; w ^= t ^ (t << 2);
+    t = (w ^ (w >> 4)) & 0x00F000F000F000F0ull; w ^= t ^ (t << 4);
+    t = (w ^ (w >> 8)) & 0x0000FF000000FF00ull; w ^= t ^ (t << 8);
+    t = (w ^ (w >> 16)) & 0x00000000FFFF0000ull; w ^= t ^ (t << 16);
+    return w;
+}
+__device__ __forceinline__ uint64_t planes_to_word(uint64_t w) {   // perfect shuffle: the inverse, steps in reverse order
+    uint64_t t;
+    t = (w ^ (w >> 16)) & 0x00000000FFFF0000ull; w ^= t ^ (t << 16);
+    t = (w ^ (w >> 8)) & 0x0000FF000000FF00ull; w ^= t ^ (t << 8);
+    t = (w ^ (w >> 4)) & 0x00F000F000F000F0ull; w ^= t ^ (t << 4);
+    t = (w ^ (w >> 2)) & 0x0C0C0C0C0C0C0C0Cull; w ^= t ^ (t << 2);
+    t = (w ^ (w >> 1)) & 0x2222222222222222ull; w ^= t ^ (t << 1);
+    return w;
+}
 #define PK_GUARD 8u               // all-bad groups behind the last read: the sieve kernel walks whole tiles without bounds checks
-// pkr (optional): the reverse complement of every packed group, so that the reverse-complement window of a
-// position is a funnel shift of two pkr words exactly as the forward window is one of two pk words; rid (optional):
-// the read every group belongs to
+// WORDS: write pk (the 2-bit words, read by the sieve-off lookup, the non-GG selection and expand_windows_kernel);
+// PLANES: write pl (the bit planes, read by the sieve kernel).  rid (optional): the read every group belongs to
+template <bool WORDS, bool PLANES>
 __global__ void __launch_bounds__(256)
 pack_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ seq_off,
             const uint32_t *__restrict__ seq_len, const uint32_t *__restrict__ grp_off,
             uint32_t n_reads, uint32_t n_groups, const uint32_t *__restrict__ dims,
-            uint64_t *__restrict__ pk, uint32_t *__restrict__ bad, uint64_t *__restrict__ pkr, uint32_t *__restrict__ rid) {
+            uint64_t *__restrict__ pk, uint32_t *__restrict__ bad, uint64_t *__restrict__ pl, uint32_t *__restrict__ rid) {
     if (dims) { n_reads = dims[0]; n_groups = dims[1]; }          // device-side framing: the host only knows upper bounds
     const uint32_t lane = threadIdx.x & 31u;
     // a warp takes 32 consecutive groups per round (warp-uniform loop)
@@ -149,13 +172,19 @@ pack_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ seq_of
             lo += __popc(starts & (0xFFFFFFFFu >> (31u - lane)));   // boundaries at groups g0 + 1 .. g0 + lane
         }
         if (g >= n_groups + PK_GUARD) continue;
-        if (g >= n_groups) { pk[g] = 0; bad[g] = 0xFFFFFFFFu; if (pkr) pkr[g] = 0; continue; }   // guard groups: all positions bad
+        if (g >= n_groups) {                                       // guard groups: all positions bad
+            if (WORDS) pk[g] = 0;
+            if (PLANES) pl[g] = 0;
+            bad[g] = 0xFFFFFFFFu;
+            continue;
+        }
         uint32_t k = g - __ldg(grp_off + lo);
         uint32_t len = __ldg(seq_len + lo);
         if (rid) rid[g] = lo;                                      // group -> read (phase B files a hit under its read)
         uint32_t b0 = k * 32u;
         uint32_t nv = len > b0 ? min(32u, len - b0) : 0u;  // real bases in this group
         uint64_t word = 0;
+        uint32_t p1 = 0, p0 = 0;                                   // the planes, first base most significant
         uint32_t badm = 0;
         if (nv) {
             uint64_t a = __ldg(seq_off + lo) + b0;
@@ -169,15 +198,20 @@ pack_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ seq_of
                 uint32_t w = __funnelshift_r(prev, cur, sh);
                 prev = cur;
                 uint32_t bb;
-                uint32_t c = classify4(w, bb);
-                word = (word << 8) | c;
+                const uint32_t code = classify4(w, bb);
+                // first base most significant: b0 << 6 | b1 << 4 | b2 << 2 | b3, resp. b0 << 3 | b1 << 2 | b2 << 1 | b3 per plane
+                if (WORDS) word = (word << 8) | ((code * 0x40100401u) >> 24);
+                if (PLANES) {
+                    p1 = (p1 << 4) | ((((code >> 1) & 0x01010101u) * 0x08040201u) >> 24);
+                    p0 = (p0 << 4) | (((code & 0x01010101u) * 0x08040201u) >> 24);
+                }
                 badm |= bb << (4u * j);
             }
         }
         if (nv < 32u) badm |= 0xFFFFFFFFu << nv;           // padding positions are bad
-        pk[g] = word;
+        if (WORDS) pk[g] = word;
+        if (PLANES) pl[g] = ((uint64_t)p1 << 32) | p0;
         bad[g] = badm;
-        if (pkr) pkr[g] = revcomp_word(word);
     }
 }
 
@@ -443,10 +477,18 @@ verify_kernel(DevDB db, unsigned long long *__restrict__ out) {
 // block, by x itself: one 8-byte load per position answers both strands, and the
 // two mask words of a strand cost two PRMTs (byte table 1 << n, selected by 3-bit
 // fields of a hash) -- the kernel is bound by the integer pipe, not by memory
-// (profiles/r02_*).  Lines hold SV_RPL records on average (~43 bits per record:
+// (profiles/r02_*, r03_*).  Lines hold SV_RPL records on average (~43 bits per record:
 // ~0.04 % false positives, the spread of the line loads included).
+// Every function here takes a 32-mer as its bit planes x1 (code bit 1 of each base) and x0 (code bit 0), base 0 the
+// most significant bit (word_to_planes): the sieve kernel builds a window with one funnel shift per plane and the
+// reverse complement of a plane is ~__brev(plane).  The build, the sieve kernel and the stage-level lookups all call
+// these, so the three cannot disagree on a hash.  A 16-mer (planes a1, a0 of 16 bits) is keyed as
+// a1[15:8] | a0 | a1[7:0], most significant first: one PRMT from the upper halves of the planes, and a layout that a
+// bit reversal maps onto itself, so the reverse complement of a key is ~__brev(key).
 #define SV_W 17u                // 16-mers per 32-mer
 #define SV_RPL 24u              // records per 128-byte line
+__device__ __forceinline__ uint32_t sv_kmer16(uint32_t x1, uint32_t x0) { return __byte_perm(x1, x0, 0x3762); }   // the 16-mer at offset 0
+__device__ __forceinline__ uint32_t sv_rc16(uint32_t m) { return ~__brev(m); }   // the key of its reverse complement
 __device__ __forceinline__ uint32_t sv_mhash(uint32_t m, uint32_t r) {   // order key of a 16-mer m with reverse complement r
     uint32_t a = m < r ? m : r;
     a *= 0x9E3779B1u; a ^= a >> 15; a *= 0x85EBCA77u;
@@ -456,34 +498,37 @@ __device__ __forceinline__ uint32_t sv_line(uint32_t mv, uint32_t n_lines) {   /
     uint32_t t = mv * 0xB5297A4Du; t ^= t >> 16; t *= 0x68E31DA5u;           // the minimum of 17 hashes is small: spread it again
     return __umulhi(t, n_lines);
 }
-// xh / rh: upper halves (first 16 bases) of the word and of its reverse complement -- symmetric in the two
-__device__ __forceinline__ uint32_t sv_block(uint32_t xh, uint32_t rh) { return ((xh ^ rh) * 0x9E3779B1u) >> 28; }
+// h0 / h16: order keys of the first and the last 16-mer of the word -- the reverse complement swaps the two, so
+// the block is the same for both strands (and independent of the line, which the minimum of all 17 keys picks)
+__device__ __forceinline__ uint32_t sv_block(uint32_t h0, uint32_t h16) { return (h0 ^ h16) >> 28; }
 // the word's two mask words: one bit in each of the block's 8 bytes
-__device__ __forceinline__ uint2 sv_masks(uint32_t xh, uint32_t xl) {
-    uint32_t e = xh * 0xC2B2AE3Du + xl * 0x27D4EB2Fu;
+__device__ __forceinline__ uint2 sv_masks(uint32_t x1, uint32_t x0) {
+    uint32_t e = x1 * 0xC2B2AE3Du + x0 * 0x27D4EB2Fu;
     e ^= e >> 15;
     const uint32_t s0 = __umulhi(e, 0x165667B1u) & 0x7777u, s1 = __umulhi(e, 0x9E3779B1u) & 0x7777u;   // 4 x 3-bit byte selectors each
     return make_uint2(__byte_perm(0x08040201u, 0x80402010u, s0), __byte_perm(0x08040201u, 0x80402010u, s1));
 }
-__device__ __forceinline__ bool sv_test(const uint2 &v, uint32_t xh, uint32_t xl) {
-    const uint2 m = sv_masks(xh, xl);
+__device__ __forceinline__ bool sv_test(const uint2 &v, uint32_t x1, uint32_t x0) {
+    const uint2 m = sv_masks(x1, x0);
     return ((~v.x & m.x) | (~v.y & m.y)) == 0u;
 }
-// minimizer of one word, the slow way (build, stage-level lookups): all 17 16-mers
-__device__ __forceinline__ uint32_t sv_minimizer(uint64_t x, uint64_t rc) {
-    uint32_t mv = 0xFFFFFFFFu;
+// (line, block) of one word, the slow way (build, stage-level lookups): all 17 16-mers
+__device__ __forceinline__ uint32_t sv_index(const DevDB &db, uint32_t x1, uint32_t x0) {
+    uint32_t mv = 0xFFFFFFFFu, h0 = 0, h16 = 0;
 #pragma unroll
     for (uint32_t j = 0; j < SV_W; ++j) {
-        const uint32_t h = sv_mhash((uint32_t)(x >> (32u - 2u * j)), (uint32_t)(rc >> (2u * j)));
+        const uint32_t m = sv_kmer16(x1 << j, x0 << j);
+        const uint32_t h = sv_mhash(m, sv_rc16(m));
         mv = h < mv ? h : mv;
+        if (j == 0) h0 = h;
+        if (j == SV_W - 1) h16 = h;
     }
-    return mv;
+    return (sv_line(mv, db.sv_lines) << 4) | sv_block(h0, h16);
 }
-__device__ __forceinline__ uint32_t sv_index(const DevDB &db, uint32_t mv, uint32_t blk) { return (sv_line(mv, db.sv_lines) << 4) | blk; }
-__device__ __forceinline__ bool sv_maybe(const DevDB &db, uint64_t word) {
-    const uint64_t rc = revcomp_word(word);
-    const uint2 v = __ldg(db.sieve + sv_index(db, sv_minimizer(word, rc), sv_block((uint32_t)(word >> 32), (uint32_t)(rc >> 32))));
-    return sv_test(v, (uint32_t)(word >> 32), (uint32_t)word);
+__device__ __forceinline__ bool sv_maybe(const DevDB &db, uint64_t word) {   // word: the 2-bit form
+    const uint64_t x = word_to_planes(word);
+    const uint32_t x1 = (uint32_t)(x >> 32), x0 = (uint32_t)x;
+    return sv_test(__ldg(db.sieve + sv_index(db, x1, x0)), x1, x0);
 }
 template <int G>
 __global__ void __launch_bounds__(256)
@@ -498,10 +543,10 @@ sieve_build_kernel(DevDB db, uint32_t *__restrict__ sieve) {
     if (a >= b || b > db.num_nodes) return;
     if ((uint32_t)p == db.quirk_bin) ++a;                          // the folded record is unreachable anyway
     for (uint64_t i = a + gl; i < b; i += G) {
-        const uint64_t word = (p << 40) | load_suffix(db.recs, i * db.sz);
-        const uint64_t rc = revcomp_word(word);
-        uint32_t *blk = sieve + 2ull * sv_index(db, sv_minimizer(word, rc), sv_block((uint32_t)(word >> 32), (uint32_t)(rc >> 32)));
-        const uint2 m = sv_masks((uint32_t)(word >> 32), (uint32_t)word);
+        const uint64_t x = word_to_planes((p << 40) | load_suffix(db.recs, i * db.sz));
+        const uint32_t x1 = (uint32_t)(x >> 32), x0 = (uint32_t)x;
+        uint32_t *blk = sieve + 2ull * sv_index(db, x1, x0);
+        const uint2 m = sv_masks(x1, x0);
         atomicOr(blk + 0, m.x); atomicOr(blk + 1, m.y);
     }
 }
@@ -595,14 +640,15 @@ __device__ __forceinline__ void sink_put(const HitSink &k, uint32_t slot, uint32
         k.hits[((uint64_t)__ldg(k.grp_off + rd) << k.sh) + atomicAdd(k.cnt + rd, 1u)] = r;
     } else { k.hits[slot] = r; atomicOr(k.hitmap + (slot >> 5), 1u << (slot & 31u)); }
 }
-// queue overflow: the exact lookup right here (rare)
-__device__ __noinline__ uint32_t resolve_inline(const DevDB &db, uint64_t w, uint32_t slot, const HitSink &sink) {
-    const uint32_t r = kt_lookup(db, w);
+// queue overflow: the exact lookup right here (rare); x: the window's planes
+__device__ __noinline__ uint32_t resolve_inline(const DevDB &db, uint64_t x, uint32_t slot, const HitSink &sink) {
+    const uint32_t r = kt_lookup(db, planes_to_word(x));
     if (r == HIT_MISS) return 0;
     sink_put(sink, slot, r);
     return 1;
 }
-// Appends the survivors of one warp step (warp-uniform call).
+// Appends the survivors of one warp step (warp-uniform call).  w / rc: the planes of the window and of its reverse
+// complement; the queue keeps planes, phase B turns them into words (only ~2.5 % of the windows get there).
 template <int NSTR>
 __device__ __forceinline__ uint32_t emit_survivors(const DevDB &db, WarpQueue &wq, uint32_t lane, bool passF, bool passR, uint64_t w, uint64_t rc,
                                                    uint32_t pos, uint64_t *__restrict__ q_words, uint32_t *__restrict__ q_slots,
@@ -628,28 +674,23 @@ __device__ __forceinline__ uint32_t emit_survivors(const DevDB &db, WarpQueue &w
 
 // Phase A.  Persistent warps; every warp owns a contiguous range of 32-position steps (one step = one
 // group of the packed stream, lane = position) and walks it SV_U steps at a time.  Per step a lane
-// builds its window and the reverse complement of it -- funnel shifts of two consecutive words of
-// the packed stream pk, resp. of its reverse-complement twin pkr, all in 32-bit halves -- and the hash
-// of the canonical 16-mer that STARTS at its position; the minimizer of a window is the minimum of
-// the 17 hashes at positions p .. p+16, taken across lanes with shuffles (doubling: 2, 4, 8, 16, 17),
-// where positions beyond lane 31 belong to the next step -- which is computed one tile ahead and
-// carried over, so nothing is computed twice.
+// builds its window -- one funnel shift per plane of two consecutive groups of the plane stream pl --
+// and the hash of the canonical 16-mer that STARTS at its position; the minimizer of a window is the
+// minimum of the 17 hashes at positions p .. p+16, taken across lanes with shuffles (doubling: 2, 4, 8,
+// 16, 17), where positions beyond lane 31 belong to the next step -- which is computed one tile ahead
+// and carried over, so nothing is computed twice.  The reverse complement of a window is derived only
+// where its strand is tested.
 // template parameters of sieve_kernel: SV_U steps per tile (= filter loads in flight per lane), SV_MINB CTAs per SM
 // the register budget is sized for (launch_stages uses U = 6 at 3 CTAs per SM; the measurements are at the launch)
 #define SV_DEAD 0xFFFFFFFFu       // SvStep.blk of a position without a valid window
-struct SvStep { uint32_t wh, wl, rh, rl, h, blk; };              // window, its reverse complement (halves), 16-mer hash, block in the line
-struct SvWords { uint64_t hi, lo, rhi, rlo; uint32_t bh, bl; };   // groups s and s + 1 of pk / pkr / bad
-__device__ __forceinline__ void sv_step(const SvWords &g, bool upper, uint32_t r2, uint32_t lane, SvStep &s) {
-    // forward window: the 128 bits hi:lo shifted left by 2 * lane, upper 64 bits
-    const uint32_t b0 = (uint32_t)(g.hi >> 32), b1 = (uint32_t)g.hi, b2 = (uint32_t)(g.lo >> 32), b3 = (uint32_t)g.lo;
-    const uint32_t x0 = upper ? b1 : b0, x1 = upper ? b2 : b1, x2 = upper ? b3 : b2;
-    s.wh = __funnelshift_l(x1, x0, r2); s.wl = __funnelshift_l(x2, x1, r2);
-    // its reverse complement: the 128 bits revcomp(lo):revcomp(hi) shifted right by 2 * lane, lower 64 bits
-    const uint32_t a0 = (uint32_t)(g.rlo >> 32), a1 = (uint32_t)g.rlo, a2 = (uint32_t)(g.rhi >> 32), a3 = (uint32_t)g.rhi;
-    const uint32_t z0 = upper ? a2 : a3, z1 = upper ? a1 : a2, z2 = upper ? a0 : a1;
-    s.rl = __funnelshift_r(z0, z1, r2); s.rh = __funnelshift_r(z1, z2, r2);
-    s.h = sv_mhash(s.wh, s.rl);
-    s.blk = __funnelshift_r(g.bh, g.bl, lane) == 0u ? sv_block(s.wh, s.rh) : SV_DEAD;   // a bad base in the 32 positions from here: no window
+struct SvStep { uint32_t w1, w0, h, blk; };                       // window planes, 16-mer hash, SV_DEAD or (later) block in the line
+// cur / next: groups s and s + 1 of pl, bh / bl: of bad
+__device__ __forceinline__ void sv_step(uint64_t cur, uint64_t next, uint32_t bh, uint32_t bl, uint32_t lane, SvStep &s) {
+    s.w1 = __funnelshift_l((uint32_t)(next >> 32), (uint32_t)(cur >> 32), lane);
+    s.w0 = __funnelshift_l((uint32_t)next, (uint32_t)cur, lane);
+    const uint32_t m = sv_kmer16(s.w1, s.w0);
+    s.h = sv_mhash(m, sv_rc16(m));
+    s.blk = __funnelshift_r(bh, bl, lane) == 0u ? 0u : SV_DEAD;   // a bad base in the 32 positions from here: no window
 }
 // x[u][lane] -> value of the (virtual) array x at index 32 * u + lane + D; the last array only serves lanes that stay inside it
 template <int D, int SV_U>
@@ -665,14 +706,12 @@ __device__ __forceinline__ void sv_shifted(const uint32_t (&x)[SV_U + 1], uint32
 __device__ __forceinline__ void sv_prefetch(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 template <int NSTR, int SV_U, int SV_MINB>
 __global__ void __launch_bounds__(256, SV_MINB)
-sieve_kernel(DevDB db, const uint64_t *__restrict__ pk, const uint32_t *__restrict__ bad, const uint64_t *__restrict__ pkr, uint32_t n_pos,
+sieve_kernel(DevDB db, const uint64_t *__restrict__ pl, const uint32_t *__restrict__ bad, uint32_t n_pos,
              const uint32_t *__restrict__ n_groups_dev, unsigned long long *__restrict__ counters,
              uint64_t *__restrict__ q_words, uint32_t *__restrict__ q_slots, unsigned long long *__restrict__ q_count,
              uint64_t q_cap, const HitSink sink) {
     if (n_groups_dev) n_pos = *n_groups_dev * 32u;
     const uint32_t lane = threadIdx.x & 31u;
-    const bool upper = lane >= 16u;
-    const uint32_t r2 = 2u * (lane & 15u);
     const uint32_t n_steps = n_pos >> 5;                           // n_pos is a multiple of 32; PK_GUARD all-bad groups follow group n_steps - 1
     const uint32_t n_warps = gridDim.x * (blockDim.x >> 5), wid = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     uint32_t per = (n_steps + n_warps - 1) / n_warps;
@@ -686,27 +725,29 @@ sieve_kernel(DevDB db, const uint64_t *__restrict__ pk, const uint32_t *__restri
     uint32_t nv = 0, nh = 0;
     if (s0 < s1) {
         SvStep st[SV_U + 1];
-        // groups s and s + 1 feed step s; the pair is carried from step to step (two 8-byte and one 4-byte load per step).
+        // groups s and s + 1 feed step s; the pair is carried from step to step (one 8-byte and one 4-byte load per step).
         // A tile may run past s1 only at the very end of the batch, into the guard groups: no bounds checks in the loop.
-        SvWords g;
-        g.hi = __ldg(pk + s0); g.rhi = __ldg(pkr + s0); g.bh = __ldg(bad + s0);
-        g.lo = __ldg(pk + s0 + 1); g.rlo = __ldg(pkr + s0 + 1); g.bl = __ldg(bad + s0 + 1);
-        sv_step(g, upper, r2, lane, st[0]);
+        uint64_t cur = __ldg(pl + s0), next = __ldg(pl + s0 + 1);
+        uint32_t bh = __ldg(bad + s0), bl = __ldg(bad + s0 + 1);
+        sv_step(cur, next, bh, bl, lane, st[0]);
         for (uint32_t s = (uint32_t)s0; s < s1; s += SV_U) {
-            {   // the three streams are read front to back: ask for the lines two ahead (a line of pk / pkr feeds 16 steps)
+            {   // both streams are read front to back: ask for the lines two ahead (a line of pl feeds 16 steps)
                 const uint32_t pf = s + 32u < n_steps ? s + 32u : n_steps;
-                sv_prefetch(pk + pf); sv_prefetch(pkr + pf); sv_prefetch(bad + pf);
+                sv_prefetch(pl + pf); sv_prefetch(bad + pf);
             }
 #pragma unroll
             for (int u = 1; u <= SV_U; ++u) {
-                g.hi = g.lo; g.rhi = g.rlo; g.bh = g.bl;
-                g.lo = __ldg(pk + s + u + 1); g.rlo = __ldg(pkr + s + u + 1); g.bl = __ldg(bad + s + u + 1);
-                sv_step(g, upper, r2, lane, st[u]);
+                cur = next; bh = bl;
+                next = __ldg(pl + s + u + 1); bl = __ldg(bad + s + u + 1);
+                sv_step(cur, next, bh, bl, lane, st[u]);
             }
             // minimizer = min of the 17 hashes at q .. q+16: windows of 3, then 9 (3 + 3 + 3), then 17 (9 + 9, one shared)
             uint32_t x[SV_U + 1], y1[SV_U + 1], y2[SV_U + 1];
 #pragma unroll
             for (int u = 0; u <= SV_U; ++u) x[u] = st[u].h;
+            sv_shifted<16, SV_U>(x, y1, lane);                                           // the window's last 16-mer
+#pragma unroll
+            for (int u = 0; u < SV_U; ++u) st[u].blk |= sv_block(x[u], y1[u]);          // SV_DEAD stays SV_DEAD
             sv_shifted<1, SV_U>(x, y1, lane); sv_shifted<2, SV_U>(x, y2, lane);
 #pragma unroll
             for (int u = 0; u <= SV_U; ++u) x[u] = __vimin3_u32(x[u], y1[u], y2[u]);     // [q, q+2]
@@ -726,8 +767,9 @@ sieve_kernel(DevDB db, const uint64_t *__restrict__ pk, const uint32_t *__restri
             for (int u = 0; u < SV_U; ++u) {
                 const bool live = st[u].blk != SV_DEAD;
                 if (__any_sync(0xFFFFFFFFu, live)) {               // the padding group behind every read holds no window at all
-                    const bool tF = sv_test(v[u], st[u].wh, st[u].wl), tR = NSTR == 2 && sv_test(v[u], st[u].rh, st[u].rl);
-                    nh += emit_survivors<NSTR>(db, wq, lane, live & tF, live & tR, ((uint64_t)st[u].wh << 32) | st[u].wl, ((uint64_t)st[u].rh << 32) | st[u].rl,
+                    const uint32_t r1 = ~__brev(st[u].w1), r0 = ~__brev(st[u].w0);   // the reverse complement's planes
+                    const bool tF = sv_test(v[u], st[u].w1, st[u].w0), tR = NSTR == 2 && sv_test(v[u], r1, r0);
+                    nh += emit_survivors<NSTR>(db, wq, lane, live & tF, live & tR, ((uint64_t)st[u].w1 << 32) | st[u].w0, ((uint64_t)r1 << 32) | r0,
                                                (s + u) * 32u + lane, q_words, q_slots, q_count, q_cap, sink);
                     nv += live ? NSTR : 0;                         // nothing is stored for a miss
                 }
@@ -762,7 +804,7 @@ queue_lookup_kernel(DevDB db, const uint64_t *__restrict__ q_words, const uint32
         uint32_t r = HIT_MISS;
         if (slot != Q_INVALID) {                                   // else: padding of a retired chunk
             uint32_t sc;
-            r = kt_lookup(db, q_words[i], &sc);
+            r = kt_lookup(db, planes_to_word(q_words[i]), &sc);   // the queue holds planes (see emit_survivors)
             nsect += sc;
         }
         const bool hit = r != HIT_MISS;
@@ -2351,14 +2393,14 @@ struct utb_batch {
     uint32_t *h_name_off, *h_name_len; char *h_text; uint32_t *h_text_len; size_t text_cap, h_text_cap;   // device-side formatting
     // device
     uint8_t *d_raw; uint64_t *d_seq_off; uint32_t *d_seq_len; uint32_t *d_grp_off;
-    uint64_t *d_pk; uint32_t *d_bad; uint32_t *d_hits; uint64_t *d_pkr;
+    uint64_t *d_pk; uint32_t *d_bad; uint32_t *d_hits; uint64_t *d_pl;
     utb_result *d_results; uint32_t *d_gen_list; uint32_t *d_gen_count; uint32_t *d_warp_list; uint32_t *d_warp_count;
     uint32_t *d_name_off, *d_name_len, *d_line_len, *d_line_off, *d_scan_sums, *d_text_len; char *d_text;
     utb_batch_out out;
     unsigned long long *d_counters;   // [4][COUNTER_SLOTS]: lookups, hits, good finds, exact-path sectors (summed on the host)
     vote_scratch vs;
     uint32_t *d_sel_cnt, *d_sel_off, *d_sel, *d_sel_gap, *d_sel_total, *h_sel_cnt, *h_sel, *h_sel_total; size_t sel_cap;   // non-GG mode (UTB_OUT_SELECTIONS)
-    uint64_t *d_qwords; uint32_t *d_qslots; unsigned long long *d_qcount; uint64_t q_cap;   // filter survivors
+    uint64_t *d_qwords; uint32_t *d_qslots; unsigned long long *d_qcount; uint64_t q_cap;   // filter survivors (window planes, slots)
     uint32_t *d_hitmap;
     uint32_t *d_rid, *d_hcnt;     // group -> read, hits per read (list mode of the survivor kernel)
     // last submit
@@ -2388,7 +2430,7 @@ extern "C" void utb_batch_destroy(utb_batch *b) {
     cudaFree(b->d_name_off); cudaFree(b->d_name_len); cudaFree(b->d_line_len); cudaFree(b->d_line_off); cudaFree(b->d_scan_sums);
     cudaFree(b->d_text_len); cudaFree(b->d_text);
     cudaFree(b->d_raw); cudaFree(b->d_seq_off); cudaFree(b->d_seq_len); cudaFree(b->d_grp_off);
-    cudaFree(b->d_pk); cudaFree(b->d_bad); cudaFree(b->d_hits); cudaFree(b->d_results); cudaFree(b->d_pkr);
+    cudaFree(b->d_pk); cudaFree(b->d_bad); cudaFree(b->d_hits); cudaFree(b->d_results); cudaFree(b->d_pl);
     cudaFree(b->d_gen_list); cudaFree(b->d_gen_count); cudaFree(b->d_warp_list); cudaFree(b->d_warp_count); cudaFree(b->d_counters);
     vs_free(&b->vs);
     cudaFree(b->d_sel_cnt); cudaFree(b->d_sel_off); cudaFree(b->d_sel); cudaFree(b->d_sel_gap); cudaFree(b->d_sel_total);
@@ -2461,7 +2503,7 @@ extern "C" int utb_batch_create(utb_db *db, size_t max_bytes, size_t max_reads, 
         BK(cudaMemset(b->d_qslots, 0xFF, b->q_cap * 4));            // Q_INVALID
         BK(cudaMalloc(&b->d_qcount, 8));
         BK(cudaMalloc(&b->d_hitmap, (npos * 2 / 32 + 8) * 4));
-        BK(cudaMalloc(&b->d_pkr, (b->max_groups + PK_GUARD + 2) * 8));
+        BK(cudaMalloc(&b->d_pl, (b->max_groups + PK_GUARD + 2) * 8));
         BK(cudaMalloc(&b->d_rid, (b->max_groups + PK_GUARD + 2) * 4));
         BK(cudaMalloc(&b->d_hcnt, (max_reads + 1) * 4));
     }
@@ -2494,20 +2536,26 @@ static int launch_stages(utb_batch *b, bool timed) {
     const uint32_t nstr = b->do_rc ? 2u : 1u;
     CK(cudaMemsetAsync(b->d_gen_count, 0, 4, b->st));
     CK(cudaMemsetAsync(b->d_counters, 0, 4 * COUNTER_SLOTS * 8, b->st));
+    // sieve on while misses dominate (it only adds a fetch to lookups that hit)
+    const bool sieve = b->db->sieve && (b->db->sieve_mode == 1 || (b->db->sieve_mode == 2 && b->db->ema_hit_rate < 0.40));
+    const bool two_phase = b->db->use_table && sieve;              // the sieve kernel reads pl; everything else reads pk
     if (timed) CK(cudaEventRecord(b->ev[0], b->st));
     if (n_reads) {
-        pack_kernel<<<gs_grid(b, (uint64_t)n_groups + PK_GUARD, 256, 32), 256, 0, b->st>>>(b->d_raw, b->d_seq_off, b->d_seq_len, b->d_grp_off,
-                                                                   n_reads, n_groups, b->dims_dev, b->d_pk, b->d_bad, b->d_pkr, b->d_rid);
+        const unsigned grid = gs_grid(b, (uint64_t)n_groups + PK_GUARD, 256, 32);
+        if (!two_phase) pack_kernel<true, false><<<grid, 256, 0, b->st>>>(b->d_raw, b->d_seq_off, b->d_seq_len, b->d_grp_off,
+                                                                        n_reads, n_groups, b->dims_dev, b->d_pk, b->d_bad, nullptr, b->d_rid);
+        else if (b->out == UTB_OUT_SELECTIONS) pack_kernel<true, true><<<grid, 256, 0, b->st>>>(b->d_raw, b->d_seq_off, b->d_seq_len, b->d_grp_off,
+                                                                        n_reads, n_groups, b->dims_dev, b->d_pk, b->d_bad, b->d_pl, b->d_rid);
+        else pack_kernel<false, true><<<grid, 256, 0, b->st>>>(b->d_raw, b->d_seq_off, b->d_seq_len, b->d_grp_off,
+                                                             n_reads, n_groups, b->dims_dev, nullptr, b->d_bad, b->d_pl, b->d_rid);
         b->launches++;
     }
     if (timed) CK(cudaEventRecord(b->ev[1], b->st));
     if (n_pos) {
         const unsigned nb = (unsigned)(((uint64_t)n_pos * nstr + 255) / 256);
-        // sieve on while misses dominate (it only adds a fetch to lookups that hit)
-        const bool sieve = b->db->sieve && (b->db->sieve_mode == 1 || (b->db->sieve_mode == 2 && b->db->ema_hit_rate < 0.40));
         const unsigned sms = (unsigned)b->db->sm_count;
         b->used_sieve = sieve; b->used_lists = 0;
-        if (b->db->use_table && sieve) {
+        if (two_phase) {
             CK(cudaMemsetAsync(b->d_qcount, 0, 8, b->st));
             // hits are sparse (only sieve survivors that really match).  GG path: the survivor kernel files every label
             // under its read (list mode, see HitSink); non-GG path: by slot, flagged in a 1-bit-per-slot map
@@ -2521,15 +2569,16 @@ static int launch_stages(utb_batch *b, bool timed) {
             b->used_lists = lists;
             if (timed) CK(cudaEventRecord(b->ev[4], b->st));
             // persistent: MINB CTAs per SM, every warp a contiguous range of steps (small batches: one tile per warp)
-            // measured on B200, 10 M x 150 bp (profiles/r02_sieve_variants.txt): U = 6 steps per tile at 3 CTAs per SM (80
-            // registers) 8.54 ms; (5, 3) 8.60; (4, 3) 8.81; (4, 4) 8.98 (64 registers: 16 of them spilled); (3, 4) 9.22;
-            // (4, 5) 9.85; (2, 5) 10.5; (6, 2) 9.66; (8, 2) 9.88 -- instructions per step, not occupancy, decide
+            // measured on B200 (1000 W), 10 M x 150 bp, windows from bit planes (profiles/r03_bench_l2s_*): U = 6 steps per
+            // tile at 3 CTAs per SM (80 registers, no spills) 7.86 ms; (6, 4) 7.98 (64 registers, 88 B spilled); (8, 3)
+            // 8.03 (32 B spilled).  Before, from 2-bit words (r02_sieve_variants.txt): (6, 3) 8.54; (5, 3) 8.60; (4, 3)
+            // 8.81; (4, 4) 8.98; (6, 2) 9.66 -- instructions per step, not occupancy, decide
             constexpr unsigned U = 6, MINB = 3;
             const unsigned wb = (n_groups + 8u * U - 1) / (8u * U);
             const unsigned pb = wb < sms * MINB ? (wb ? wb : 1u) : sms * MINB;
             const uint32_t *sv_groups = b->dims_dev ? b->dims_dev + 1 : nullptr;
-            if (nstr == 2) sieve_kernel<2, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pk, b->d_bad, b->d_pkr, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
-            else sieve_kernel<1, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pk, b->d_bad, b->d_pkr, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
+            if (nstr == 2) sieve_kernel<2, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pl, b->d_bad, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
+            else sieve_kernel<1, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pl, b->d_bad, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
             if (timed) CK(cudaEventRecord(b->ev[5], b->st));
             if (lists) queue_lookup_kernel<true><<<sms * 6, 256, 0, b->st>>>(d, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink, b->d_counters);
             else queue_lookup_kernel<false><<<sms * 6, 256, 0, b->st>>>(d, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink, b->d_counters);
@@ -2979,7 +3028,7 @@ extern "C" int utb_pack_sequence(utb_db *db, const char *seq, uint32_t len, uint
     CK(cudaMemcpy(d_off, &off, 8, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_len, &len, 4, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(d_grp, grp, 8, cudaMemcpyHostToDevice));
-    pack_kernel<<<(n_groups + PK_GUARD + 255) / 256, 256>>>(d_raw, d_off, d_len, d_grp, 1, n_groups, nullptr, d_pk, d_bad, nullptr, nullptr);
+    pack_kernel<true, false><<<(n_groups + PK_GUARD + 255) / 256, 256>>>(d_raw, d_off, d_len, d_grp, 1, n_groups, nullptr, d_pk, d_bad, nullptr, nullptr);
     expand_windows_kernel<<<(n_pos + 255) / 256, 256>>>(d_pk, d_bad, n_pos, d_f, d_r, d_v);
     CK(cudaGetLastError());
     CK(cudaMemcpy(fwd, d_f, (size_t)len * 8, cudaMemcpyDeviceToHost));
