@@ -13,7 +13,8 @@
  *   XT_read32()            itree.c:733-828   utb_ctr_open + utb_db_upload
  *   readSamplesFPdelim()   itree.c:1202-1223 (inside utb_ctr_open)
  *   XT_doSearch32()        itree.c:833-1108  utb_search_file / utb_search_mem
- *     XT_INITIATE_WS       itree.c:860-901     framing kernels (exact host reader behind them)
+ *     XT_INITIATE_WS       itree.c:860-901     framing kernels (exact host reader behind them;
+ *                                              FASTQ: utb_searcher_set_input)
  *     XT_WORD_SEARCH       itree.c:903-933     pack + sieve kernels
  *     XT_getIX32/xtSuffixBS itree.c:699-730    table lookup kernel (or the probe sequence verbatim)
  *     full aufbau vote     itree.c:1028-1098   vote kernels
@@ -34,7 +35,7 @@ enum {
     UTB_OK = 0,
     UTB_ERR_ARG = 1,      /* bad argument                                     */
     UTB_ERR_IO = 2,       /* cannot open / short read                         */
-    UTB_ERR_FORMAT = 3,   /* malformed CTR or FASTA                           */
+    UTB_ERR_FORMAT = 3,   /* malformed CTR, FASTA or FASTQ                    */
     UTB_ERR_NOMEM = 4,
     UTB_ERR_CUDA = 5,     /* CUDA runtime error or no usable device           */
     UTB_ERR_LIMIT = 6     /* input exceeds a documented limit                 */
@@ -161,6 +162,21 @@ int utb_vote_hits_sparse(utb_db *db, const uint32_t *hits, const uint64_t *off,
 int utb_frame_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
                       uint64_t *seq_off, uint32_t *seq_len, uint32_t *name_off, uint32_t *name_len,
                       size_t *n_reads, size_t *used, int *ref_exit);
+/* The FASTQ twin of utb_frame_records (strict 4-line records, see
+ * utb_searcher_set_input): per read also the offset of its quality line,
+ * whose length equals seq_len.  On a malformed record the call returns
+ * UTB_ERR_FORMAT, the records before it are valid, *err_record is its
+ * 1-based number and *err_code one of UTB_FQ_*; otherwise both are 0. */
+enum {
+    UTB_FQ_NOHEADER = 1,     /* header line does not begin with '@'              */
+    UTB_FQ_NOSEPARATOR = 2,  /* third line does not begin with '+'               */
+    UTB_FQ_QUALLEN = 3,      /* quality length differs from sequence length      */
+    UTB_FQ_TOOLONG = 4,      /* a line of UTB_LINELEN (16777216) bytes or more   */
+    UTB_FQ_TRUNCATED = 5     /* the input ends inside a record                   */
+};
+int utb_frame_fastq_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
+                            uint64_t *seq_off, uint32_t *seq_len, uint64_t *qual_off, uint32_t *name_off, uint32_t *name_len,
+                            size_t *n_reads, size_t *used, size_t *err_record, int *err_code);
 /* The reference's output lines (itree.c:1032, 1040, 1096) for n_reads result
  * records; names are taken from bytes[name_off[r] .. +name_len[r]). */
 int utb_format_results(const utb_ctr *ctr, const char *bytes, const uint32_t *name_off, const uint32_t *name_len,
@@ -219,6 +235,36 @@ int utb_main(int argc, char **argv);
  * first search; utb_search_file / utb_search_mem then produce that output. */
 int utb_searcher_set_shallow(utb_searcher *s, int on);
 int utb_main_shallow(int argc, char **argv);
+
+/* ---- input format ----------------------------------------------------------- */
+/* utb_search_file / utb_search_mem read linearised FASTA (two lines per
+ * record) by default.  UTB_INPUT_FASTQ switches them to strict 4-line FASTQ:
+ *   header     begins with '@'; the name is the bytes after it up to the first
+ *              ' ' or the newline (a tab does not end it; with CRLF input a
+ *              '\r' stays in a name without a space, as for FASTA);
+ *   sequence   one trailing '\r' trimmed; a byte that is not ACGTacgt breaks
+ *              windows, as for FASTA;
+ *   separator  begins with '+'; the rest of the line is ignored;
+ *   quality    one trailing '\r' trimmed; its length must equal the sequence
+ *              length; its bytes are not otherwise checked.
+ * Every line is shorter than 16777216 bytes.  Wrapped (multi-line) FASTQ is a
+ * format error.  An empty sequence with an empty quality is a read without
+ * windows.  The last record may lack its final '\n' (not when its quality line
+ * is empty).  A NUL byte is an ordinary byte: it stays in a name and, in a
+ * sequence, breaks windows like any byte that is not a base (the FASTA reader
+ * instead cuts the name and the sequence line at a NUL, as the reference's
+ * strlen() does).  For input without NUL bytes the output is byte for byte
+ * that of the same search on the FASTA made of each record's header (with '>'
+ * for '@') and sequence line.  A
+ * malformed record is handled as for FASTA: every line of the records before
+ * it is written, the search returns UTB_ERR_FORMAT with *ref_exit = 2, and
+ * utb_last_error() names the 1-based record and the rule (UTB_FQ_*).
+ * min_qual = q > 0 (FASTQ only, q <= 222): a base whose quality byte is below
+ * 33 + q counts as 'N', so every window over it is skipped.  The caller's
+ * buffer is never modified.  Call before a search, like
+ * utb_searcher_set_shallow; memory the FASTQ path needs is allocated here. */
+enum { UTB_INPUT_FASTA = 0, UTB_INPUT_FASTQ = 1 };
+int utb_searcher_set_input(utb_searcher *s, int format, uint32_t min_qual);
 
 /* ---- utree-compress equivalent (XT_cmp32, itree.c:1234-1315; SURVEY 8f-2) -- */
 /* .ubt -> .ctr, byte-identical to the reference compressor (first-bin quirk

@@ -141,6 +141,21 @@ __device__ __forceinline__ uint64_t planes_to_word(uint64_t w) {   // perfect sh
     t = (w ^ (w >> 1)) & 0x2222222222222222ull; w ^= t ^ (t << 1);
     return w;
 }
+// The read that owns group g0 + lane, for a warp that takes the 32 groups from g0 on (warp-uniform call, g0 < the
+// batch's groups): the largest r with grp_off[r] <= g0 by one bisection per warp; every read owns >= 1 group, so the
+// reads of the other 31 groups start at one of the next 31 boundaries: a coalesced load of those, a warp-wide OR of
+// "a read starts at group g0 + j", and a population count give each lane its read
+__device__ __forceinline__ uint32_t group_read(const uint32_t *__restrict__ grp_off, uint32_t n_reads, uint32_t g0, uint32_t lane) {
+    uint32_t lo = 0, hi = n_reads;                                 // invariant: grp_off[lo] <= g0 < grp_off[hi]
+    while (hi - lo > 1) {
+        uint32_t mid = (lo + hi) >> 1;
+        if (__ldg(grp_off + mid) <= g0) lo = mid; else hi = mid;
+    }
+    const uint32_t nb = lo + 1u + lane;                            // boundary held by this lane
+    const uint32_t bnd = nb < n_reads ? __ldg(grp_off + nb) : 0xFFFFFFFFu;
+    const uint32_t starts = __reduce_or_sync(0xFFFFFFFFu, bnd - g0 < 32u ? 1u << (bnd - g0) : 0u);
+    return lo + __popc(starts & (0xFFFFFFFFu >> (31u - lane)));    // boundaries at groups g0 + 1 .. g0 + lane
+}
 #define PK_GUARD 8u               // all-bad groups behind the last read: the sieve kernel walks whole tiles without bounds checks
 // WORDS: write pk (the 2-bit words, read by the sieve-off lookup, the non-GG selection and expand_windows_kernel);
 // PLANES: write pl (the bit planes, read by the sieve kernel).  rid (optional): the read every group belongs to
@@ -155,22 +170,7 @@ pack_kernel(const uint8_t *__restrict__ raw, const uint64_t *__restrict__ seq_of
     // a warp takes 32 consecutive groups per round (warp-uniform loop)
     for (uint64_t gw = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) & ~31ull; gw < (uint64_t)n_groups + PK_GUARD; gw += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t g = (uint32_t)gw + lane;
-        // read owning the warp's first group: largest r with grp_off[r] <= g0 (one bisection per warp); every read owns
-        // >= 1 group, so the reads of the other 31 groups start at one of the next 31 boundaries: a coalesced load of
-        // those, a warp-wide OR of "a read starts at group g0 + j", and a population count give each lane its read
-        uint32_t lo = 0;
-        const uint32_t g0 = (uint32_t)gw;
-        if (g0 < n_groups) {
-            uint32_t hi = n_reads;                             // invariant: grp_off[lo] <= g0 < grp_off[hi]
-            while (hi - lo > 1) {
-                uint32_t mid = (lo + hi) >> 1;
-                if (__ldg(grp_off + mid) <= g0) lo = mid; else hi = mid;
-            }
-            const uint32_t nb = lo + 1u + lane;                // boundary held by this lane
-            const uint32_t bnd = nb < n_reads ? __ldg(grp_off + nb) : 0xFFFFFFFFu;
-            const uint32_t starts = __reduce_or_sync(0xFFFFFFFFu, bnd - g0 < 32u ? 1u << (bnd - g0) : 0u);
-            lo += __popc(starts & (0xFFFFFFFFu >> (31u - lane)));   // boundaries at groups g0 + 1 .. g0 + lane
-        }
+        const uint32_t lo = (uint32_t)gw < n_groups ? group_read(grp_off, n_reads, (uint32_t)gw, lane) : 0u;
         if (g >= n_groups + PK_GUARD) continue;
         if (g >= n_groups) {                                       // guard groups: all positions bad
             if (WORDS) pk[g] = 0;
@@ -1875,11 +1875,12 @@ nl_count_kernel(const uint8_t *__restrict__ raw, uint64_t n_bytes, uint32_t *__r
     __syncthreads();
     if (threadIdx.x == 0) { uint32_t t = 0; for (int w = 0; w < 8; ++w) t += sh[w]; blk_cnt[blockIdx.x] = t; }
 }
-// blk_off: exclusive scan of blk_cnt.  nl[i] = position of newline i, for i < limit.
+// blk_off: exclusive scan of blk_cnt.  nl[i] = position of newline i, for i < limit (LPR lines per record of dims[0]).
+template <uint32_t LPR>
 __global__ void __launch_bounds__(256)
 nl_index_kernel(const uint8_t *__restrict__ raw, uint64_t n_bytes, const uint32_t *__restrict__ blk_off,
                 uint32_t limit, const uint32_t *__restrict__ dims, uint32_t *__restrict__ nl) {
-    if (dims) limit = 2u * dims[0];
+    if (dims) limit = LPR * dims[0];
     __shared__ uint32_t sh[8];
     const uint64_t at = ((uint64_t)blockIdx.x * 256u + threadIdx.x) * FR_BPT;
     uint64_t m = nl_mask64(raw, at, n_bytes);
@@ -1927,12 +1928,78 @@ frame_parse_kernel(const uint8_t *__restrict__ raw, const uint32_t *__restrict__
 // its newline count is even; with that, no NUL byte (strlen() semantics, itree.c:887) and every record well formed
 // (frame_parse_kernel), the next chunk starts on a header line again -- by induction the framing equals the
 // reference's strictly pairwise fgets (itree.c:869-871).  Anything else is reported as record 0 / FRE_CHUNK and
-// the host re-reads from this chunk on with its exact reader.
+// the host re-reads from this chunk on with its exact reader.  LPR: lines per record, 2 for FASTA; 4 for FASTQ,
+// where the same induction holds with "a multiple of 4" (the cut rule is argued in pipeline.c, fastq_cut).
+template <uint32_t LPR>
 __global__ void frame_setup_kernel(const uint32_t *__restrict__ info, uint32_t max_reads, uint32_t *__restrict__ dims, uint32_t *__restrict__ err) {
     const uint32_t n_lines = info[0], nul = info[1];
-    const bool bad = nul || (n_lines & 1u) || !n_lines || (n_lines >> 1) > max_reads;
-    dims[0] = bad ? 0u : n_lines >> 1;
+    const bool bad = nul || (n_lines % LPR) || !n_lines || (n_lines / LPR) > max_reads;
+    dims[0] = bad ? 0u : n_lines / LPR;
     if (bad) atomicMin(err, (uint32_t)FRE_CHUNK);
+}
+// One thread per FASTQ record r: lines 4r .. 4r+3 are its header, sequence, separator and quality line, line i
+// being (nl[i-1], nl[i]].  The rules, and the order in which they are checked, are the host framer's
+// (pipeline.c, fq_record): the host re-frames a flagged chunk and reports the error itself.
+__global__ void __launch_bounds__(256)
+frame_parse_fastq_kernel(const uint8_t *__restrict__ raw, const uint32_t *__restrict__ nl, uint32_t n_reads, const uint32_t *__restrict__ dims,
+                         uint64_t *__restrict__ seq_off, uint32_t *__restrict__ seq_len, uint64_t *__restrict__ qual_off,
+                         uint32_t *__restrict__ name_off, uint32_t *__restrict__ name_len,
+                         uint32_t *__restrict__ slots, uint32_t *__restrict__ err) {
+    if (dims) n_reads = dims[0];
+    for (uint64_t r64 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r64 < n_reads; r64 += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t r = (uint32_t)r64;
+        const uint32_t hs = r ? nl[4 * r - 1] + 1u : 0u, hn = nl[4 * r], ss = hn + 1u, sn = nl[4 * r + 1];
+        const uint32_t ps = sn + 1u, pn = nl[4 * r + 2], qs = pn + 1u, qn = nl[4 * r + 3];
+        uint32_t length = sn - ss, qlength = qn - qs;
+        if (length && raw[ss + length - 1] == '\r') --length;
+        if (qlength && raw[qs + qlength - 1] == '\r') --qlength;
+        uint32_t code = 0;
+        if (hn + 1u - hs >= UTB_LINELEN || sn + 1u - ss >= UTB_LINELEN || pn + 1u - ps >= UTB_LINELEN || qn + 1u - qs >= UTB_LINELEN)
+            code = UTB_FQ_TOOLONG;
+        else if (raw[hs] != '@') code = UTB_FQ_NOHEADER;
+        else if (raw[ps] != '+') code = UTB_FQ_NOSEPARATOR;
+        else if (qlength != length) code = UTB_FQ_QUALLEN;
+        if (code) { atomicMin(err, (r << 3) | code); length = 0; } // a flagged record gets no bases: its quality line may be
+                                                                   // shorter, and qual_mask_kernel reads seq_len quality bytes
+        uint32_t e = hs + 1u;                                      // name: up to the first ' ' or the newline, as for FASTA
+        while (e < hn && raw[e] != ' ') ++e;
+        seq_off[r] = ss; seq_len[r] = length; qual_off[r] = qs;
+        name_off[r] = hs + 1u; name_len[r] = e - hs - 1u;
+        slots[r] = (length + 1u + 31u) / 32u;                      // utb_read_slots
+    }
+}
+// Quality masking (FASTQ with min_qual > 0): every base whose quality byte is below 33 + min_qual becomes 'N' in
+// the device copy of the input, so pack_kernel marks it bad and the slide skips every window over it, as it does
+// for any byte that is not a base (itree.c:919-926).  One thread per 32-base group with pack_kernel's group -> read
+// mapping: a read is spread over as many threads as it has groups, however long it is.  thr4: 33 + min_qual in
+// every byte.  Only sequence bytes are written, and quality bytes are only read.
+__global__ void __launch_bounds__(256)
+qual_mask_kernel(uint8_t *raw, const uint64_t *__restrict__ seq_off, const uint64_t *__restrict__ qual_off,
+                 const uint32_t *__restrict__ seq_len, const uint32_t *__restrict__ grp_off,
+                 uint32_t n_reads, uint32_t n_groups, const uint32_t *__restrict__ dims, uint32_t thr4) {
+    if (dims) { n_reads = dims[0]; n_groups = dims[1]; }
+    const uint32_t lane = threadIdx.x & 31u;
+    for (uint64_t gw = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) & ~31ull; gw < n_groups; gw += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t g = (uint32_t)gw + lane;
+        const uint32_t lo = group_read(grp_off, n_reads, (uint32_t)gw, lane);
+        if (g >= n_groups) continue;
+        const uint32_t b0 = (g - __ldg(grp_off + lo)) * 32u, len = __ldg(seq_len + lo);
+        const uint32_t nv = len > b0 ? min(32u, len - b0) : 0u;    // real bases in this group
+        if (!nv) continue;
+        const uint64_t a = __ldg(qual_off + lo) + b0;
+        const uint32_t *p = reinterpret_cast<const uint32_t *>(raw + (a & ~3ull));
+        const uint32_t sh = (uint32_t)(a & 3u) * 8u, nw = (nv + 3u) >> 2;
+        uint32_t prev = p[0], m = 0;
+        for (uint32_t j = 0; j < nw; ++j) {
+            const uint32_t cur = p[j + 1];
+            const uint32_t lt = __vcmpltu4(__funnelshift_r(prev, cur, sh), thr4) & 0x01010101u;
+            m |= ((lt * 0x01020408u) >> 24) << (4u * j);           // bit i: base b0 + i is masked
+            prev = cur;
+        }
+        if (nv < 32u) m &= (1u << nv) - 1u;
+        uint8_t *s = raw + __ldg(seq_off + lo) + b0;
+        for (; m; m &= m - 1u) s[__ffs(m) - 1] = 'N';
+    }
 }
 
 #define FW_WARPS 8
@@ -2410,6 +2477,10 @@ struct utb_batch {
     uint32_t *d_nl, *d_blk, *d_frame_err, *h_frame_err; int framed_on_device;
     uint32_t *d_frame_info;                                        // [0] newlines of the chunk, [1] NUL seen
     uint32_t *d_dims, *h_dims; const uint32_t *dims_dev;           // [0] records, [1] position groups of the batch as the device derived them
+    size_t nl_cap;                                                 // entries of d_nl
+    // FASTQ input (utb_batch_set_input): per read the offset of its quality line; min_qual > 0 masks low-quality bases
+    int fastq; uint32_t min_qual;
+    uint64_t *h_qual_off, *d_qual_off;
 };
 
 extern "C" uint64_t utb_read_slots(uint32_t len) { return ((uint64_t)len + 1 + 31) / 32; }
@@ -2438,6 +2509,7 @@ extern "C" void utb_batch_destroy(utb_batch *b) {
     cudaFree(b->d_qwords); cudaFree(b->d_qslots); cudaFree(b->d_qcount); cudaFree(b->d_hitmap); cudaFree(b->d_rid); cudaFree(b->d_hcnt);
     cudaFree(b->d_nl); cudaFree(b->d_blk); cudaFree(b->d_frame_err); cudaFreeHost(b->h_frame_err);
     cudaFree(b->d_frame_info); cudaFree(b->d_dims); cudaFreeHost(b->h_dims);
+    cudaFreeHost(b->h_qual_off); cudaFree(b->d_qual_off);
     if (b->done) cudaEventDestroy(b->done);
     for (int i = 0; i < 7; ++i) if (b->ev[i]) cudaEventDestroy(b->ev[i]);
     if (b->st) cudaStreamDestroy(b->st);
@@ -2685,6 +2757,16 @@ extern "C" void utb_pinned_free(void *p) { if (p) cudaFreeHost(p); }
 extern "C" uint32_t *utb_batch_name_off(utb_batch *b) { return b->h_name_off; }
 extern "C" uint32_t *utb_batch_name_len(utb_batch *b) { return b->h_name_len; }
 
+// FASTQ with min_qual > 0: low-quality bases of the device copy become 'N' (after grp_off, before pack_kernel)
+static int launch_mask(utb_batch *b) {
+    const uint32_t thr = 33u + b->min_qual;
+    qual_mask_kernel<<<gs_grid(b, (uint64_t)b->n_groups, 256, 32), 256, 0, b->st>>>(
+        b->d_raw, b->d_seq_off, b->d_qual_off, b->d_seq_len, b->d_grp_off, (uint32_t)b->n_reads, b->n_groups, b->dims_dev, thr * 0x01010101u);
+    b->launches++;
+    CK(cudaGetLastError());
+    return UTB_OK;
+}
+
 static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out, uint64_t total_groups) {
     if (!b) { utb_set_error("utb_batch_submit: null batch"); return UTB_ERR_ARG; }
     if (n_bytes > b->max_bytes || n_reads > b->max_reads) { utb_set_error("utb_batch_submit: batch over capacity"); return UTB_ERR_LIMIT; }
@@ -2729,6 +2811,11 @@ static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_r
             scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_text_len);
             scan_apply_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, nullptr, nt, b->d_scan_sums, b->d_grp_off);
             b->launches += 4;
+        }
+        if (b->fastq && b->min_qual) {
+            CK(cudaMemcpyAsync(b->d_qual_off, b->h_qual_off, n_reads * 8, cudaMemcpyHostToDevice, b->st));
+            int rm = launch_mask(b);
+            if (rm) return rm;
         }
     }
     return finish_submit(b);
@@ -2780,9 +2867,16 @@ static int finish_submit(utb_batch *b) {
 // utb_batch_frame_error() tells after the wait whether the chunk or one of its records was malformed,
 // utb_batch_reads() how many records it held.
 static int ensure_chunk_buffers(utb_batch *b) {
+    const size_t nl_cap = (b->fastq ? 4 : 2) * b->max_reads + 2;  // lines per record
+    if (b->d_nl && b->nl_cap < nl_cap) {                           // a FASTQ batch: grown once, by utb_batch_set_input
+        void *q = nullptr;
+        CK(cudaMalloc(&q, nl_cap * 4));
+        cudaFree(b->d_nl);
+        b->d_nl = (uint32_t *)q; b->nl_cap = nl_cap;
+    }
     if (b->d_nl) return UTB_OK;
     void *p[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    cudaError_t e = cudaMalloc(&p[0], (2 * b->max_reads + 2) * 4);
+    cudaError_t e = cudaMalloc(&p[0], nl_cap * 4);
     if (e == cudaSuccess) e = cudaMalloc(&p[1], (b->max_bytes / FR_BLOCK + 2) * 4);
     if (e == cudaSuccess) e = cudaMalloc(&p[2], 4);
     if (e == cudaSuccess) e = cudaMalloc(&p[3], 8);
@@ -2790,6 +2884,7 @@ static int ensure_chunk_buffers(utb_batch *b) {
     if (e != cudaSuccess) { for (int i = 0; i < 4; ++i) cudaFree(p[i]); cudaFreeHost(p[4]); CK(e); }
     b->d_nl = (uint32_t *)p[0]; b->d_blk = (uint32_t *)p[1]; b->d_frame_err = (uint32_t *)p[2]; b->d_frame_info = (uint32_t *)p[3];
     b->h_frame_err = (uint32_t *)p[4];
+    b->nl_cap = nl_cap;
     return UTB_OK;
 }
 static int ensure_shallow_buffers(utb_batch *b) {
@@ -2815,6 +2910,25 @@ extern "C" int utb_batch_prepare(utb_batch *b, utb_batch_out out, int chunked) {
     if (!rc && chunked) rc = ensure_chunk_buffers(b);
     return rc;
 }
+// The input format of the batch's later submits (FASTA, or FASTQ with min_qual); allocates what FASTQ needs.
+extern "C" int utb_batch_set_input(utb_batch *b, int fastq, uint32_t min_qual, int chunked) {
+    if (!b || (!fastq && min_qual) || min_qual > 222) { utb_set_error("utb_batch_set_input: bad argument"); return UTB_ERR_ARG; }
+    CK(cudaSetDevice(b->db->device));
+    if (fastq && !b->h_qual_off) {                                 // both arrays or neither
+        void *h = nullptr, *d = nullptr;
+        cudaError_t e = cudaMallocHost(&h, b->max_reads * 8);
+        if (e == cudaSuccess) e = cudaMalloc(&d, b->max_reads * 8);
+        if (e != cudaSuccess) { cudaFreeHost(h); cudaFree(d); CK(e); }
+        b->h_qual_off = (uint64_t *)h; b->d_qual_off = (uint64_t *)d;
+    }
+    const int old_fastq = b->fastq;
+    b->fastq = fastq ? 1 : 0;                                      // ensure_chunk_buffers sizes the newline index by it
+    const int rc = chunked ? ensure_chunk_buffers(b) : UTB_OK;     // keeps the old index if the larger one cannot be had
+    if (rc) { b->fastq = old_fastq; return rc; }
+    b->min_qual = min_qual;
+    return UTB_OK;
+}
+extern "C" uint64_t *utb_batch_qual_off(utb_batch *b) { return b->h_qual_off; }
 extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out) {
     if (!b || !n_bytes || out == UTB_OUT_RESULTS) { utb_set_error("utb_batch_submit_chunk: bad argument"); return UTB_ERR_ARG; }
     if (n_bytes > b->max_bytes || n_reads > b->max_reads || n_bytes >= 0xFFFFFFFFull) { utb_set_error("utb_batch_submit_chunk: batch over capacity"); return UTB_ERR_LIMIT; }
@@ -2836,16 +2950,24 @@ extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_by
     const uint32_t fb = (uint32_t)((n_bytes + FR_BLOCK - 1) / FR_BLOCK), n = (uint32_t)n_ub, nt = (n + SCAN_TILE - 1) / SCAN_TILE;
     nl_count_kernel<<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, b->d_frame_info + 1);
     scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_blk, fb, b->d_frame_info);       // block counts -> exclusive offsets, total newlines
-    frame_setup_kernel<<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
-    nl_index_kernel<<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, 0, b->d_dims, b->d_nl);
-    frame_parse_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, b->d_nl, n, b->d_dims, b->d_seq_off, b->d_seq_len, b->d_name_off,
-                                                                  b->d_name_len, b->d_line_len, b->d_frame_err);
+    if (b->fastq) {
+        frame_setup_kernel<4><<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
+        nl_index_kernel<4><<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, 0, b->d_dims, b->d_nl);
+        frame_parse_fastq_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, b->d_nl, n, b->d_dims, b->d_seq_off, b->d_seq_len,
+                                                                            b->d_qual_off, b->d_name_off, b->d_name_len, b->d_line_len, b->d_frame_err);
+    } else {
+        frame_setup_kernel<2><<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
+        nl_index_kernel<2><<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, 0, b->d_dims, b->d_nl);
+        frame_parse_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, b->d_nl, n, b->d_dims, b->d_seq_off, b->d_seq_len, b->d_name_off,
+                                                                      b->d_name_len, b->d_line_len, b->d_frame_err);
+    }
     // grp_off = exclusive scan of the per-read group counts; the total (dims[1]) stays on the device
     scan_sums_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->d_dims, nt, b->d_scan_sums);
     scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_dims + 1);
     scan_apply_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->d_dims, nt, b->d_scan_sums, b->d_grp_off);
     b->launches += 8;
     CK(cudaGetLastError());
+    if (b->fastq && b->min_qual) { int rm = launch_mask(b); if (rm) return rm; }
     CK(cudaMemcpyAsync(b->h_frame_err, b->d_frame_err, 4, cudaMemcpyDeviceToHost, b->st));
     return finish_submit(b);
 }

@@ -39,6 +39,7 @@
 #define DEFAULT_BATCH_BYTES ((size_t)128 << 20)   /* ~2.3 ms of PCIe per batch: launch and sync costs are a few percent of that */
 #define RAMP_BYTES ((size_t)32 << 20)              /* first / last batches: small, so the pipeline fills and drains fast */
 #define MAX_TEAM 64
+#define MAX_RECORD(lines) ((lines) * (size_t)UTB_LINELEN + 4096)   /* a record of maximal lines, and slack */
 
 /* ---- thread team: leader + helpers, fork/join with barriers ----------------- */
 typedef void (*team_fn)(void *ctx, int part, int nparts);
@@ -124,6 +125,8 @@ struct utb_searcher {
     char *arena; size_t arena_cap; /* page-locked output of utb_search_mem: the devices copy their text straight into it; valid until
                                     * the next search on this searcher or its destruction */
     int spread;                    /* more than one physical GPU: page-locked buffers are interleaved over the NUMA nodes */
+    int fastq;                     /* input is 4-line FASTQ (utb_searcher_set_input) */
+    uint32_t min_qual;             /* FASTQ: bases with a quality byte below 33 + min_qual count as 'N' (0: off) */
 };
 
 static double now_s(void) {
@@ -158,6 +161,38 @@ static void mem_interleave(int on) {
 #endif
 }
 
+/* the output lines of a batch are built on the device: long labels take fewer reads per batch */
+static size_t batch_reads_for(utb_searcher *s) {
+    s->batch_reads = utb_text_max_reads(s->batch_bytes, s->batch_bytes / 64, s->max_label);
+    return s->batch_reads;
+}
+/* (Re)creates the batches of every slot with s->batch_bytes, prepared for the searcher's mode: nothing is allocated
+ * inside a search.  All or nothing: the new batches replace the old ones only when every one of them could be made. */
+static int slots_create(utb_searcher *s) {
+    utb_batch **nb = (utb_batch **)calloc((size_t)s->n_slots, sizeof(utb_batch *));
+    if (!nb) { utb_set_error("out of memory"); return UTB_ERR_NOMEM; }
+    int rc = UTB_OK;
+    for (int i = 0; i < s->n_slots && !rc; ++i) {
+        if (s->spread) mem_interleave(1);
+        rc = utb_batch_create(s->dbs[i % s->n_devices], s->batch_bytes, s->batch_reads, &nb[i]);
+        if (!rc) rc = utb_batch_prepare(nb[i], UTB_OUT_TEXT, s->device_frame);
+        if (!rc && s->shallow) rc = utb_batch_prepare(nb[i], UTB_OUT_SELECTIONS, s->device_frame);
+        if (!rc && s->fastq) rc = utb_batch_set_input(nb[i], 1, s->min_qual, s->device_frame);
+        if (s->spread) mem_interleave(0);
+    }
+    for (int i = 0; i < s->n_slots; ++i) {
+        slot_t *sl = &s->slots[i];
+        if (rc) { utb_batch_destroy(nb[i]); continue; }
+        utb_batch_destroy(sl->b);
+        sl->b = nb[i];
+        sl->dev_index = i % s->n_devices;
+        sl->name_off = utb_batch_name_off(sl->b);                  /* pinned: the device formatter reads them too */
+        sl->name_len = utb_batch_name_len(sl->b);
+    }
+    free(nb);
+    return rc;
+}
+
 int utb_searcher_create(const utb_ctr *ctr, const int *devices, int n_devices,
                         int host_threads, utb_searcher **out) {
     if (!ctr || !out || n_devices < 1 || !devices) { utb_set_error("utb_searcher_create: bad argument"); return UTB_ERR_ARG; }
@@ -167,16 +202,14 @@ int utb_searcher_create(const utb_ctr *ctr, const int *devices, int n_devices,
     s->ctr = ctr; s->n_devices = n_devices; s->host_threads = host_threads < 1 ? 1 : host_threads;
     const char *e = getenv("UTB_BATCH_MB");
     s->batch_bytes = e && atoi(e) > 0 ? (size_t)atoi(e) << 20 : DEFAULT_BATCH_BYTES;
-    if (s->batch_bytes < 2 * (size_t)UTB_LINELEN + 4096) s->batch_bytes = 2 * (size_t)UTB_LINELEN + 4096; /* one max record must fit */
+    if (s->batch_bytes < MAX_RECORD(2)) s->batch_bytes = MAX_RECORD(2);   /* one max record must fit */
     e = getenv("UTB_HOST_FRAME");
     s->device_frame = !(e && atoi(e) != 0);
     for (uint32_t i = 0; i < ctr->max_ix; ++i) {
         size_t l = ctr->off[i + 1] - ctr->off[i];
         if (l > s->max_label) s->max_label = l;
     }
-    /* the output lines of a batch are built on the device: long labels take fewer reads per batch */
-    s->batch_reads = utb_text_max_reads(s->batch_bytes, s->batch_bytes / 64, s->max_label);
-    if (!s->batch_reads) { free(s); utb_set_error("batch too large for device-side formatting"); return UTB_ERR_LIMIT; }
+    if (!batch_reads_for(s)) { free(s); utb_set_error("batch too large for device-side formatting"); return UTB_ERR_LIMIT; }
     s->devices = (int *)malloc(sizeof(int) * (size_t)n_devices);
     s->dbs = (utb_db **)calloc((size_t)n_devices, sizeof(utb_db *));
     e = getenv("UTB_SLOTS");                                       /* stream slots per device (tuning) */
@@ -199,17 +232,8 @@ int utb_searcher_create(const utb_ctr *ctr, const int *devices, int n_devices,
         else rc = utb_db_clone(s->dbs[0], devices[d], &s->dbs[d]);
         if (rc) { s->n_devices = d; utb_searcher_destroy(s); return rc; }
     }
-    for (int i = 0; i < s->n_slots; ++i) {
-        slot_t *sl = &s->slots[i];
-        sl->dev_index = i % n_devices;
-        if (s->spread) mem_interleave(1);
-        int rc = utb_batch_create(s->dbs[sl->dev_index], s->batch_bytes, s->batch_reads, &sl->b);
-        if (!rc) rc = utb_batch_prepare(sl->b, UTB_OUT_TEXT, s->device_frame);   /* nothing is allocated inside a search */
-        if (s->spread) mem_interleave(0);
-        if (rc) { utb_searcher_destroy(s); return rc; }
-        sl->name_off = utb_batch_name_off(sl->b);                  /* pinned: the device formatter reads them too */
-        sl->name_len = utb_batch_name_len(sl->b);
-    }
+    int rc = slots_create(s);
+    if (rc) { utb_searcher_destroy(s); return rc; }
     *out = s;
     return UTB_OK;
 }
@@ -228,6 +252,36 @@ int utb_searcher_set_shallow(utb_searcher *s, int on) {
         int rc = utb_batch_prepare(s->slots[i].b, UTB_OUT_SELECTIONS, s->device_frame);
         if (rc) return rc;
     }
+    return UTB_OK;
+}
+
+int utb_searcher_set_input(utb_searcher *s, int format, uint32_t min_qual) {
+    if (!s || (format != UTB_INPUT_FASTA && format != UTB_INPUT_FASTQ) || (format == UTB_INPUT_FASTA && min_qual) || min_qual > 222) {
+        utb_set_error("utb_searcher_set_input: bad argument (format %d, min_qual %u)", format, min_qual);
+        return UTB_ERR_ARG;
+    }
+    const int fastq = format == UTB_INPUT_FASTQ;
+    /* on failure the searcher keeps its batches and its format */
+    const int old_fastq = s->fastq;
+    const uint32_t old_qual = s->min_qual;
+    if (fastq && s->batch_bytes < MAX_RECORD(4)) {                 /* a batch must hold one record of four maximal lines */
+        const size_t keep = s->batch_bytes;
+        s->batch_bytes = MAX_RECORD(4);
+        int rc = batch_reads_for(s) ? UTB_OK : UTB_ERR_LIMIT;
+        if (rc) utb_set_error("batch too large for device-side formatting");
+        s->fastq = fastq; s->min_qual = min_qual;
+        if (!rc) rc = slots_create(s);
+        if (rc) { s->batch_bytes = keep; batch_reads_for(s); s->fastq = old_fastq; s->min_qual = old_qual; }
+        return rc;
+    }
+    for (int i = 0; i < s->n_slots; ++i) {
+        int rc = utb_batch_set_input(s->slots[i].b, fastq, min_qual, s->device_frame);
+        if (rc) {                                                  /* back to the old format: allocates nothing */
+            for (int j = 0; j < i; ++j) (void)utb_batch_set_input(s->slots[j].b, old_fastq, old_qual, s->device_frame);
+            return rc;
+        }
+    }
+    s->fastq = fastq; s->min_qual = min_qual;
     return UTB_OK;
 }
 
@@ -601,6 +655,7 @@ enum { FE_NONE = 0, FE_NOHEADER, FE_SEQ_GT, FE_EMPTY, FE_TOOLONG };
 typedef struct {
     const char *buf; size_t fill; int eof;
     uint64_t *seq_off; uint32_t *seq_len; uint32_t *name_off, *name_len;
+    uint64_t *qual_off;            /* FASTQ */
     size_t cnt[MAX_TEAM];          /* newlines per segment */
     size_t base[MAX_TEAM];         /* newlines before the segment */
     size_t n_rec;                  /* complete records in the buffer (clamped to max_rec) */
@@ -832,6 +887,96 @@ static void frame_buffer(team_t *team, frame_ctx *F, size_t *n_out, size_t *n_co
     *n_out = n; *n_complete = F->n_rec; *used = F->end_of_records;
 }
 
+/* ---- FASTQ framer ------------------------------------------------------------------------------ */
+/* Strict 4-line records: line 4r is the header of record r, 4r+1 its sequence, 4r+2 the separator, 4r+3 the
+ * quality, whatever they contain.  As for FASTA a line's role follows from its index: count_part counts the
+ * newlines per segment, then every worker parses the records whose header line starts right after a newline of
+ * its own segment.  The rules and their order are those of frame_parse_fastq_kernel, so a chunk the device
+ * flagged is re-framed here with the same verdict. */
+static inline size_t fq_line(const frame_ctx *c, size_t s, size_t *end) {   /* start of the next line; *end: the '\n' or fill */
+    const char *q = s < c->fill ? (const char *)memchr(c->buf + s, '\n', c->fill - s) : NULL;
+    *end = q ? (size_t)(q - c->buf) : c->fill;
+    return q ? *end + 1 : c->fill;
+}
+/* Parses record r whose header line starts at hs; returns the byte after its quality line. */
+static size_t fq_record(frame_ctx *c, size_t r, size_t hs, int *err) {
+    const char *buf = c->buf;
+    size_t hn, sn, pn, qn;
+    const size_t ss = fq_line(c, hs, &hn), ps = fq_line(c, ss, &sn), qs = fq_line(c, ps, &pn), next = fq_line(c, qs, &qn);
+    size_t length = sn - ss, qlength = qn - qs;
+    if (length && buf[ss + length - 1] == '\r') --length;
+    if (qlength && buf[qs + qlength - 1] == '\r') --qlength;
+    *err = FE_NONE;
+    if (ss - hs >= UTB_LINELEN || ps - ss >= UTB_LINELEN || qs - ps >= UTB_LINELEN || next - qs >= UTB_LINELEN) *err = UTB_FQ_TOOLONG;
+    else if (buf[hs] != '@') *err = UTB_FQ_NOHEADER;
+    else if (buf[ps] != '+') *err = UTB_FQ_NOSEPARATOR;
+    else if (qlength != length) *err = UTB_FQ_QUALLEN;
+    if (*err) return next;
+    size_t e = hs + 1;                                             /* name: up to the first ' ' or the newline, as for FASTA */
+    while (e < hn && buf[e] != ' ') ++e;
+    c->name_off[r] = (uint32_t)(hs + 1);
+    c->name_len[r] = (uint32_t)(e - hs - 1);
+    c->seq_off[r] = ss; c->seq_len[r] = (uint32_t)length; c->qual_off[r] = qs;
+    return next;
+}
+static void fq_part(void *c_, int part, int nparts) {
+    frame_ctx *c = (frame_ctx *)c_;
+    size_t a = c->fill * (size_t)part / (size_t)nparts, b = c->fill * (size_t)(part + 1) / (size_t)nparts;
+    c->err_rec[part] = (size_t)-1; c->err_code[part] = FE_NONE; c->groups[part] = 0;
+    size_t s, L;                                                   /* first line start owned by this segment, and its index */
+    if (part == 0) { s = 0; L = 0; }
+    else {
+        const char *q = a < b ? (const char *)memchr(c->buf + a, '\n', b - a) : NULL;
+        if (!q) return;
+        s = (size_t)(q - c->buf) + 1; L = c->base[part] + 1;
+    }
+    while (L & 3) {                                                /* not a header line: its record belongs to an earlier segment */
+        const char *q = s < b ? (const char *)memchr(c->buf + s, '\n', b - s) : NULL;
+        if (!q) return;
+        s = (size_t)(q - c->buf) + 1; ++L;
+    }
+    uint64_t groups = 0;
+    for (size_t r = L >> 2; r < c->n_rec; ++r) {
+        int err;
+        const size_t next = fq_record(c, r, s, &err);
+        if (err) { c->err_rec[part] = r; c->err_code[part] = err; break; }
+        groups += utb_read_slots(c->seq_len[r]);
+        if (r == c->n_rec - 1) c->end_of_records = next;
+        if (next > b || c->buf[next - 1] != '\n') break;          /* the next header is ours iff this record's last newline is in [a, b) */
+        s = next;
+    }
+    c->groups[part] = groups;
+}
+static const char *fq_text(int code) {
+    switch (code) {
+    case UTB_FQ_NOHEADER: return "ERROR: FASTQ header line does not begin with '@'";
+    case UTB_FQ_NOSEPARATOR: return "ERROR: FASTQ separator line does not begin with '+'";
+    case UTB_FQ_QUALLEN: return "ERROR: FASTQ quality length differs from the sequence length";
+    case UTB_FQ_TRUNCATED: return "ERROR: truncated FASTQ record";
+    default: return "ERROR: line longer than the reference reader's 16777215-byte limit";
+    }
+}
+/* Frames buf[0..fill) as FASTQ: on return *n_out records are valid (those before the first malformed one), *used
+ * is the byte after the last complete record, *err is UTB_FQ_* of the record at index *n_out (or FE_NONE); an input
+ * that ends inside a record is UTB_FQ_TRUNCATED at index *n_complete. */
+static void fq_buffer(team_t *team, frame_ctx *F, size_t *n_out, size_t *n_complete, size_t *used, int *err) {
+    team_run(team, count_part, F);
+    size_t nl_total = 0;
+    for (int p = 0; p < team->n; ++p) { F->base[p] = nl_total; nl_total += F->cnt[p]; }
+    const size_t n_lines = nl_total + ((F->eof && F->fill && F->buf[F->fill - 1] != '\n') ? 1 : 0);   /* a last line without '\n' counts at EOF */
+    F->n_rec = n_lines / 4;
+    int truncated = F->eof && (n_lines & 3);
+    if (F->n_rec > F->max_rec) { F->n_rec = F->max_rec; truncated = 0; }   /* the rest comes back with the carry */
+    F->end_of_records = 0;
+    for (int p = 0; p < team->n; ++p) { F->err_rec[p] = (size_t)-1; F->err_code[p] = FE_NONE; F->groups[p] = 0; }
+    if (F->n_rec) team_run(team, fq_part, F);
+    size_t n = F->n_rec; *err = FE_NONE;
+    for (int p = 0; p < team->n; ++p) if (F->err_rec[p] < n) { n = F->err_rec[p]; *err = F->err_code[p]; }
+    if (!*err && truncated) *err = UTB_FQ_TRUNCATED;
+    F->groups_valid = n == F->n_rec;                               /* per-worker sums cover exactly the framed records */
+    *n_out = n; *n_complete = F->n_rec; *used = F->end_of_records;
+}
+
 /* Host-stage entry points (CPU-only tests drive the framer and the formatter through these). */
 int utb_frame_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
                       uint64_t *seq_off, uint32_t *seq_len, uint32_t *name_off, uint32_t *name_len,
@@ -858,6 +1003,33 @@ int utb_frame_records(const char *buf, size_t n, int eof, int threads, size_t ma
     return UTB_OK;
 }
 
+int utb_frame_fastq_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
+                            uint64_t *seq_off, uint32_t *seq_len, uint64_t *qual_off, uint32_t *name_off, uint32_t *name_len,
+                            size_t *n_reads, size_t *used, size_t *err_record, int *err_code) {
+    if ((!buf && n) || !seq_off || !seq_len || !qual_off || !name_off || !name_len || !n_reads || !used) {
+        utb_set_error("utb_frame_fastq_records: null argument"); return UTB_ERR_ARG;
+    }
+    *n_reads = 0; *used = 0;
+    if (err_record) *err_record = 0;
+    if (err_code) *err_code = 0;
+    if (!n) return UTB_OK;
+    team_t team;
+    if (team_init(&team, threads)) { utb_set_error("cannot start worker threads"); return UTB_ERR_NOMEM; }
+    frame_ctx F;
+    memset(&F, 0, sizeof F);
+    F.buf = buf; F.fill = n; F.eof = eof; F.max_rec = max_reads;
+    F.seq_off = seq_off; F.seq_len = seq_len; F.qual_off = qual_off; F.name_off = name_off; F.name_len = name_len;
+    size_t nr, nc, u; int err;
+    fq_buffer(&team, &F, &nr, &nc, &u, &err);
+    team_destroy(&team);
+    *n_reads = nr; *used = u;
+    if (!err) return UTB_OK;
+    if (err_record) *err_record = nr + 1;
+    if (err_code) *err_code = err;
+    utb_set_error("%s [record %zu]", fq_text(err), nr + 1);
+    return UTB_ERR_FORMAT;
+}
+
 int utb_format_results(const utb_ctr *ctr, const char *bytes, const uint32_t *name_off, const uint32_t *name_len,
                        const utb_result *results, size_t n_reads, char *out, size_t out_cap, size_t *out_len) {
     if (!ctr || !bytes || !name_off || !name_len || !results || !out || !out_len) { utb_set_error("utb_format_results: null argument"); return UTB_ERR_ARG; }
@@ -873,6 +1045,27 @@ int utb_format_results(const utb_ctr *ctr, const char *bytes, const uint32_t *na
     *out_len = len;
     free(buf);
     return rc;
+}
+
+/* Where the device fast path cuts a FASTQ chunk: right before the last line L that begins with '@' and whose line
+ * L+2 begins with '+' (0: none).  In well-formed input the header lines pass.  A quality line that begins with '@'
+ * fails, because its line L+2 is the next record's sequence line (unless that begins with '+').  The cut is only a
+ * guess: by induction the chunk starts on a header line, so a cut before a line whose index is not a multiple of 4
+ * leaves a line count that is not one either; frame_setup_kernel<4> rejects such a chunk (FRE_CHUNK) and the
+ * reader rewinds to it with the host framer, which takes every line's role from its index.  A cut before a line
+ * whose index is a multiple of 4 is a record boundary of the strict 4-line framing, whatever the line holds.  So
+ * correctness never rests on the cut, only the speed does. */
+static size_t fastq_cut(const char *buf, size_t fill) {
+    size_t next1 = 0, next2 = 0;                                   /* starts of the two lines after the candidate (0: none) */
+    for (size_t hi = fill - 1; hi > 0;) {                          /* newline at index < fill - 1: a line starts after it */
+        const char *q = (const char *)memrchr(buf, '\n', hi);
+        if (!q) break;
+        const size_t i = (size_t)(q - buf), L = i + 1;
+        if (buf[L] == '@' && next2 && buf[next2] == '+') return L;
+        next2 = next1; next1 = L;
+        hi = i;
+    }
+    return 0;
 }
 
 static int run_search(utb_searcher *s, source_t *src, sink_t *sink, int do_rc, utb_stats *stats, int *ref_exit) {
@@ -945,7 +1138,7 @@ read_loop:
             if (left != (size_t)-1 && left + carry_len <= 3 * RAMP) want = RAMP;
             else if (left != (size_t)-1 && left + carry_len < want + 2 * RAMP && want > 2 * RAMP) want = left + carry_len - 2 * RAMP;
             if (want < carry_len + 4096) want = carry_len + 4096;  /* a carried partial record must be able to complete */
-            if (want < 2 * (size_t)UTB_LINELEN + 4096) want = 2 * (size_t)UTB_LINELEN + 4096;
+            if (want < MAX_RECORD(s->fastq ? 4 : 2)) want = MAX_RECORD(s->fastq ? 4 : 2);
             if (want < cap) cap = want;
         }
         if (zero_copy) {
@@ -974,6 +1167,7 @@ read_loop:
              * without '\n', a chunk without a second header. */
             size_t used = 0;
             if (src->eof) { if (buf[fill - 1] == '\n') used = fill; }
+            else if (s->fastq) used = fastq_cut(buf, fill);
             else for (size_t hi = fill - 1; hi > 0;) {             /* newline at index < fill - 1 followed by '>' */
                 const char *q = (const char *)memrchr(buf, '\n', hi);
                 if (!q) break;
@@ -1020,9 +1214,15 @@ read_loop:
         F.idx = idx; F.idx_cap = idx ? idx_cap : 0;
         F.seq_off = utb_batch_seq_off(sl->b); F.seq_len = utb_batch_seq_len(sl->b);
         F.name_off = sl->name_off; F.name_len = sl->name_len;
-        size_t n, n_complete, end_of_records; int err_code, dangling;
-        frame_buffer(&rd_team, &F, &n, &n_complete, &end_of_records, &err_code, &dangling);
-        if (err_code) { fmt_err = 1; snprintf(fmt_msg, sizeof fmt_msg, "%s [L %llu]", fe_text(err_code), (unsigned long long)(n_reads_total + n + 1)); }
+        size_t n, n_complete, end_of_records; int err_code, dangling = 0;
+        if (s->fastq) {                                            /* a truncated record is an error like any other */
+            F.qual_off = utb_batch_qual_off(sl->b);
+            fq_buffer(&rd_team, &F, &n, &n_complete, &end_of_records, &err_code);
+            if (err_code) { fmt_err = 1; snprintf(fmt_msg, sizeof fmt_msg, "%s [record %llu]", fq_text(err_code), (unsigned long long)(n_reads_total + n + 1)); }
+        } else {
+            frame_buffer(&rd_team, &F, &n, &n_complete, &end_of_records, &err_code, &dangling);
+            if (err_code) { fmt_err = 1; snprintf(fmt_msg, sizeof fmt_msg, "%s [L %llu]", fe_text(err_code), (unsigned long long)(n_reads_total + n + 1)); }
+        }
         /* capacity: reads and 32-base position groups */
         size_t max_reads = utb_batch_max_reads(sl->b);
         uint64_t max_slots = utb_batch_max_slots(sl->b), groups = 0;
