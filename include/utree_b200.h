@@ -14,7 +14,7 @@
  *   readSamplesFPdelim()   itree.c:1202-1223 (inside utb_ctr_open)
  *   XT_doSearch32()        itree.c:833-1108  utb_search_file / utb_search_mem
  *     XT_INITIATE_WS       itree.c:860-901     framing kernels (exact host reader behind them;
- *                                              FASTQ: utb_searcher_set_input)
+ *                                              FASTQ, wrapped FASTA: utb_searcher_set_input)
  *     XT_WORD_SEARCH       itree.c:903-933     pack + sieve kernels
  *     XT_getIX32/xtSuffixBS itree.c:699-730    table lookup kernel (or the probe sequence verbatim)
  *     full aufbau vote     itree.c:1028-1098   vote kernels
@@ -177,6 +177,24 @@ enum {
 int utb_frame_fastq_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
                             uint64_t *seq_off, uint32_t *seq_len, uint64_t *qual_off, uint32_t *name_off, uint32_t *name_len,
                             size_t *n_reads, size_t *used, size_t *err_record, int *err_code);
+/* The wrapped-FASTA framer (UTB_INPUT_FASTA_WRAPPED, see utb_searcher_set_input):
+ * the joined sequence of read r is seq_out[seq_off[r] .. +seq_len[r]), the
+ * reads back to back; seq_cap >= n is required (a joined sequence is never
+ * longer than its lines).  With eof = 0 the record after the last header line
+ * is carried: *used stops before it, since without the next header it is not
+ * known to be complete.  At most max_reads records are framed.  On a malformed
+ * record the call returns UTB_ERR_FORMAT, the records before it are valid,
+ * *err_record is its 1-based number and *err_code one of UTB_FW_*; otherwise
+ * both are 0. */
+enum {
+    UTB_FW_NOHEADER = 1,     /* the input does not begin with '>'                */
+    UTB_FW_TOOLONG = 4       /* a line of UTB_LINELEN (16777216) bytes or more,
+                              * or a joined sequence of more than 16777214 bases */
+};
+int utb_frame_wrapped_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
+                              char *seq_out, size_t seq_cap, uint64_t *seq_off, uint32_t *seq_len,
+                              uint32_t *name_off, uint32_t *name_len,
+                              size_t *n_reads, size_t *used, size_t *err_record, int *err_code);
 /* The reference's output lines (itree.c:1032, 1040, 1096) for n_reads result
  * records; names are taken from bytes[name_off[r] .. +name_len[r]). */
 int utb_format_results(const utb_ctr *ctr, const char *bytes, const uint32_t *name_off, const uint32_t *name_len,
@@ -262,8 +280,40 @@ int utb_main_shallow(int argc, char **argv);
  * min_qual = q > 0 (FASTQ only, q <= 222): a base whose quality byte is below
  * 33 + q counts as 'N', so every window over it is skipped.  The caller's
  * buffer is never modified.  Call before a search, like
- * utb_searcher_set_shallow; memory the FASTQ path needs is allocated here. */
-enum { UTB_INPUT_FASTA = 0, UTB_INPUT_FASTQ = 1 };
+ * utb_searcher_set_shallow; memory the FASTQ path needs is allocated here.
+ *
+ * UTB_INPUT_FASTA_WRAPPED (min_qual must be 0) reads FASTA whose sequences
+ * span any number of lines, as genomes and assemblies are usually written:
+ *   records    a header is a line that begins with '>'; every following line
+ *              up to the next header, or to the end of the input, belongs to
+ *              that record's sequence.  Lines may have any length (ragged
+ *              widths are fine).
+ *   name       as for FASTA: the bytes after '>' up to the first ' ' or the
+ *              line end; a '\r' stays in a name that has no space.
+ *   sequence   the record's non-header lines concatenated, each without its
+ *              '\n' and one '\r' directly before the line end (or before the
+ *              end of the input).  Empty lines add nothing.  Any other byte is
+ *              kept: a '>' inside a line, ';' or a NUL is an ordinary byte and
+ *              breaks windows like any byte that is not a base.
+ *   empty      a header followed by another header, or by the end of the
+ *              input, is a read without windows.  The last line may lack its
+ *              '\n'.
+ * Malformed input: the input does not begin with '>' (a leading blank line
+ * included; UTB_FW_NOHEADER), or a line of 16777216 bytes or more counting its
+ * '\n', or a joined sequence of more than 16777214 bases (UTB_FW_TOOLONG).  It
+ * is handled as for FASTQ: every line of the records before the bad one is
+ * written, the search returns UTB_ERR_FORMAT with *ref_exit = 2, and
+ * utb_last_error() names the 1-based record and the rule.  A record larger
+ * than the batch buffer in bytes (lines averaging under about 1.5 bases, or
+ * millions of blank lines, below the base limit) is refused with the
+ * pipeline's "record larger than the batch buffer" error; batches are grown to
+ * at least 64 MiB + 4 KiB here.  For input without NUL bytes the output is
+ * byte for byte that of the same search in UTB_INPUT_FASTA mode on lin(input),
+ * which writes each record's header line unchanged, then its joined sequence,
+ * then '\n' (GG and shallow, RC on and off, one or many devices).  The
+ * sequences are joined on the device; the caller's buffer is never written,
+ * and what this input needs is allocated here, not inside a search. */
+enum { UTB_INPUT_FASTA = 0, UTB_INPUT_FASTQ = 1, UTB_INPUT_FASTA_WRAPPED = 2 };
 int utb_searcher_set_input(utb_searcher *s, int format, uint32_t min_qual);
 
 /* ---- utree-compress equivalent (XT_cmp32, itree.c:1234-1315; SURVEY 8f-2) -- */

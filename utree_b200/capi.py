@@ -15,8 +15,9 @@ LIB_PATH = os.path.join(HERE, "csrc", "libutree_b200.so")
 UTB_NONE, UTB_STAR, UTB_WALK = 0, 1, 2
 CUT_EMPTY, CUT_FULL = 0xFFFFFFFF, 0xFFFFFFFE
 BAD32 = 0xFFFFFFFF
-INPUT_FASTA, INPUT_FASTQ = 0, 1
+INPUT_FASTA, INPUT_FASTQ, INPUT_FASTA_WRAPPED = 0, 1, 2
 FQ_NOHEADER, FQ_NOSEPARATOR, FQ_QUALLEN, FQ_TOOLONG, FQ_TRUNCATED = 1, 2, 3, 4, 5
+FW_NOHEADER, FW_TOOLONG = 1, 4
 
 
 class UtbError(RuntimeError):
@@ -50,7 +51,7 @@ EXPORTS = [
     "utb_batch_create", "utb_batch_destroy", "utb_batch_bytes", "utb_batch_seq_off", "utb_batch_seq_len",
     "utb_batch_max_bytes", "utb_batch_max_reads", "utb_read_slots", "utb_batch_max_slots",
     "utb_batch_submit", "utb_batch_wait", "utb_batch_name_off", "utb_batch_name_len", "utb_batch_rerun_device", "utb_batch_counts", "utb_batch_lookup_detail", "utb_db_clone", "utb_db_device",
-    "utb_lookup_words", "utb_pack_sequence", "utb_vote_hits", "utb_vote_hits_sparse", "utb_frame_records", "utb_frame_fastq_records", "utb_format_results",
+    "utb_lookup_words", "utb_pack_sequence", "utb_vote_hits", "utb_vote_hits_sparse", "utb_frame_records", "utb_frame_fastq_records", "utb_frame_wrapped_records", "utb_format_results",
     "utb_searcher_create", "utb_searcher_destroy", "utb_search_file", "utb_search_mem", "utb_free",
     "utb_main", "utb_main_shallow", "utb_build_ubt", "utb_build_main", "utb_searcher_set_shallow", "utb_searcher_set_input", "utb_measure_rand32", "utb_compress_ubt", "utb_compress_main",
 ]
@@ -171,6 +172,27 @@ def frame_fastq_records(buf: bytes, eof=True, threads=1, max_reads=None):
                                    C.byref(n), C.byref(used), C.byref(er), C.byref(ec))
     recs = [(buf[name_off[i]:name_off[i] + name_len[i]], buf[seq_off[i]:seq_off[i] + seq_len[i]],
              buf[qual_off[i]:qual_off[i] + seq_len[i]]) for i in range(n.value)]
+    return rc, used.value, recs, (er.value, ec.value)
+
+
+def frame_wrapped_records(buf: bytes, eof=True, threads=1, max_reads=None):
+    """Host wrapped-FASTA framer (utb_frame_wrapped_records).  Returns (rc, used, [(name, joined sequence)],
+    (err_record, err_code)); err_record is 1-based, (0, 0) when every record is well formed."""
+    cap = max_reads if max_reads is not None else len(buf) // 2 + 2
+    seq_out = np.zeros(len(buf) + 1, dtype=np.uint8)
+    seq_off = np.zeros(cap, dtype=np.uint64)
+    seq_len = np.zeros(cap, dtype=np.uint32)
+    name_off = np.zeros(cap, dtype=np.uint32)
+    name_len = np.zeros(cap, dtype=np.uint32)
+    n, used, er, ec = C.c_size_t(), C.c_size_t(), C.c_size_t(), C.c_int()
+    L = lib()
+    L.utb_frame_wrapped_records.argtypes = [C.c_char_p, C.c_size_t, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_size_t] + \
+        [C.c_void_p] * 4 + [C.POINTER(C.c_size_t), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t), C.POINTER(C.c_int)]
+    rc = L.utb_frame_wrapped_records(buf, len(buf), int(eof), threads, cap, seq_out.ctypes.data, len(buf), seq_off.ctypes.data,
+                                     seq_len.ctypes.data, name_off.ctypes.data, name_len.ctypes.data,
+                                     C.byref(n), C.byref(used), C.byref(er), C.byref(ec))
+    joined = seq_out.tobytes()
+    recs = [(buf[name_off[i]:name_off[i] + name_len[i]], joined[seq_off[i]:seq_off[i] + seq_len[i]]) for i in range(n.value)]
     return rc, used.value, recs, (er.value, ec.value)
 
 
@@ -337,11 +359,15 @@ class Searcher:
         lib().utb_searcher_set_shallow.argtypes = [C.c_void_p, C.c_int]
         _ck(lib().utb_searcher_set_shallow(self.h, int(on)))
 
-    def set_input(self, fastq=True, min_qual=0):
+    def set_input(self, fastq=True, min_qual=0, wrapped=False):
         """Input format of the following searches (utb_searcher_set_input): 4-line FASTQ, bases whose quality byte is
-        below 33 + min_qual counted as N (0: no masking); fastq=False: FASTA."""
+        below 33 + min_qual counted as N (0: no masking); fastq=False: FASTA, linearised, or with wrapped=True
+        wrapped (multi-line) FASTA."""
+        if fastq and wrapped:
+            raise ValueError("set_input: wrapped input is FASTA only (fastq=False, wrapped=True)")
         lib().utb_searcher_set_input.argtypes = [C.c_void_p, C.c_int, C.c_uint32]
-        _ck(lib().utb_searcher_set_input(self.h, INPUT_FASTQ if fastq else INPUT_FASTA, min_qual))
+        fmt = INPUT_FASTQ if fastq else INPUT_FASTA_WRAPPED if wrapped else INPUT_FASTA
+        _ck(lib().utb_searcher_set_input(self.h, fmt, min_qual))
 
     def search_file(self, fasta, out, do_rc=True):
         st, ex = Stats(), C.c_int()

@@ -1755,8 +1755,11 @@ fmt_len_kernel(DevDB db, const utb_result *__restrict__ res, const uint32_t *__r
         line_len[r] = n;
     }
 }
-// exclusive scan of u32 (n up to 2^31): block sums, scan of the sums by one block, local scan + base
+// exclusive scan of u32 (n up to 2^31): block sums, scan of the sums by one block, local scan + base.
+// MAX: the exclusive max-scan instead (identity 0), in the same three kernels
 #define SCAN_TILE 2048u
+template <bool MAX> __device__ __forceinline__ uint32_t scan_op(uint32_t a, uint32_t b) { return MAX ? max(a, b) : a + b; }
+template <bool MAX>
 __global__ void __launch_bounds__(256)
 scan_sums_kernel(const uint32_t *__restrict__ in, uint32_t n, const uint32_t *__restrict__ n_dev, uint32_t n_tiles, uint32_t *__restrict__ sums) {
     if (n_dev) n = *n_dev;
@@ -1764,14 +1767,15 @@ scan_sums_kernel(const uint32_t *__restrict__ in, uint32_t n, const uint32_t *__
     for (uint32_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {   // n_tiles covers the host's upper bound of n: tiles past n sum to 0
         const uint32_t base = t * SCAN_TILE;
         uint32_t acc = 0;
-        for (uint32_t i = threadIdx.x; i < SCAN_TILE; i += 256) if (base + i < n) acc += in[base + i];
-        for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xFFFFFFFFu, acc, o);
+        for (uint32_t i = threadIdx.x; i < SCAN_TILE; i += 256) if (base + i < n) acc = scan_op<MAX>(acc, in[base + i]);
+        for (int o = 16; o; o >>= 1) acc = scan_op<MAX>(acc, __shfl_xor_sync(0xFFFFFFFFu, acc, o));
         if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = acc;
         __syncthreads();
-        if (threadIdx.x == 0) { uint32_t x = 0; for (int w = 0; w < 8; ++w) x += sh[w]; sums[t] = x; }
+        if (threadIdx.x == 0) { uint32_t x = 0; for (int w = 0; w < 8; ++w) x = scan_op<MAX>(x, sh[w]); sums[t] = x; }
         __syncthreads();
     }
 }
+template <bool MAX>
 __global__ void __launch_bounds__(1024)
 scan_top_kernel(uint32_t *__restrict__ sums, uint32_t nb, uint32_t *__restrict__ total) {
     __shared__ uint32_t sh[1024];
@@ -1783,15 +1787,19 @@ scan_top_kernel(uint32_t *__restrict__ sums, uint32_t nb, uint32_t *__restrict__
         for (uint32_t o = 1; o < 1024; o <<= 1) {
             uint32_t t = threadIdx.x >= o ? sh[threadIdx.x - o] : 0;
             __syncthreads();
-            sh[threadIdx.x] += t;
+            sh[threadIdx.x] = scan_op<MAX>(sh[threadIdx.x], t);
             __syncthreads();
         }
-        if (i < nb) sums[i] = carry + sh[threadIdx.x] - v;           // exclusive
-        carry += sh[1023];
+        if (MAX) { if (i < nb) sums[i] = max(carry, threadIdx.x ? sh[threadIdx.x - 1] : 0u); carry = max(carry, sh[1023]); }
+        else {
+            if (i < nb) sums[i] = carry + sh[threadIdx.x] - v;       // exclusive
+            carry += sh[1023];
+        }
         __syncthreads();
     }
     if (threadIdx.x == 0) *total = carry;
 }
+template <bool MAX>
 __global__ void __launch_bounds__(256)
 scan_apply_kernel(const uint32_t *__restrict__ in, uint32_t n, const uint32_t *__restrict__ n_dev, uint32_t n_tiles,
                   const uint32_t *__restrict__ sums, uint32_t *__restrict__ out) {
@@ -1806,14 +1814,17 @@ scan_apply_kernel(const uint32_t *__restrict__ in, uint32_t n, const uint32_t *_
             const uint32_t i = base + c + threadIdx.x;
             const uint32_t v = i < n ? in[i] : 0;
             uint32_t x = v;
-            for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xFFFFFFFFu, x, o); if ((threadIdx.x & 31) >= (uint32_t)o) x += y; }
+            for (int o = 1; o < 32; o <<= 1) { uint32_t y = __shfl_up_sync(0xFFFFFFFFu, x, o); if ((threadIdx.x & 31) >= (uint32_t)o) x = scan_op<MAX>(x, y); }
             if ((threadIdx.x & 31) == 31) sh[threadIdx.x >> 5] = x;
             __syncthreads();
             uint32_t wbase = run;
-            for (uint32_t w = 0; w < (threadIdx.x >> 5); ++w) wbase += sh[w];
-            if (i < n) out[i] = wbase + x - v;
+            for (uint32_t w = 0; w < (threadIdx.x >> 5); ++w) wbase = scan_op<MAX>(wbase, sh[w]);
+            if (MAX) {                                                 // exclusive: the inclusive value of the lane before
+                const uint32_t y = __shfl_up_sync(0xFFFFFFFFu, x, 1);
+                if (i < n) out[i] = max(wbase, (threadIdx.x & 31) ? y : 0u);
+            } else if (i < n) out[i] = wbase + x - v;
             __syncthreads();
-            if (threadIdx.x == 255) run = wbase + x;
+            if (threadIdx.x == 255) run = scan_op<MAX>(wbase, x);
             __syncthreads();
         }
     }
@@ -1999,6 +2010,139 @@ qual_mask_kernel(uint8_t *raw, const uint64_t *__restrict__ seq_off, const uint6
         if (nv < 32u) m &= (1u << nv) - 1u;
         uint8_t *s = raw + __ldg(seq_off + lo) + b0;
         for (; m; m &= m - 1u) s[__ffs(m) - 1] = 'N';
+    }
+}
+
+// ---- wrapped FASTA (UTB_INPUT_FASTA_WRAPPED) ----------------------------------------------------------------
+// A record is a header line (a line that begins with '>') and every line up to the next header; its sequence is
+// the concatenation of those lines without their '\n' and one '\r' before it.  No newline index: a chunk may hold
+// n_bytes / 2 lines.  Everything is per 64-byte tile (nl_mask64's unit), one thread per tile:
+//   wrap_tile_kernel   last line start and header count per tile
+//   max-scan / sum-scan  -> the line in force at each tile's start, the index of its first record
+//   wrap_keep_kernel   which bytes are sequence bytes (kmask), their count per tile, the long-line rule, and
+//                      where every header starts (name_off)
+//   sum-scan           -> where each tile's sequence bytes go in d_join
+//   wrap_join_kernel   the sequence bytes, packed into d_join (stores coalesced per warp)
+//   wrap_record_kernel one thread per record: name, seq_off / seq_len (from kmask, O(1)), the base limit, slots
+// The reader cuts a chunk right before a line that begins with '>', which in wrapped FASTA always starts a record:
+// by induction every chunk starts on a header and ends with '\n'.  A chunk that does not begin with '>', or holds
+// more headers than the batch has reads, is flagged FRE_CHUNK and re-framed by the host (pipeline.c, wr_buffer),
+// which applies the same rules.
+struct WrapTile { uint64_t nl, ls, hs, cr; };   // newlines, line starts, header starts, '\r' bytes of one tile
+__device__ __forceinline__ WrapTile wrap_tile(const uint8_t *__restrict__ raw, uint64_t at, uint64_t n_bytes) {
+    WrapTile w = {0, 0, 0, 0};
+    if (at >= n_bytes) return w;
+    uint64_t gt = 0;
+    const uint4 *p = reinterpret_cast<const uint4 *>(raw + at);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const uint4 v = __ldg(p + q);
+        const uint32_t x[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const uint32_t sh = 16 * q + 4 * k;
+            w.nl |= (uint64_t)(((__vcmpeq4(x[k], 0x0A0A0A0Au) & 0x01010101u) * 0x01020408u) >> 24) << sh;
+            w.cr |= (uint64_t)(((__vcmpeq4(x[k], 0x0D0D0D0Du) & 0x01010101u) * 0x01020408u) >> 24) << sh;
+            gt |= (uint64_t)(((__vcmpeq4(x[k], 0x3E3E3E3Eu) & 0x01010101u) * 0x01020408u) >> 24) << sh;
+        }
+    }
+    const uint64_t left = n_bytes - at, valid = left < 64 ? (1ull << left) - 1ull : ~0ull;
+    const uint64_t first = at == 0 || raw[at - 1] == '\n';          // byte at starts a line
+    w.nl &= valid; w.cr &= valid;
+    w.ls = ((w.nl << 1) | first) & valid;
+    w.hs = w.ls & gt;
+    return w;
+}
+__global__ void __launch_bounds__(256)
+wrap_tile_kernel(const uint8_t *__restrict__ raw, uint64_t n_bytes, uint32_t n_tiles,
+                 uint32_t *__restrict__ last_ls, uint32_t *__restrict__ hdr_cnt, uint32_t *__restrict__ err) {
+    const uint32_t t = blockIdx.x * 256u + threadIdx.x;
+    if (t >= n_tiles) return;
+    const uint64_t at = (uint64_t)t * 64u;
+    const WrapTile w = wrap_tile(raw, at, n_bytes);
+    last_ls[t] = w.ls ? (uint32_t)(at + 63u - (uint32_t)__clzll((long long)w.ls)) : 0u;   // 0: none (the max-scan's identity)
+    hdr_cnt[t] = __popcll(w.hs);
+    if (t == 0 && raw[0] != '>') atomicMin(err, (uint32_t)FRE_CHUNK);
+}
+// ls_in[t]: start of the line in force at tile t's first byte (exclusive max-scan of last_ls); rec0[t]: records
+// that start before tile t (exclusive sum-scan of hdr_cnt).  kmask[t]: the tile's sequence bytes -- not in a header
+// line, not '\n', not a '\r' right before '\n'.
+__global__ void __launch_bounds__(256)
+wrap_keep_kernel(const uint8_t *__restrict__ raw, uint64_t n_bytes, uint32_t n_tiles, const uint32_t *__restrict__ ls_in,
+                 const uint32_t *__restrict__ rec0, const uint32_t *__restrict__ dims, uint64_t *__restrict__ kmask,
+                 uint32_t *__restrict__ keep_cnt, uint32_t *__restrict__ name_off, uint32_t *__restrict__ err) {
+    const uint32_t t = blockIdx.x * 256u + threadIdx.x;
+    if (t >= n_tiles) return;
+    const uint64_t at = (uint64_t)t * 64u;
+    const WrapTile w = wrap_tile(raw, at, n_bytes);
+    const uint32_t lin = ls_in[t], r0 = rec0[t], n_reads = dims[0];
+    // in-header-line mask: every byte takes the header flag of the nearest line start at or before it (segmented
+    // copy by doubling; bit 0 is seeded from the line in force when no line starts there)
+    uint64_t f = w.ls | 1ull, v = w.hs | ((!(w.ls & 1ull) && raw[lin] == '>') ? 1ull : 0ull);
+#pragma unroll
+    for (int s = 1; s < 64; s <<= 1) { v = (v & f) | ((v << s) & ~f); f |= f << s; }
+    const uint64_t left = n_bytes - at;
+    const uint64_t ends = (w.nl >> 1) | (left > 64 ? (uint64_t)(raw[at + 64] == '\n') << 63 : 1ull << (left - 1));   // byte before a line end
+    const uint64_t valid = left < 64 ? (1ull << left) - 1ull : ~0ull;
+    const uint64_t k = ~v & ~w.nl & ~(w.cr & ends) & valid;
+    kmask[t] = k;
+    keep_cnt[t] = __popcll(k);
+    // a line of UTB_LINELEN bytes or more, counting its '\n': only the tile's first newline can end a line that
+    // starts before the tile; its record is the last one that starts before it
+    if (w.nl) {
+        const uint32_t j = __ffsll((long long)w.nl) - 1;
+        if (!(w.ls & ((2ull << j) - 1ull)) && at + j + 1u - lin >= UTB_LINELEN && r0)
+            atomicMin(err, ((r0 - 1u) << 3) | UTB_FW_TOOLONG);
+    }
+    uint32_t r = r0;
+    for (uint64_t h = w.hs; h && r < n_reads; h &= h - 1ull, ++r) name_off[r] = (uint32_t)(at + __ffsll((long long)h));   // the byte after '>'
+}
+// Packs the sequence bytes of the block's 256 tiles into join: each thread takes 4 bytes at a stride of 1 KiB, so a
+// warp's stores fall into a few consecutive sectors.
+__global__ void __launch_bounds__(256)
+wrap_join_kernel(const uint8_t *__restrict__ raw, uint64_t n_bytes, uint32_t n_tiles, const uint64_t *__restrict__ kmask,
+                 const uint32_t *__restrict__ join_off, uint8_t *__restrict__ join) {
+    __shared__ uint64_t km[256];
+    __shared__ uint32_t jo[256];
+    const uint32_t t0 = blockIdx.x * 256u;
+    if (t0 + threadIdx.x < n_tiles) { km[threadIdx.x] = kmask[t0 + threadIdx.x]; jo[threadIdx.x] = join_off[t0 + threadIdx.x]; }
+    __syncthreads();
+    const uint64_t base = (uint64_t)t0 * 64u;
+#pragma unroll 4
+    for (uint32_t c = 0; c < FR_BLOCK; c += 1024u) {
+        const uint32_t o = c + 4u * threadIdx.x, lt = o >> 6, sh = o & 63u;
+        if (base + o >= n_bytes) break;
+        const uint64_t m = km[lt];
+        uint32_t bits = (uint32_t)(m >> sh) & 0xFu;
+        if (!bits) continue;
+        const uint32_t x = *reinterpret_cast<const uint32_t *>(raw + base + o);
+        uint32_t d = jo[lt] + __popcll(m & ((1ull << sh) - 1ull));
+        for (; bits; bits &= bits - 1u) join[d++] = (uint8_t)(x >> (8u * (__ffs(bits) - 1u)));
+    }
+}
+__device__ __forceinline__ uint32_t wrap_join_at(const uint64_t *__restrict__ kmask, const uint32_t *__restrict__ join_off, uint32_t p) {
+    return join_off[p >> 6] + __popcll(kmask[p >> 6] & ((1ull << (p & 63u)) - 1ull));   // sequence bytes before byte p
+}
+// One thread per record r: its header starts at name_off[r] - 1; a header line holds no sequence byte, so the
+// record's sequence starts at the join offset of its header and ends at the next record's (or the total).
+__global__ void __launch_bounds__(256)
+wrap_record_kernel(const uint8_t *__restrict__ raw, uint64_t n_bytes, const uint64_t *__restrict__ kmask,
+                   const uint32_t *__restrict__ join_off, const uint32_t *__restrict__ join_total, uint32_t n_reads,
+                   const uint32_t *__restrict__ dims, uint64_t *__restrict__ seq_off, uint32_t *__restrict__ seq_len,
+                   const uint32_t *__restrict__ name_off, uint32_t *__restrict__ name_len,
+                   uint32_t *__restrict__ slots, uint32_t *__restrict__ err) {
+    if (dims) n_reads = dims[0];
+    for (uint64_t r64 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r64 < n_reads; r64 += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t r = (uint32_t)r64, hs = name_off[r] - 1u;
+        const uint32_t so = wrap_join_at(kmask, join_off, hs);
+        const uint32_t eo = r + 1u < n_reads ? wrap_join_at(kmask, join_off, name_off[r + 1u] - 1u) : *join_total;
+        uint32_t length = eo - so;
+        if (length > UTB_MAXSEQ) { atomicMin(err, (r << 3) | UTB_FW_TOOLONG); length = 0; }
+        uint32_t e = hs + 1u;                                      // name: up to the first ' ' or the newline, as for FASTA
+        while (e < n_bytes && raw[e] != ' ' && raw[e] != '\n') ++e;
+        seq_off[r] = so; seq_len[r] = length;
+        name_len[r] = e - hs - 1u;
+        slots[r] = (length + 1u + 31u) / 32u;                      // utb_read_slots
     }
 }
 
@@ -2481,6 +2625,12 @@ struct utb_batch {
     // FASTQ input (utb_batch_set_input): per read the offset of its quality line; min_qual > 0 masks low-quality bases
     int fastq; uint32_t min_qual;
     uint64_t *h_qual_off, *d_qual_off;
+    // wrapped FASTA (utb_batch_set_input): pack_kernel reads the joined sequence bytes d_join instead of d_raw; a
+    // host-framed batch brings them in h_join.  Device framing: per 64-byte tile last line start, line in force,
+    // header count, first record, sequence-byte count, join offset (d_wt, 6 x wt_cap) and sequence-byte mask
+    int wrapped; const uint8_t *d_pack;                            // pack_kernel's input: d_raw, or d_join
+    char *h_join; uint8_t *d_join;
+    uint32_t *d_wt, *d_wsums, *d_wtotal; uint64_t *d_kmask; size_t wt_cap;
 };
 
 extern "C" uint64_t utb_read_slots(uint32_t len) { return ((uint64_t)len + 1 + 31) / 32; }
@@ -2510,6 +2660,7 @@ extern "C" void utb_batch_destroy(utb_batch *b) {
     cudaFree(b->d_nl); cudaFree(b->d_blk); cudaFree(b->d_frame_err); cudaFreeHost(b->h_frame_err);
     cudaFree(b->d_frame_info); cudaFree(b->d_dims); cudaFreeHost(b->h_dims);
     cudaFreeHost(b->h_qual_off); cudaFree(b->d_qual_off);
+    cudaFreeHost(b->h_join); cudaFree(b->d_join); cudaFree(b->d_wt); cudaFree(b->d_wsums); cudaFree(b->d_wtotal); cudaFree(b->d_kmask);
     if (b->done) cudaEventDestroy(b->done);
     for (int i = 0; i < 7; ++i) if (b->ev[i]) cudaEventDestroy(b->ev[i]);
     if (b->st) cudaStreamDestroy(b->st);
@@ -2565,6 +2716,7 @@ extern "C" int utb_batch_create(utb_db *db, size_t max_bytes, size_t max_reads, 
     BK(cudaMalloc(&b->d_counters, 4 * COUNTER_SLOTS * 8));
     if (vs_alloc(db, max_bytes, &b->vs)) { utb_batch_destroy(b); return UTB_ERR_CUDA; }
     BK(cudaMemset(b->d_raw, 0, max_bytes + 128));
+    b->d_pack = b->d_raw;
     if (db->sieve) {                                               // queue for a quarter of the lookup slots; overflow resolves inline
         b->q_cap = npos * 2 / 4 + 4096;
         const char *qc = getenv("UTB_QCAP");                       // tests: a tiny queue forces the overflow path
@@ -2614,11 +2766,11 @@ static int launch_stages(utb_batch *b, bool timed) {
     if (timed) CK(cudaEventRecord(b->ev[0], b->st));
     if (n_reads) {
         const unsigned grid = gs_grid(b, (uint64_t)n_groups + PK_GUARD, 256, 32);
-        if (!two_phase) pack_kernel<true, false><<<grid, 256, 0, b->st>>>(b->d_raw, b->d_seq_off, b->d_seq_len, b->d_grp_off,
+        if (!two_phase) pack_kernel<true, false><<<grid, 256, 0, b->st>>>(b->d_pack, b->d_seq_off, b->d_seq_len, b->d_grp_off,
                                                                         n_reads, n_groups, b->dims_dev, b->d_pk, b->d_bad, nullptr, b->d_rid);
-        else if (b->out == UTB_OUT_SELECTIONS) pack_kernel<true, true><<<grid, 256, 0, b->st>>>(b->d_raw, b->d_seq_off, b->d_seq_len, b->d_grp_off,
+        else if (b->out == UTB_OUT_SELECTIONS) pack_kernel<true, true><<<grid, 256, 0, b->st>>>(b->d_pack, b->d_seq_off, b->d_seq_len, b->d_grp_off,
                                                                         n_reads, n_groups, b->dims_dev, b->d_pk, b->d_bad, b->d_pl, b->d_rid);
-        else pack_kernel<false, true><<<grid, 256, 0, b->st>>>(b->d_raw, b->d_seq_off, b->d_seq_len, b->d_grp_off,
+        else pack_kernel<false, true><<<grid, 256, 0, b->st>>>(b->d_pack, b->d_seq_off, b->d_seq_len, b->d_grp_off,
                                                              n_reads, n_groups, b->dims_dev, nullptr, b->d_bad, b->d_pl, b->d_rid);
         b->launches++;
     }
@@ -2673,9 +2825,9 @@ static int launch_stages(utb_batch *b, bool timed) {
         in.hitmap = b->used_sieve ? b->d_hitmap : nullptr;
         const uint32_t nt = (n_reads + SCAN_TILE - 1) / SCAN_TILE;
         shallow_select_kernel<<<gs_grid(b, n_reads, 128, 32), 128, 0, b->st>>>(d, in, b->d_pk, b->d_bad, n_reads, b->dims_dev, b->d_sel_cnt, b->d_sel_gap);
-        scan_sums_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_sel_cnt, n_reads, b->dims_dev, nt, b->d_scan_sums);
-        scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_sel_total);
-        scan_apply_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_sel_cnt, n_reads, b->dims_dev, nt, b->d_scan_sums, b->d_sel_off);
+        scan_sums_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_sel_cnt, n_reads, b->dims_dev, nt, b->d_scan_sums);
+        scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_sel_total);
+        scan_apply_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_sel_cnt, n_reads, b->dims_dev, nt, b->d_scan_sums, b->d_sel_off);
         shallow_compact_kernel<<<gs_grid(b, n_reads, 128, 32), 128, 0, b->st>>>(in, n_reads, b->dims_dev, b->d_sel_cnt, b->d_sel_off, b->d_sel_gap, b->d_sel);
         b->launches += 5;
     } else if (n_reads) {
@@ -2799,17 +2951,22 @@ static int submit_impl(utb_batch *b, const char *src, size_t n_bytes, size_t n_r
             CK(cudaMemcpyAsync(b->d_name_len, b->h_name_len, n_reads * 4, cudaMemcpyHostToDevice, b->st));
         }
     }
+    b->d_pack = b->wrapped ? b->d_join : b->d_raw;
     if (n_reads) {
         CK(cudaMemcpyAsync(b->d_raw, src ? src : b->h_bytes, n_bytes, cudaMemcpyHostToDevice, b->st));
+        if (b->wrapped) {                                          // the host framer joined the sequences back to back
+            const uint64_t nj = b->h_seq_off[n_reads - 1] + b->h_seq_len[n_reads - 1];
+            if (nj) CK(cudaMemcpyAsync(b->d_join, b->h_join, nj, cudaMemcpyHostToDevice, b->st));
+        }
         CK(cudaMemcpyAsync(b->d_seq_off, b->h_seq_off, n_reads * 8, cudaMemcpyHostToDevice, b->st));
         CK(cudaMemcpyAsync(b->d_seq_len, b->h_seq_len, n_reads * 4, cudaMemcpyHostToDevice, b->st));
         if (!total_groups) CK(cudaMemcpyAsync(b->d_grp_off, b->h_grp_off, (n_reads + 1) * 4, cudaMemcpyHostToDevice, b->st));
         else {                                                     // grp_off = exclusive scan of the per-read slot counts
             const uint32_t n = (uint32_t)n_reads, nt = (n + SCAN_TILE - 1) / SCAN_TILE;
             slots_kernel<<<(n + 255) / 256, 256, 0, b->st>>>(b->d_seq_len, n, b->d_line_len);
-            scan_sums_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, nullptr, nt, b->d_scan_sums);
-            scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_text_len);
-            scan_apply_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, nullptr, nt, b->d_scan_sums, b->d_grp_off);
+            scan_sums_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, nullptr, nt, b->d_scan_sums);
+            scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_text_len);
+            scan_apply_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, nullptr, nt, b->d_scan_sums, b->d_grp_off);
             b->launches += 4;
         }
         if (b->fastq && b->min_qual) {
@@ -2842,9 +2999,9 @@ static int finish_submit(utb_batch *b) {
         CK(cudaMemsetAsync(b->d_text_len, 0, 4, b->st));
         if (n) {
             fmt_len_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->db->d, b->d_results, b->d_name_len, n, b->dims_dev, b->d_line_len);
-            scan_sums_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->dims_dev, nt, b->d_scan_sums);
-            scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_text_len);
-            scan_apply_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->dims_dev, nt, b->d_scan_sums, b->d_line_off);
+            scan_sums_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->dims_dev, nt, b->d_scan_sums);
+            scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_text_len);
+            scan_apply_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->dims_dev, nt, b->d_scan_sums, b->d_line_off);
             fmt_write_kernel<<<gs_grid(b, n, FW_WARPS, 32), FW_WARPS * 32, 0, b->st>>>(
                 b->db->d, b->d_results, b->d_raw, b->d_name_off, b->d_name_len, b->d_line_off, n, b->dims_dev, b->d_text);
             b->launches += 5;
@@ -2910,9 +3067,33 @@ extern "C" int utb_batch_prepare(utb_batch *b, utb_batch_out out, int chunked) {
     if (!rc && chunked) rc = ensure_chunk_buffers(b);
     return rc;
 }
-// The input format of the batch's later submits (FASTA, or FASTQ with min_qual); allocates what FASTQ needs.
-extern "C" int utb_batch_set_input(utb_batch *b, int fastq, uint32_t min_qual, int chunked) {
-    if (!b || (!fastq && min_qual) || min_qual > 222) { utb_set_error("utb_batch_set_input: bad argument"); return UTB_ERR_ARG; }
+// The input format of the batch's later submits (UTB_INPUT_*; min_qual for FASTQ); allocates what the format needs.
+static int ensure_wrapped_buffers(utb_batch *b, int chunked) {
+    if (!b->h_join) {
+        void *h = nullptr, *d = nullptr;
+        cudaError_t e = cudaMallocHost(&h, b->max_bytes + 64);
+        if (e == cudaSuccess) e = cudaMalloc(&d, b->max_bytes + 128);   // pack_kernel's over-read, as for d_raw
+        if (e == cudaSuccess) e = cudaMemset(d, 0, b->max_bytes + 128);
+        if (e != cudaSuccess) { cudaFreeHost(h); cudaFree(d); CK(e); }
+        b->h_join = (char *)h; b->d_join = (uint8_t *)d;
+    }
+    if (!chunked || b->d_wt) return UTB_OK;
+    const size_t nt = b->max_bytes / 64 + 2;
+    void *p[4] = {nullptr, nullptr, nullptr, nullptr};
+    cudaError_t e = cudaMalloc(&p[0], 6 * nt * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&p[1], (nt / SCAN_TILE + 2) * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&p[2], 8);
+    if (e == cudaSuccess) e = cudaMalloc(&p[3], nt * 8);
+    if (e != cudaSuccess) { for (int i = 0; i < 4; ++i) cudaFree(p[i]); CK(e); }
+    b->d_wt = (uint32_t *)p[0]; b->d_wsums = (uint32_t *)p[1]; b->d_wtotal = (uint32_t *)p[2]; b->d_kmask = (uint64_t *)p[3];
+    b->wt_cap = nt;
+    return UTB_OK;
+}
+extern "C" int utb_batch_set_input(utb_batch *b, int format, uint32_t min_qual, int chunked) {
+    if (!b || format < UTB_INPUT_FASTA || format > UTB_INPUT_FASTA_WRAPPED || (format != UTB_INPUT_FASTQ && min_qual) || min_qual > 222) {
+        utb_set_error("utb_batch_set_input: bad argument"); return UTB_ERR_ARG;
+    }
+    const int fastq = format == UTB_INPUT_FASTQ;
     CK(cudaSetDevice(b->db->device));
     if (fastq && !b->h_qual_off) {                                 // both arrays or neither
         void *h = nullptr, *d = nullptr;
@@ -2921,19 +3102,22 @@ extern "C" int utb_batch_set_input(utb_batch *b, int fastq, uint32_t min_qual, i
         if (e != cudaSuccess) { cudaFreeHost(h); cudaFree(d); CK(e); }
         b->h_qual_off = (uint64_t *)h; b->d_qual_off = (uint64_t *)d;
     }
+    if (format == UTB_INPUT_FASTA_WRAPPED) { int rw = ensure_wrapped_buffers(b, chunked); if (rw) return rw; }
     const int old_fastq = b->fastq;
-    b->fastq = fastq ? 1 : 0;                                      // ensure_chunk_buffers sizes the newline index by it
+    b->fastq = fastq;                                              // ensure_chunk_buffers sizes the newline index by it
     const int rc = chunked ? ensure_chunk_buffers(b) : UTB_OK;     // keeps the old index if the larger one cannot be had
     if (rc) { b->fastq = old_fastq; return rc; }
     b->min_qual = min_qual;
+    b->wrapped = format == UTB_INPUT_FASTA_WRAPPED;
     return UTB_OK;
 }
 extern "C" uint64_t *utb_batch_qual_off(utb_batch *b) { return b->h_qual_off; }
+extern "C" char *utb_batch_join(utb_batch *b) { return b->h_join; }
 extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out) {
     if (!b || !n_bytes || out == UTB_OUT_RESULTS) { utb_set_error("utb_batch_submit_chunk: bad argument"); return UTB_ERR_ARG; }
     if (n_bytes > b->max_bytes || n_reads > b->max_reads || n_bytes >= 0xFFFFFFFFull) { utb_set_error("utb_batch_submit_chunk: batch over capacity"); return UTB_ERR_LIMIT; }
     CK(cudaSetDevice(b->db->device));
-    { int ra = ensure_chunk_buffers(b); if (ra) return ra; }
+    { int ra = ensure_chunk_buffers(b); if (!ra && b->wrapped) ra = ensure_wrapped_buffers(b, 1); if (ra) return ra; }
     int rt = out == UTB_OUT_SELECTIONS ? ensure_shallow_buffers(b) : ensure_text_buffers(b);
     if (rt) return rt;
     // upper bounds the launches are sized for: every read owns ceil((len+1)/32) <= len/32 + 1 groups
@@ -2943,29 +3127,53 @@ extern "C" int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_by
     if (g_ub * 32ull * (do_rc ? 2u : 1u) >= 0xFFFFFFFFull) { utb_set_error("utb_batch_submit_chunk: chunk too large for the 32-bit slot space"); return UTB_ERR_LIMIT; }
     b->n_reads = n_ub; b->n_groups = (uint32_t)g_ub; b->do_rc = do_rc ? 1 : 0;
     b->out = out; b->dims_dev = b->d_dims; b->framed_on_device = 1;
+    b->d_pack = b->wrapped ? b->d_join : b->d_raw;
     *b->h_frame_err = FR_ERR_NONE;
     CK(cudaMemcpyAsync(b->d_raw, src ? src : b->h_bytes, n_bytes, cudaMemcpyHostToDevice, b->st));
     CK(cudaMemsetAsync(b->d_frame_err, 0xFF, 4, b->st));
     CK(cudaMemsetAsync(b->d_frame_info, 0, 8, b->st));
     const uint32_t fb = (uint32_t)((n_bytes + FR_BLOCK - 1) / FR_BLOCK), n = (uint32_t)n_ub, nt = (n + SCAN_TILE - 1) / SCAN_TILE;
-    nl_count_kernel<<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, b->d_frame_info + 1);
-    scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_blk, fb, b->d_frame_info);       // block counts -> exclusive offsets, total newlines
-    if (b->fastq) {
-        frame_setup_kernel<4><<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
-        nl_index_kernel<4><<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, 0, b->d_dims, b->d_nl);
-        frame_parse_fastq_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, b->d_nl, n, b->d_dims, b->d_seq_off, b->d_seq_len,
-                                                                            b->d_qual_off, b->d_name_off, b->d_name_len, b->d_line_len, b->d_frame_err);
+    if (b->wrapped) {
+        const uint32_t T = (uint32_t)((n_bytes + 63) / 64), tt = (T + SCAN_TILE - 1) / SCAN_TILE;
+        uint32_t *last_ls = b->d_wt, *ls_in = last_ls + b->wt_cap, *hdr = ls_in + b->wt_cap, *rec0 = hdr + b->wt_cap;
+        uint32_t *keep = rec0 + b->wt_cap, *join_off = keep + b->wt_cap;
+        wrap_tile_kernel<<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, T, last_ls, hdr, b->d_frame_err);
+        scan_sums_kernel<true><<<gs_grid(b, tt, 1, 8), 256, 0, b->st>>>(last_ls, T, nullptr, tt, b->d_wsums);
+        scan_top_kernel<true><<<1, 1024, 0, b->st>>>(b->d_wsums, tt, b->d_wtotal + 1);
+        scan_apply_kernel<true><<<gs_grid(b, tt, 1, 8), 256, 0, b->st>>>(last_ls, T, nullptr, tt, b->d_wsums, ls_in);
+        scan_sums_kernel<false><<<gs_grid(b, tt, 1, 8), 256, 0, b->st>>>(hdr, T, nullptr, tt, b->d_wsums);
+        scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_wsums, tt, b->d_frame_info);          // total headers
+        scan_apply_kernel<false><<<gs_grid(b, tt, 1, 8), 256, 0, b->st>>>(hdr, T, nullptr, tt, b->d_wsums, rec0);
+        frame_setup_kernel<1><<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
+        wrap_keep_kernel<<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, T, ls_in, rec0, b->d_dims, b->d_kmask, keep, b->d_name_off, b->d_frame_err);
+        scan_sums_kernel<false><<<gs_grid(b, tt, 1, 8), 256, 0, b->st>>>(keep, T, nullptr, tt, b->d_wsums);
+        scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_wsums, tt, b->d_wtotal);              // total sequence bytes
+        scan_apply_kernel<false><<<gs_grid(b, tt, 1, 8), 256, 0, b->st>>>(keep, T, nullptr, tt, b->d_wsums, join_off);
+        wrap_join_kernel<<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, T, b->d_kmask, join_off, b->d_join);
+        wrap_record_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_kmask, join_off, b->d_wtotal, n, b->d_dims,
+                                                                      b->d_seq_off, b->d_seq_len, b->d_name_off, b->d_name_len, b->d_line_len, b->d_frame_err);
+        b->launches += 14;
     } else {
-        frame_setup_kernel<2><<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
-        nl_index_kernel<2><<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, 0, b->d_dims, b->d_nl);
-        frame_parse_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, b->d_nl, n, b->d_dims, b->d_seq_off, b->d_seq_len, b->d_name_off,
-                                                                      b->d_name_len, b->d_line_len, b->d_frame_err);
+        nl_count_kernel<<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, b->d_frame_info + 1);
+        scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_blk, fb, b->d_frame_info);       // block counts -> exclusive offsets, total newlines
+        if (b->fastq) {
+            frame_setup_kernel<4><<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
+            nl_index_kernel<4><<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, 0, b->d_dims, b->d_nl);
+            frame_parse_fastq_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, b->d_nl, n, b->d_dims, b->d_seq_off, b->d_seq_len,
+                                                                                b->d_qual_off, b->d_name_off, b->d_name_len, b->d_line_len, b->d_frame_err);
+        } else {
+            frame_setup_kernel<2><<<1, 1, 0, b->st>>>(b->d_frame_info, (uint32_t)n_ub, b->d_dims, b->d_frame_err);
+            nl_index_kernel<2><<<fb, 256, 0, b->st>>>(b->d_raw, n_bytes, b->d_blk, 0, b->d_dims, b->d_nl);
+            frame_parse_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->d_raw, b->d_nl, n, b->d_dims, b->d_seq_off, b->d_seq_len, b->d_name_off,
+                                                                          b->d_name_len, b->d_line_len, b->d_frame_err);
+        }
+        b->launches += 5;
     }
     // grp_off = exclusive scan of the per-read group counts; the total (dims[1]) stays on the device
-    scan_sums_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->d_dims, nt, b->d_scan_sums);
-    scan_top_kernel<<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_dims + 1);
-    scan_apply_kernel<<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->d_dims, nt, b->d_scan_sums, b->d_grp_off);
-    b->launches += 8;
+    scan_sums_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->d_dims, nt, b->d_scan_sums);
+    scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_dims + 1);
+    scan_apply_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->d_dims, nt, b->d_scan_sums, b->d_grp_off);
+    b->launches += 3;
     CK(cudaGetLastError());
     if (b->fastq && b->min_qual) { int rm = launch_mask(b); if (rm) return rm; }
     CK(cudaMemcpyAsync(b->h_frame_err, b->d_frame_err, 4, cudaMemcpyDeviceToHost, b->st));

@@ -125,7 +125,7 @@ struct utb_searcher {
     char *arena; size_t arena_cap; /* page-locked output of utb_search_mem: the devices copy their text straight into it; valid until
                                     * the next search on this searcher or its destruction */
     int spread;                    /* more than one physical GPU: page-locked buffers are interleaved over the NUMA nodes */
-    int fastq;                     /* input is 4-line FASTQ (utb_searcher_set_input) */
+    int format;                    /* UTB_INPUT_FASTA, _FASTQ (4-line) or _FASTA_WRAPPED (utb_searcher_set_input) */
     uint32_t min_qual;             /* FASTQ: bases with a quality byte below 33 + min_qual count as 'N' (0: off) */
 };
 
@@ -177,7 +177,7 @@ static int slots_create(utb_searcher *s) {
         rc = utb_batch_create(s->dbs[i % s->n_devices], s->batch_bytes, s->batch_reads, &nb[i]);
         if (!rc) rc = utb_batch_prepare(nb[i], UTB_OUT_TEXT, s->device_frame);
         if (!rc && s->shallow) rc = utb_batch_prepare(nb[i], UTB_OUT_SELECTIONS, s->device_frame);
-        if (!rc && s->fastq) rc = utb_batch_set_input(nb[i], 1, s->min_qual, s->device_frame);
+        if (!rc && s->format != UTB_INPUT_FASTA) rc = utb_batch_set_input(nb[i], s->format, s->min_qual, s->device_frame);
         if (s->spread) mem_interleave(0);
     }
     for (int i = 0; i < s->n_slots; ++i) {
@@ -256,32 +256,32 @@ int utb_searcher_set_shallow(utb_searcher *s, int on) {
 }
 
 int utb_searcher_set_input(utb_searcher *s, int format, uint32_t min_qual) {
-    if (!s || (format != UTB_INPUT_FASTA && format != UTB_INPUT_FASTQ) || (format == UTB_INPUT_FASTA && min_qual) || min_qual > 222) {
+    if (!s || format < UTB_INPUT_FASTA || format > UTB_INPUT_FASTA_WRAPPED || (format != UTB_INPUT_FASTQ && min_qual) || min_qual > 222) {
         utb_set_error("utb_searcher_set_input: bad argument (format %d, min_qual %u)", format, min_qual);
         return UTB_ERR_ARG;
     }
-    const int fastq = format == UTB_INPUT_FASTQ;
     /* on failure the searcher keeps its batches and its format */
-    const int old_fastq = s->fastq;
+    const int old_format = s->format;
     const uint32_t old_qual = s->min_qual;
-    if (fastq && s->batch_bytes < MAX_RECORD(4)) {                 /* a batch must hold one record of four maximal lines */
+    /* a batch must hold one FASTQ record of four maximal lines; wrapped FASTA takes the same floor */
+    if (format != UTB_INPUT_FASTA && s->batch_bytes < MAX_RECORD(4)) {
         const size_t keep = s->batch_bytes;
         s->batch_bytes = MAX_RECORD(4);
         int rc = batch_reads_for(s) ? UTB_OK : UTB_ERR_LIMIT;
         if (rc) utb_set_error("batch too large for device-side formatting");
-        s->fastq = fastq; s->min_qual = min_qual;
+        s->format = format; s->min_qual = min_qual;
         if (!rc) rc = slots_create(s);
-        if (rc) { s->batch_bytes = keep; batch_reads_for(s); s->fastq = old_fastq; s->min_qual = old_qual; }
+        if (rc) { s->batch_bytes = keep; batch_reads_for(s); s->format = old_format; s->min_qual = old_qual; }
         return rc;
     }
     for (int i = 0; i < s->n_slots; ++i) {
-        int rc = utb_batch_set_input(s->slots[i].b, fastq, min_qual, s->device_frame);
+        int rc = utb_batch_set_input(s->slots[i].b, format, min_qual, s->device_frame);
         if (rc) {                                                  /* back to the old format: allocates nothing */
-            for (int j = 0; j < i; ++j) (void)utb_batch_set_input(s->slots[j].b, old_fastq, old_qual, s->device_frame);
+            for (int j = 0; j < i; ++j) (void)utb_batch_set_input(s->slots[j].b, old_format, old_qual, s->device_frame);
             return rc;
         }
     }
-    s->fastq = fastq; s->min_qual = min_qual;
+    s->format = format; s->min_qual = min_qual;
     return UTB_OK;
 }
 
@@ -656,8 +656,13 @@ typedef struct {
     const char *buf; size_t fill; int eof;
     uint64_t *seq_off; uint32_t *seq_len; uint32_t *name_off, *name_len;
     uint64_t *qual_off;            /* FASTQ */
-    size_t cnt[MAX_TEAM];          /* newlines per segment */
-    size_t base[MAX_TEAM];         /* newlines before the segment */
+    char *join;                    /* wrapped FASTA: the joined sequences */
+    size_t hfirst[MAX_TEAM];       /* wrapped FASTA: first header of each segment (fill: none) */
+    uint64_t jsum[MAX_TEAM];       /* wrapped FASTA: sequence bytes of each worker's records, then where they go */
+    size_t err_at[MAX_TEAM];       /* wrapped FASTA: where each worker's first bad record starts */
+    size_t n_valid;                /* wrapped FASTA: records before the first bad one */
+    size_t cnt[MAX_TEAM];          /* newlines per segment (wrapped FASTA: headers) */
+    size_t base[MAX_TEAM];         /* newlines before the segment (wrapped FASTA: headers) */
     size_t n_rec;                  /* complete records in the buffer (clamped to max_rec) */
     size_t max_rec;                /* capacity of the per-read arrays */
     size_t err_rec[MAX_TEAM]; int err_code[MAX_TEAM];
@@ -977,6 +982,116 @@ static void fq_buffer(team_t *team, frame_ctx *F, size_t *n_out, size_t *n_compl
     *n_out = n; *n_complete = F->n_rec; *used = F->end_of_records;
 }
 
+/* ---- wrapped FASTA framer ---------------------------------------------------------------------- */
+/* A header is a line that begins with '>', a record its header and every line up to the next header.  A line's
+ * role follows from its first byte, so pass 1 lets every worker count the headers that start in its segment; pass
+ * 2 parses the records whose header lies in the segment, walking past its end as far as the record goes, and sums
+ * their sequence bytes; pass 3 copies each worker's sequences to where the sums of the workers before it put them.
+ * The rules are those of wrap_keep_kernel and wrap_record_kernel, so a chunk the device flagged is re-framed here
+ * with the same verdict. */
+static void wr_count_part(void *c_, int part, int nparts) {
+    frame_ctx *c = (frame_ctx *)c_;
+    const size_t a = c->fill * (size_t)part / (size_t)nparts, b = c->fill * (size_t)(part + 1) / (size_t)nparts;
+    size_t n = 0, first = c->fill;
+    if (a == 0 && b > 0 && c->buf[0] == '>') { n = 1; first = 0; }
+    const char *p = c->buf + (a ? a - 1 : 0), *e = c->buf + (b ? b - 1 : 0);   /* a '\n' in [a-1, b-1): a line starts in [a, b) */
+    while (p < e) {
+        const char *q = (const char *)memchr(p, '\n', (size_t)(e - p));
+        if (!q) break;
+        if (q[1] == '>') { if (!n) first = (size_t)(q + 1 - c->buf); ++n; }
+        p = q + 1;
+    }
+    c->cnt[part] = n; c->hfirst[part] = first;
+}
+/* The record whose header starts at hs: *name_end ends its name, *len is the length of its joined sequence (which
+ * is written to dst unless that is NULL), *err a UTB_FW_* code or FE_NONE.  Returns where the next record starts. */
+static size_t wr_record(const frame_ctx *c, size_t hs, char *dst, size_t *name_end, uint64_t *len, int *err) {
+    const char *buf = c->buf;
+    const size_t fill = c->fill;
+    const char *q = (const char *)memchr(buf + hs, '\n', fill - hs);
+    const size_t hn = q ? (size_t)(q - buf) : fill;
+    size_t s = q ? hn + 1 : fill;
+    *err = s - hs >= UTB_LINELEN ? UTB_FW_TOOLONG : FE_NONE;
+    size_t e = hs + 1;                                             /* name: up to the first ' ' or the line end, as for FASTA */
+    while (e < hn && buf[e] != ' ') ++e;
+    *name_end = e;
+    uint64_t n = 0;
+    while (s < fill && buf[s] != '>') {                            /* the sequence lines */
+        const char *r = (const char *)memchr(buf + s, '\n', fill - s);
+        const size_t end = r ? (size_t)(r - buf) : fill, next = r ? end + 1 : fill;
+        if (next - s >= UTB_LINELEN) *err = UTB_FW_TOOLONG;
+        size_t k = end - s;
+        if (k && buf[end - 1] == '\r') --k;                        /* one '\r' before the line end or the end of the input */
+        if (dst) memcpy(dst + n, buf + s, k);
+        n += k;
+        s = next;
+    }
+    if (n > UTB_MAXSEQ) *err = UTB_FW_TOOLONG;
+    *len = n;
+    return s;
+}
+static void wr_part(void *c_, int part, int nparts) {
+    frame_ctx *c = (frame_ctx *)c_;
+    (void)nparts;
+    c->err_rec[part] = (size_t)-1; c->err_code[part] = FE_NONE; c->groups[part] = 0; c->jsum[part] = 0;
+    const size_t r1 = c->base[part] + c->cnt[part] < c->n_rec ? c->base[part] + c->cnt[part] : c->n_rec;
+    uint64_t groups = 0, js = 0;
+    size_t hs = c->hfirst[part];
+    for (size_t r = c->base[part]; r < r1; ++r) {
+        size_t ne; uint64_t len; int err;
+        const size_t next = wr_record(c, hs, NULL, &ne, &len, &err);
+        if (err) { c->err_rec[part] = r; c->err_code[part] = err; c->err_at[part] = hs; break; }
+        c->name_off[r] = (uint32_t)(hs + 1);
+        c->name_len[r] = (uint32_t)(ne - hs - 1);
+        c->seq_len[r] = (uint32_t)len;
+        groups += utb_read_slots((uint32_t)len); js += len;
+        if (r == c->n_rec - 1) c->end_of_records = next;
+        hs = next;                                                 /* the next header: this worker's while r + 1 < r1 */
+    }
+    c->groups[part] = groups; c->jsum[part] = js;
+}
+static void wr_copy_part(void *c_, int part, int nparts) {
+    frame_ctx *c = (frame_ctx *)c_;
+    (void)nparts;
+    const size_t r1 = c->base[part] + c->cnt[part] < c->n_valid ? c->base[part] + c->cnt[part] : c->n_valid;
+    uint64_t at = c->jsum[part];
+    for (size_t r = c->base[part]; r < r1; ++r) {
+        size_t ne; uint64_t len; int err;
+        c->seq_off[r] = at;
+        (void)wr_record(c, (size_t)c->name_off[r] - 1, c->join + at, &ne, &len, &err);
+        at += len;
+    }
+}
+static const char *wr_text(int code) {
+    return code == UTB_FW_NOHEADER ? "ERROR: wrapped FASTA input does not begin with '>'"
+                                   : "ERROR: line of 16777216 bytes or more, or sequence of more than 16777214 bases";
+}
+/* Frames buf[0..fill) as wrapped FASTA into F->join: on return *n_out records are valid (those before the first
+ * malformed one), *n_complete were framed (without EOF the record after the last header is carried), *used is the
+ * byte after the last of them (a malformed record: where it starts), *err is UTB_FW_* of the record at index
+ * *n_out or FE_NONE. */
+static void wr_buffer(team_t *team, frame_ctx *F, size_t *n_out, size_t *n_complete, size_t *used, int *err) {
+    *n_out = *n_complete = *used = 0; *err = FE_NONE;
+    F->end_of_records = 0; F->groups_valid = 0;
+    if (!F->fill) return;
+    if (F->buf[0] != '>') { *err = UTB_FW_NOHEADER; return; }
+    team_run(team, wr_count_part, F);
+    size_t h = 0;
+    for (int p = 0; p < team->n; ++p) { F->base[p] = h; h += F->cnt[p]; }
+    F->n_rec = F->eof ? h : h - 1;                                 /* buf[0] is a header, so h >= 1 */
+    if (F->n_rec > F->max_rec) F->n_rec = F->max_rec;              /* the rest comes back with the carry */
+    for (int p = 0; p < team->n; ++p) { F->err_rec[p] = (size_t)-1; F->err_code[p] = FE_NONE; F->groups[p] = 0; F->jsum[p] = 0; }
+    if (F->n_rec) team_run(team, wr_part, F);
+    size_t n = F->n_rec, at = 0;
+    for (int p = 0; p < team->n; ++p) if (F->err_rec[p] < n) { n = F->err_rec[p]; *err = F->err_code[p]; at = F->err_at[p]; }
+    uint64_t j = 0;
+    for (int p = 0; p < team->n; ++p) { const uint64_t k = F->jsum[p]; F->jsum[p] = j; j += k; }
+    F->n_valid = n;
+    if (n) team_run(team, wr_copy_part, F);
+    F->groups_valid = n == F->n_rec;
+    *n_out = n; *n_complete = F->n_rec; *used = *err ? at : F->end_of_records;
+}
+
 /* Host-stage entry points (CPU-only tests drive the framer and the formatter through these). */
 int utb_frame_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
                       uint64_t *seq_off, uint32_t *seq_len, uint32_t *name_off, uint32_t *name_len,
@@ -1027,6 +1142,35 @@ int utb_frame_fastq_records(const char *buf, size_t n, int eof, int threads, siz
     if (err_record) *err_record = nr + 1;
     if (err_code) *err_code = err;
     utb_set_error("%s [record %zu]", fq_text(err), nr + 1);
+    return UTB_ERR_FORMAT;
+}
+
+int utb_frame_wrapped_records(const char *buf, size_t n, int eof, int threads, size_t max_reads,
+                              char *seq_out, size_t seq_cap, uint64_t *seq_off, uint32_t *seq_len,
+                              uint32_t *name_off, uint32_t *name_len,
+                              size_t *n_reads, size_t *used, size_t *err_record, int *err_code) {
+    if ((!buf && n) || (!seq_out && n) || !seq_off || !seq_len || !name_off || !name_len || !n_reads || !used) {
+        utb_set_error("utb_frame_wrapped_records: null argument"); return UTB_ERR_ARG;
+    }
+    if (seq_cap < n) { utb_set_error("utb_frame_wrapped_records: seq_cap %zu is less than the %zu input bytes", seq_cap, n); return UTB_ERR_ARG; }
+    *n_reads = 0; *used = 0;
+    if (err_record) *err_record = 0;
+    if (err_code) *err_code = 0;
+    if (!n) return UTB_OK;
+    team_t team;
+    if (team_init(&team, threads)) { utb_set_error("cannot start worker threads"); return UTB_ERR_NOMEM; }
+    frame_ctx F;
+    memset(&F, 0, sizeof F);
+    F.buf = buf; F.fill = n; F.eof = eof; F.max_rec = max_reads; F.join = seq_out;
+    F.seq_off = seq_off; F.seq_len = seq_len; F.name_off = name_off; F.name_len = name_len;
+    size_t nr, nc, u; int err;
+    wr_buffer(&team, &F, &nr, &nc, &u, &err);
+    team_destroy(&team);
+    *n_reads = nr; *used = u;
+    if (!err) return UTB_OK;
+    if (err_record) *err_record = nr + 1;
+    if (err_code) *err_code = err;
+    utb_set_error("%s [record %zu]", wr_text(err), nr + 1);
     return UTB_ERR_FORMAT;
 }
 
@@ -1138,7 +1282,7 @@ read_loop:
             if (left != (size_t)-1 && left + carry_len <= 3 * RAMP) want = RAMP;
             else if (left != (size_t)-1 && left + carry_len < want + 2 * RAMP && want > 2 * RAMP) want = left + carry_len - 2 * RAMP;
             if (want < carry_len + 4096) want = carry_len + 4096;  /* a carried partial record must be able to complete */
-            if (want < MAX_RECORD(s->fastq ? 4 : 2)) want = MAX_RECORD(s->fastq ? 4 : 2);
+            if (want < MAX_RECORD(s->format != UTB_INPUT_FASTA ? 4 : 2)) want = MAX_RECORD(s->format != UTB_INPUT_FASTA ? 4 : 2);
             if (want < cap) cap = want;
         }
         if (zero_copy) {
@@ -1167,8 +1311,9 @@ read_loop:
              * without '\n', a chunk without a second header. */
             size_t used = 0;
             if (src->eof) { if (buf[fill - 1] == '\n') used = fill; }
-            else if (s->fastq) used = fastq_cut(buf, fill);
-            else for (size_t hi = fill - 1; hi > 0;) {             /* newline at index < fill - 1 followed by '>' */
+            else if (s->format == UTB_INPUT_FASTQ) used = fastq_cut(buf, fill);
+            else for (size_t hi = fill - 1; hi > 0;) {             /* newline at index < fill - 1 followed by '>' (wrapped FASTA:
+                                                                    * always a header, so the chunk ends on a record boundary) */
                 const char *q = (const char *)memrchr(buf, '\n', hi);
                 if (!q) break;
                 const size_t i = (size_t)(q - buf);
@@ -1215,10 +1360,14 @@ read_loop:
         F.seq_off = utb_batch_seq_off(sl->b); F.seq_len = utb_batch_seq_len(sl->b);
         F.name_off = sl->name_off; F.name_len = sl->name_len;
         size_t n, n_complete, end_of_records; int err_code, dangling = 0;
-        if (s->fastq) {                                            /* a truncated record is an error like any other */
+        if (s->format == UTB_INPUT_FASTQ) {                        /* a truncated record is an error like any other */
             F.qual_off = utb_batch_qual_off(sl->b);
             fq_buffer(&rd_team, &F, &n, &n_complete, &end_of_records, &err_code);
             if (err_code) { fmt_err = 1; snprintf(fmt_msg, sizeof fmt_msg, "%s [record %llu]", fq_text(err_code), (unsigned long long)(n_reads_total + n + 1)); }
+        } else if (s->format == UTB_INPUT_FASTA_WRAPPED) {        /* the sequences are joined into the slot's second staging buffer */
+            F.join = utb_batch_join(sl->b);
+            wr_buffer(&rd_team, &F, &n, &n_complete, &end_of_records, &err_code);
+            if (err_code) { fmt_err = 1; snprintf(fmt_msg, sizeof fmt_msg, "%s [record %llu]", wr_text(err_code), (unsigned long long)(n_reads_total + n + 1)); }
         } else {
             frame_buffer(&rd_team, &F, &n, &n_complete, &end_of_records, &err_code, &dangling);
             if (err_code) { fmt_err = 1; snprintf(fmt_msg, sizeof fmt_msg, "%s [L %llu]", fe_text(err_code), (unsigned long long)(n_reads_total + n + 1)); }

@@ -46,8 +46,9 @@ typedef enum {
 int utb_batch_prepare(utb_batch *b, utb_batch_out out, int chunked);
 int utb_batch_submit_ex(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out, uint64_t total_groups);
 int utb_batch_submit_chunk(utb_batch *b, const char *src, size_t n_bytes, size_t n_reads, int do_rc, utb_batch_out out);
-int utb_batch_set_input(utb_batch *b, int fastq, uint32_t min_qual, int chunked);
+int utb_batch_set_input(utb_batch *b, int format, uint32_t min_qual, int chunked);   /* format: UTB_INPUT_* */
 uint64_t *utb_batch_qual_off(utb_batch *b);   /* pinned, per read: where its quality line starts (FASTQ batches) */
+char *utb_batch_join(utb_batch *b);           /* pinned, max_bytes: the joined sequences of a host-framed wrapped-FASTA batch */
 int utb_batch_frame_error(const utb_batch *b, size_t *record, int *code);
 size_t utb_batch_reads(const utb_batch *b);
 uint64_t utb_batch_launches(const utb_batch *b);
