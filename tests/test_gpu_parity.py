@@ -92,16 +92,23 @@ def test_vote_matches_oracle(gpu, dbname, sparse, env):
         h = np.repeat(labs, cnt).astype(np.uint32)
         lists.append(rng.permutation(h))
     lists.append(np.zeros(0, dtype=np.uint32))
+    # sprinkle misses between the hits of every third list: they must be ignored (HIT_MISS, HIT_NOWIN, ids >= max_ix)
+    bad = np.array([0xFFFFFFFF, 0xFFFFFFFE, ctr.max_ix, ctr.max_ix + 1, 0xFFFF, 0x10000, 0xFFFFFFFD], dtype=np.uint64)
+    bad = bad[bad >= ctr.max_ix].astype(np.uint32)
+    for i in range(0, len(lists), 3):
+        h = lists[i]
+        m = bad[rng.integers(0, bad.size, int(rng.integers(1, h.size + 2)))]
+        pos = np.concatenate([np.arange(h.size) * 2 + 1, rng.integers(0, 2 * h.size + 2, m.size)])
+        lists[i] = np.concatenate([h, m])[np.argsort(pos, kind="stable")]
     off = np.zeros(len(lists) + 1, dtype=np.uint64)
     off[1:] = np.cumsum([l.size for l in lists])
-    # sprinkle misses between the hits: they must be ignored
     try:
         res = db.vote_hits(np.concatenate(lists), off, sparse=sparse)
     finally:
         for k in env:
             del os.environ[k]
     for i, h in enumerate(lists):
-        v = orc.vote(h)
+        v = orc.vote(h[h < ctr.max_ix])
         r = res[i]
         assert r["kind"] == v.kind, i
         if v.kind == 0:
