@@ -20,6 +20,8 @@
 //             read is padded to a multiple of 32 positions with >= 1 bad
 //             position, so a 32-mer window can never straddle two reads.
 //   pl      : the same bases as two bit planes per group (sieve on; the sieve kernel's input)
+//   smask   : sieve on: the sieve survivors of every group, one 64-bit mask (forward strand in bits 0-31, reverse
+//             complement in 32-63), written by the sieve kernel, expanded and looked up by queue_lookup_kernel
 //   hits    : sieve on (GG path): per read the labels of its hits back to back from the read's first slot, hcnt[read]
 //             of them; otherwise one u32 per (position, strand), with a 1-bit-per-slot hitmap in the non-GG path
 //   results : one utb_result per read;  text : the output lines
@@ -27,8 +29,8 @@
 // Kernels: nl_count / nl_index / frame_parse (XT_INITIATE_WS, itree.c:860-901),
 // pack_kernel (XT_WORD_SEARCH's 2-bit packing, itree.c:919-926), sieve_kernel
 // (membership pre-filter, one 8-byte fetch per position for both strands, one DRAM
-// line per ~9 positions) and queue_lookup_kernel (XT_getIX32 + xtSuffixBS on the
-// survivors, itree.c:699-730), lookup_kernel (the same without pre-filter, or the
+// line per ~9 positions, survivors as one mask per group) and queue_lookup_kernel
+// (XT_getIX32 + xtSuffixBS on the survivors of the masks, itree.c:699-730), lookup_kernel (the same without pre-filter, or the
 // reference's exact probe sequence), vote_thread / vote_warp / vote_block (full
 // aufbau vote, itree.c:1028-1098), fmt_* (the fprintf lines, itree.c:1032-1096).
 #include <cuda_runtime.h>
@@ -595,33 +597,14 @@ lookup_kernel(DevDB db, const uint64_t *__restrict__ pk, const uint32_t *__restr
 // In one fused kernel every warp waits for its slowest lane, i.e. for the one
 // or two lanes per warp whose word passes the sieve and goes on to the table,
 // while the other ~30 lanes idle.  So the work is split into two dense passes:
-// phase A (sieve_kernel) tests every window against the sieve and appends the
-// survivors to a queue through per-warp chunks; phase B (queue_lookup_kernel)
-// runs the exact lookup over the queue with every lane busy.
-#define Q_CHUNK 128u              // queue slots a warp reserves per atomic (>= 64: two ballots per step)
-#define Q_INVALID 0xFFFFFFFFu
-// A warp's private window into the survivor queue: the global counter sees one
-// atomic per Q_CHUNK survivors instead of one per warp-step.
-struct WarpQueue {
-    uint64_t base;
-    uint32_t used;
-    bool have;
-};
-__device__ __forceinline__ void wq_init(WarpQueue &q) { q.base = 0; q.used = Q_CHUNK; q.have = false; }
-__device__ __forceinline__ void wq_retire(const WarpQueue &q, uint32_t lane, uint32_t *__restrict__ q_slots) {
-    if (q.have) for (uint32_t j = q.used + lane; j < Q_CHUNK; j += 32) q_slots[q.base + j] = Q_INVALID;   // pad the tail
-}
-// make room for c more entries (warp-uniform call); q_cap is a multiple of Q_CHUNK
-__device__ __forceinline__ void wq_reserve(WarpQueue &q, uint32_t c, uint32_t lane, uint32_t *__restrict__ q_slots,
-                                           unsigned long long *__restrict__ q_count, uint64_t q_cap) {
-    if (q.used + c <= Q_CHUNK) return;
-    wq_retire(q, lane, q_slots);
-    unsigned long long nb = 0;
-    if (lane == 0) nb = atomicAdd(q_count, (unsigned long long)Q_CHUNK);
-    q.base = __shfl_sync(0xFFFFFFFFu, nb, 0);
-    q.used = 0;
-    q.have = q.base + Q_CHUNK <= q_cap;                            // beyond capacity: the caller resolves inline
-}
+// phase A (sieve_kernel) tests every window against the sieve and records its
+// survivors as one 64-bit mask per 32-position step (bits 0-31 the forward
+// strand of lanes 0-31, bits 32-63 the reverse complement); phase B
+// (queue_lookup_kernel) expands the masks into a per-warp list and runs the
+// exact lookup over it with every lane busy.  A step's mask sits at the step's
+// index, so phase A needs no reservation, no capacity and no overflow path, and
+// stores one 8-byte word per step whatever the number of survivors.
+//
 // Where the labels of the hits go.  List mode (cnt != null, the GG path): appended to the hit list of the READ the slot
 // belongs to -- the list starts at the read's first slot in `hits`, cnt[read] counts it; rid maps a 32-position
 // group to its read.  The vote then reads one or two sectors per read instead of a hit map plus one gather per hit,
@@ -634,43 +617,6 @@ struct HitSink {
     uint32_t *cnt;
     uint32_t sh;                                                    // log2(slots per group): 5 + (strands == 2)
 };
-__device__ __forceinline__ void sink_put(const HitSink &k, uint32_t slot, uint32_t r) {   // one hit, any thread
-    if (k.cnt) {
-        const uint32_t rd = __ldg(k.rid + (slot >> k.sh));
-        k.hits[((uint64_t)__ldg(k.grp_off + rd) << k.sh) + atomicAdd(k.cnt + rd, 1u)] = r;
-    } else { k.hits[slot] = r; atomicOr(k.hitmap + (slot >> 5), 1u << (slot & 31u)); }
-}
-// queue overflow: the exact lookup right here (rare); x: the window's planes
-__device__ __noinline__ uint32_t resolve_inline(const DevDB &db, uint64_t x, uint32_t slot, const HitSink &sink) {
-    const uint32_t r = kt_lookup(db, planes_to_word(x));
-    if (r == HIT_MISS) return 0;
-    sink_put(sink, slot, r);
-    return 1;
-}
-// Appends the survivors of one warp step (warp-uniform call).  w / rc: the planes of the window and of its reverse
-// complement; the queue keeps planes, phase B turns them into words (only ~2.5 % of the windows get there).
-template <int NSTR>
-__device__ __forceinline__ uint32_t emit_survivors(const DevDB &db, WarpQueue &wq, uint32_t lane, bool passF, bool passR, uint64_t w, uint64_t rc,
-                                                   uint32_t pos, uint64_t *__restrict__ q_words, uint32_t *__restrict__ q_slots,
-                                                   unsigned long long *__restrict__ q_count, uint64_t q_cap, const HitSink &sink) {
-    const uint32_t bF = __ballot_sync(0xFFFFFFFFu, passF);
-    const uint32_t bR = NSTR == 2 ? __ballot_sync(0xFFFFFFFFu, passR) : 0u;
-    const uint32_t cF = __popc(bF), c = cF + __popc(bR);
-    uint32_t nh = 0;
-    if (!c) return 0;
-    wq_reserve(wq, c, lane, q_slots, q_count, q_cap);
-    const uint32_t lt = (1u << lane) - 1u;
-    if (wq.have) {
-        const uint64_t at = wq.base + wq.used;
-        if (passF) { const uint64_t i = at + __popc(bF & lt); q_words[i] = w; q_slots[i] = pos * NSTR; }
-        if (passR) { const uint64_t i = at + cF + __popc(bR & lt); q_words[i] = rc; q_slots[i] = pos * NSTR + 1u; }
-    } else {
-        if (passF) nh += resolve_inline(db, w, pos * NSTR, sink);
-        if (passR) nh += resolve_inline(db, rc, pos * NSTR + 1u, sink);
-    }
-    wq.used += c;
-    return nh;
-}
 
 // Phase A.  Persistent warps; every warp owns a contiguous range of 32-position steps (one step = one
 // group of the packed stream, lane = position) and walks it SV_U steps at a time.  Per step a lane
@@ -679,7 +625,8 @@ __device__ __forceinline__ uint32_t emit_survivors(const DevDB &db, WarpQueue &w
 // minimum of the 17 hashes at positions p .. p+16, taken across lanes with shuffles (doubling: 2, 4, 8,
 // 16, 17), where positions beyond lane 31 belong to the next step -- which is computed one tile ahead
 // and carried over, so nothing is computed twice.  The reverse complement of a window is derived only
-// where its strand is tested.
+// where its strand is tested.  The survivor masks of a tile's steps are gathered in registers (lane u
+// keeps step u's) and stored with one coalesced store from lanes < SV_U; a step without a window gets 0.
 // template parameters of sieve_kernel: SV_U steps per tile (= filter loads in flight per lane), SV_MINB CTAs per SM
 // the register budget is sized for (launch_stages uses U = 6 at 3 CTAs per SM; the measurements are at the launch)
 #define SV_DEAD 0xFFFFFFFFu       // SvStep.blk of a position without a valid window
@@ -708,8 +655,9 @@ template <int NSTR, int SV_U, int SV_MINB>
 __global__ void __launch_bounds__(256, SV_MINB)
 sieve_kernel(DevDB db, const uint64_t *__restrict__ pl, const uint32_t *__restrict__ bad, uint32_t n_pos,
              const uint32_t *__restrict__ n_groups_dev, unsigned long long *__restrict__ counters,
-             uint64_t *__restrict__ q_words, uint32_t *__restrict__ q_slots, unsigned long long *__restrict__ q_count,
-             uint64_t q_cap, const HitSink sink) {
+             uint64_t *__restrict__ smask) {
+    // the last tile of the batch stores the masks of up to SV_U - 1 steps past n_steps: guard groups, masks 0
+    static_assert(SV_U <= (int)PK_GUARD, "a tile must not run past the guard groups");
     if (n_groups_dev) n_pos = *n_groups_dev * 32u;
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t n_steps = n_pos >> 5;                           // n_pos is a multiple of 32; PK_GUARD all-bad groups follow group n_steps - 1
@@ -720,9 +668,7 @@ sieve_kernel(DevDB db, const uint64_t *__restrict__ pl, const uint32_t *__restri
     const uint32_t s1 = s0 + per < n_steps ? (uint32_t)(s0 + per) : n_steps;
     const uint2 *__restrict__ sieve = db.sieve;
     const uint32_t n_lines = db.sv_lines;
-    WarpQueue wq;
-    wq_init(wq);
-    uint32_t nv = 0, nh = 0;
+    uint32_t nv = 0;
     if (s0 < s1) {
         SvStep st[SV_U + 1];
         // groups s and s + 1 feed step s; the pair is carried from step to step (one 8-byte and one 4-byte load per step).
@@ -763,65 +709,133 @@ sieve_kernel(DevDB db, const uint64_t *__restrict__ pl, const uint32_t *__restri
                 v[u] = make_uint2(0, 0);
                 if (st[u].blk != SV_DEAD) v[u] = __ldg(sieve + ((sv_line(x[u], n_lines) << 4) | st[u].blk));
             }
+            uint64_t mk = 0;                                       // lane u: the mask of step s + u
 #pragma unroll
             for (int u = 0; u < SV_U; ++u) {
                 const bool live = st[u].blk != SV_DEAD;
                 if (__any_sync(0xFFFFFFFFu, live)) {               // the padding group behind every read holds no window at all
                     const uint32_t r1 = ~__brev(st[u].w1), r0 = ~__brev(st[u].w0);   // the reverse complement's planes
                     const bool tF = sv_test(v[u], st[u].w1, st[u].w0), tR = NSTR == 2 && sv_test(v[u], r1, r0);
-                    nh += emit_survivors<NSTR>(db, wq, lane, live & tF, live & tR, ((uint64_t)st[u].w1 << 32) | st[u].w0, ((uint64_t)r1 << 32) | r0,
-                                               (s + u) * 32u + lane, q_words, q_slots, q_count, q_cap, sink);
-                    nv += live ? NSTR : 0;                         // nothing is stored for a miss
+                    const uint32_t bF = __ballot_sync(0xFFFFFFFFu, live & tF);
+                    const uint32_t bR = NSTR == 2 ? __ballot_sync(0xFFFFFFFFu, live & tR) : 0u;
+                    if (lane == (uint32_t)u) mk = ((uint64_t)bR << 32) | bF;
+                    nv += live ? NSTR : 0;
                 }
             }
+            if (lane < (uint32_t)SV_U) smask[s + lane] = mk;
             st[0] = st[SV_U];
         }
     }
-    wq_retire(wq, lane, q_slots);
-    for (int o = 16; o; o >>= 1) { nv += __shfl_xor_sync(0xFFFFFFFFu, nv, o); nh += __shfl_xor_sync(0xFFFFFFFFu, nh, o); }
-    if (lane == 0) {
-        const uint32_t cs = (blockIdx.x * 8 + (threadIdx.x >> 5)) & (COUNTER_SLOTS - 1);
-        if (nv) atomicAdd(counters + cs, (unsigned long long)nv);
-        if (nh) atomicAdd(counters + COUNTER_SLOTS + cs, (unsigned long long)nh);
-    }
+    for (int o = 16; o; o >>= 1) nv += __shfl_xor_sync(0xFFFFFFFFu, nv, o);
+    if (lane == 0 && nv) atomicAdd(counters + ((blockIdx.x * 8 + (threadIdx.x >> 5)) & (COUNTER_SLOTS - 1)), (unsigned long long)nv);
 }
 
-// Phase B: one survivor per thread, ONE random 32-byte table access each (no chain to wait for).  LISTS: the hits
-// of a warp that belong to the same read (neighbours in the queue do) reserve their places in that read's list
-// with one atomic and store side by side.
+// Phase B, one survivor per lane (warp-uniform call; lanes with !valid take part but look nothing up): ONE random
+// 32-byte table access (no chain to wait for).  word: the survivor's 2-bit word; slot: position * strands + strand.
+// LISTS: the hits of a warp that belong to the same read (neighbours in step order do) reserve their places in that
+// read's list with one atomic and store side by side.
 template <bool LISTS>
-__global__ void __launch_bounds__(256, 6)
-queue_lookup_kernel(DevDB db, const uint64_t *__restrict__ q_words, const uint32_t *__restrict__ q_slots,
-                    const unsigned long long *__restrict__ q_count, uint64_t q_cap,
-                    const HitSink sink, unsigned long long *__restrict__ counters) {
-    const uint64_t n = *q_count < q_cap ? *q_count : q_cap;       // both multiples of Q_CHUNK: every entry below n was written
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    const uint32_t lane = threadIdx.x & 31u;
-    uint32_t nh = 0, nsect = 0;
-    // n and the stride are multiples of 32: the lanes of a warp leave the loop together
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const uint32_t slot = q_slots[i];
-        uint32_t r = HIT_MISS;
-        if (slot != Q_INVALID) {                                   // else: padding of a retired chunk
-            uint32_t sc;
-            r = kt_lookup(db, planes_to_word(q_words[i]), &sc);   // the queue holds planes (see emit_survivors)
-            nsect += sc;
-        }
-        const bool hit = r != HIT_MISS;
-        nh += hit;
-        if (!LISTS) {
-            if (hit) { sink.hits[slot] = r; atomicOr(sink.hitmap + (slot >> 5), 1u << (slot & 31u)); }
-            continue;
-        }
-        if (!__any_sync(0xFFFFFFFFu, hit)) continue;
-        const uint32_t rd = hit ? __ldg(sink.rid + (slot >> sink.sh)) : 0xFFFFFFFFu;
-        const uint32_t peers = __match_any_sync(0xFFFFFFFFu, rd);
-        const uint32_t leader = (uint32_t)__ffs(peers) - 1u;
-        uint32_t base = 0;
-        if (hit && lane == leader) base = atomicAdd(sink.cnt + rd, (uint32_t)__popc(peers));
-        base = __shfl_sync(0xFFFFFFFFu, base, leader);
-        if (hit) sink.hits[((uint64_t)__ldg(sink.grp_off + rd) << sink.sh) + base + __popc(peers & ((1u << lane) - 1u))] = r;
+__device__ __forceinline__ void survivor_lookup(const DevDB &db, const HitSink &sink, bool valid, uint64_t word, uint32_t slot,
+                                                uint32_t lane, uint32_t &nh, uint32_t &nsect) {
+    uint32_t r = HIT_MISS;
+    if (valid) {
+        uint32_t sc;
+        r = kt_lookup(db, word, &sc);
+        nsect += sc;
     }
+    const bool hit = r != HIT_MISS;
+    nh += hit;
+    if (!LISTS) {
+        if (hit) { sink.hits[slot] = r; atomicOr(sink.hitmap + (slot >> 5), 1u << (slot & 31u)); }
+        return;
+    }
+    if (!__any_sync(0xFFFFFFFFu, hit)) return;
+    const uint32_t rd = hit ? __ldg(sink.rid + (slot >> sink.sh)) : 0xFFFFFFFFu;
+    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, rd);
+    const uint32_t leader = (uint32_t)__ffs(peers) - 1u;
+    uint32_t base = 0;
+    if (hit && lane == leader) base = atomicAdd(sink.cnt + rd, (uint32_t)__popc(peers));
+    base = __shfl_sync(0xFFFFFFFFu, base, leader);
+    if (hit) sink.hits[((uint64_t)__ldg(sink.grp_off + rd) << sink.sh) + base + __popc(peers & ((1u << lane) - 1u))] = r;
+}
+// The survivor of list entry e = (step in round) << 6 | bit of the round from step s0 (warp-uniform call): its window
+// rebuilt from the round's planes (lane l holds p = pl[s0 + l], every lane q = pl[s0 + 32]) -- one funnel shift per
+// plane, ~__brev of both for the reverse complement -- as a 2-bit word, and its slot
+__device__ __forceinline__ void survivor_of(uint32_t e, uint64_t p, uint64_t q, uint64_t s0, uint32_t sh, uint64_t &word, uint32_t &slot) {
+    const uint32_t st = e >> 6, bit = e & 63u;
+    const uint64_t cur = __shfl_sync(0xFFFFFFFFu, p, st), nx = __shfl_sync(0xFFFFFFFFu, p, (st + 1u) & 31u);
+    const uint64_t next = st == 31u ? q : nx;
+    uint32_t w1 = __funnelshift_l((uint32_t)(next >> 32), (uint32_t)(cur >> 32), bit & 31u);
+    uint32_t w0 = __funnelshift_l((uint32_t)next, (uint32_t)cur, bit & 31u);
+    if (bit >= 32u) { w1 = ~__brev(w1); w0 = ~__brev(w0); }        // the reverse complement's planes
+    word = planes_to_word(((uint64_t)w1 << 32) | w0);
+    slot = ((((uint32_t)s0 + st) * 32u + (bit & 31u)) << (sh - 5u)) + (bit >> 5);
+}
+// Phase B.  Persistent warps take rounds of 32 steps in turn; lane l reads the mask and the planes of step s0 + l
+// (mask 0 at or past n_steps: the masks there are guard groups' or stale ones of an earlier, larger batch), one round
+// ahead, so that those loads are not on the path of the lookups.  The set bits are expanded into a warp-private list
+// in shared memory, in step order, as (step in round) << 6 | bit: a popc, a warp scan for the offsets, then every
+// lane writes its own bits.  A round holds at most 32 x 64 entries.  The list is consumed 32 entries at a time; the
+// fewer than 32 left at the end of a round stay in registers as (word, slot), one per lane (lanes < pend), and go
+// first in the next round's first 32, so lanes are idle only in the warp's very last call.
+#define SB_WARPS 8u                // warps per CTA of queue_lookup_kernel
+#define SB_MINB 5u                 // and its CTAs per SM: 48 registers, no spills (at 6, 40 registers and 36 B spilled:
+                                   // 2.86 against 2.15 ms on B200, 1000 W, profiles/r06_bench_l2s_*)
+template <bool LISTS>
+__global__ void __launch_bounds__(SB_WARPS * 32, SB_MINB)
+queue_lookup_kernel(DevDB db, const uint64_t *__restrict__ smask, const uint64_t *__restrict__ pl, uint32_t n_steps,
+                    const uint32_t *__restrict__ n_groups_dev, const HitSink sink, unsigned long long *__restrict__ counters) {
+    __shared__ uint16_t list_all[SB_WARPS][32 * 64];
+    if (n_groups_dev) n_steps = *n_groups_dev;                     // device-side framing: the host only knows an upper bound
+    const uint32_t lane = threadIdx.x & 31u;
+    uint16_t *list = list_all[threadIdx.x >> 5];
+    const uint64_t stride = (uint64_t)gridDim.x * SB_WARPS * 32u;
+    uint32_t nh = 0, nsect = 0;
+    uint32_t pend = 0, p_slot = 0;                                 // carried survivors: lanes < pend hold one each
+    uint64_t p_word = 0;
+    uint64_t s0 = ((uint64_t)blockIdx.x * SB_WARPS + (threadIdx.x >> 5)) * 32u;
+    uint64_t m_nx = 0, p_nx = 0, q_nx = 0;                         // the next round's mask, planes of s0 + lane, of s0 + 32
+    if (s0 < n_steps) {                                            // pl holds n_steps + PK_GUARD groups
+        m_nx = s0 + lane < n_steps ? __ldg(smask + s0 + lane) : 0ull;
+        p_nx = s0 + lane <= n_steps ? __ldg(pl + s0 + lane) : 0ull;
+        q_nx = s0 + 32u <= n_steps ? __ldg(pl + s0 + 32u) : 0ull;
+    }
+    for (; s0 < n_steps; s0 += stride) {
+        uint64_t m = m_nx;
+        const uint64_t p = p_nx, q = q_nx, s1 = s0 + stride;
+        if (s1 < n_steps) {
+            m_nx = s1 + lane < n_steps ? __ldg(smask + s1 + lane) : 0ull;
+            p_nx = s1 + lane <= n_steps ? __ldg(pl + s1 + lane) : 0ull;
+            q_nx = s1 + 32u <= n_steps ? __ldg(pl + s1 + 32u) : 0ull;
+        }
+        const uint32_t c = __popcll(m);
+        uint32_t incl = c;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+            if (lane >= (uint32_t)o) incl += t;
+        }
+        const uint32_t total = __shfl_sync(0xFFFFFFFFu, incl, 31);
+        if (!total) continue;
+        for (uint32_t at = incl - c; m; m &= m - 1, ++at) list[at] = (uint16_t)((lane << 6) | (uint32_t)(__ffsll(m) - 1));
+        __syncwarp();
+        uint32_t next = 0, avail = pend + total;                   // next: first list entry not yet taken
+        for (; avail >= 32u; avail -= 32u) {
+            uint64_t word; uint32_t slot;
+            survivor_of(list[(next + lane - pend) & (32u * 64u - 1u)], p, q, s0, sink.sh, word, slot);
+            if (lane < pend) { word = p_word; slot = p_slot; }
+            next += 32u - pend; pend = 0;
+            survivor_lookup<LISTS>(db, sink, true, word, slot, lane, nh, nsect);
+        }
+        {
+            uint64_t word; uint32_t slot;
+            survivor_of(list[(next + lane - pend) & (32u * 64u - 1u)], p, q, s0, sink.sh, word, slot);
+            if (lane >= pend && lane < avail) { p_word = word; p_slot = slot; }
+        }
+        pend = avail;
+        __syncwarp();                                              // the list is rewritten by the next round
+    }
+    if (pend) survivor_lookup<LISTS>(db, sink, lane < pend, p_word, p_slot, lane, nh, nsect);
     for (int o = 16; o; o >>= 1) { nh += __shfl_xor_sync(0xFFFFFFFFu, nh, o); nsect += __shfl_xor_sync(0xFFFFFFFFu, nsect, o); }
     if (lane == 0) {
         const uint32_t c = blockIdx.x & (COUNTER_SLOTS - 1);
@@ -2611,7 +2625,7 @@ struct utb_batch {
     unsigned long long *d_counters;   // [4][COUNTER_SLOTS]: lookups, hits, good finds, exact-path sectors (summed on the host)
     vote_scratch vs;
     uint32_t *d_sel_cnt, *d_sel_off, *d_sel, *d_sel_gap, *d_sel_total, *h_sel_cnt, *h_sel, *h_sel_total; size_t sel_cap;   // non-GG mode (UTB_OUT_SELECTIONS)
-    uint64_t *d_qwords; uint32_t *d_qslots; unsigned long long *d_qcount; uint64_t q_cap;   // filter survivors (window planes, slots)
+    uint64_t *d_smask;            // filter survivors: one mask per 32-position step (sieve_kernel -> queue_lookup_kernel)
     uint32_t *d_hitmap;
     uint32_t *d_rid, *d_hcnt;     // group -> read, hits per read (list mode of the survivor kernel)
     // last submit
@@ -2656,7 +2670,7 @@ extern "C" void utb_batch_destroy(utb_batch *b) {
     vs_free(&b->vs);
     cudaFree(b->d_sel_cnt); cudaFree(b->d_sel_off); cudaFree(b->d_sel); cudaFree(b->d_sel_gap); cudaFree(b->d_sel_total);
     cudaFreeHost(b->h_sel_cnt); cudaFreeHost(b->h_sel); cudaFreeHost(b->h_sel_total);
-    cudaFree(b->d_qwords); cudaFree(b->d_qslots); cudaFree(b->d_qcount); cudaFree(b->d_hitmap); cudaFree(b->d_rid); cudaFree(b->d_hcnt);
+    cudaFree(b->d_smask); cudaFree(b->d_hitmap); cudaFree(b->d_rid); cudaFree(b->d_hcnt);
     cudaFree(b->d_nl); cudaFree(b->d_blk); cudaFree(b->d_frame_err); cudaFreeHost(b->h_frame_err);
     cudaFree(b->d_frame_info); cudaFree(b->d_dims); cudaFreeHost(b->h_dims);
     cudaFreeHost(b->h_qual_off); cudaFree(b->d_qual_off);
@@ -2717,15 +2731,8 @@ extern "C" int utb_batch_create(utb_db *db, size_t max_bytes, size_t max_reads, 
     if (vs_alloc(db, max_bytes, &b->vs)) { utb_batch_destroy(b); return UTB_ERR_CUDA; }
     BK(cudaMemset(b->d_raw, 0, max_bytes + 128));
     b->d_pack = b->d_raw;
-    if (db->sieve) {                                               // queue for a quarter of the lookup slots; overflow resolves inline
-        b->q_cap = npos * 2 / 4 + 4096;
-        const char *qc = getenv("UTB_QCAP");                       // tests: a tiny queue forces the overflow path
-        if (qc && atoll(qc) > 0) b->q_cap = (uint64_t)atoll(qc);
-        b->q_cap = (b->q_cap + Q_CHUNK - 1) / Q_CHUNK * Q_CHUNK;    // whole chunks: the consumer reads [0, min(count, cap)) and every entry of it is written
-        BK(cudaMalloc(&b->d_qwords, b->q_cap * 8));
-        BK(cudaMalloc(&b->d_qslots, b->q_cap * 4));
-        BK(cudaMemset(b->d_qslots, 0xFF, b->q_cap * 4));            // Q_INVALID
-        BK(cudaMalloc(&b->d_qcount, 8));
+    if (db->sieve) {
+        BK(cudaMalloc(&b->d_smask, (b->max_groups + PK_GUARD + 2) * 8));
         BK(cudaMalloc(&b->d_hitmap, (npos * 2 / 32 + 8) * 4));
         BK(cudaMalloc(&b->d_pl, (b->max_groups + PK_GUARD + 2) * 8));
         BK(cudaMalloc(&b->d_rid, (b->max_groups + PK_GUARD + 2) * 4));
@@ -2780,7 +2787,6 @@ static int launch_stages(utb_batch *b, bool timed) {
         const unsigned sms = (unsigned)b->db->sm_count;
         b->used_sieve = sieve; b->used_lists = 0;
         if (two_phase) {
-            CK(cudaMemsetAsync(b->d_qcount, 0, 8, b->st));
             // hits are sparse (only sieve survivors that really match).  GG path: the survivor kernel files every label
             // under its read (list mode, see HitSink); non-GG path: by slot, flagged in a 1-bit-per-slot map
             HitSink sink;
@@ -2793,19 +2799,21 @@ static int launch_stages(utb_batch *b, bool timed) {
             b->used_lists = lists;
             if (timed) CK(cudaEventRecord(b->ev[4], b->st));
             // persistent: MINB CTAs per SM, every warp a contiguous range of steps (small batches: one tile per warp)
-            // measured on B200 (1000 W), 10 M x 150 bp, windows from bit planes (profiles/r03_bench_l2s_*): U = 6 steps per
-            // tile at 3 CTAs per SM (80 registers, no spills) 7.86 ms; (6, 4) 7.98 (64 registers, 88 B spilled); (8, 3)
-            // 8.03 (32 B spilled).  Before, from 2-bit words (r02_sieve_variants.txt): (6, 3) 8.54; (5, 3) 8.60; (4, 3)
-            // 8.81; (4, 4) 8.98; (6, 2) 9.66 -- instructions per step, not occupancy, decide
+            // measured on B200 (1000 W), 10 M x 150 bp, survivors as masks (profiles/README.md, round 6): U = 6 steps per
+            // tile at 3 CTAs per SM (80 registers, no spills) 6.27 ms; (6, 4) 6.24 (64 registers, 12 B spilled); (8, 3)
+            // 6.28 (80 registers, no spills) -- one run each, within 0.5 %.  With the survivor queue (r03_bench_l2s_*):
+            // (6, 3) 7.86; (6, 4) 7.98 (88 B spilled); (8, 3) 8.03 (32 B spilled).  From 2-bit words
+            // (r02_sieve_variants.txt): (6, 3) 8.54; (5, 3) 8.60; (4, 3) 8.81; (4, 4) 8.98; (6, 2) 9.66 -- instructions
+            // per step, not occupancy, decide
             constexpr unsigned U = 6, MINB = 3;
             const unsigned wb = (n_groups + 8u * U - 1) / (8u * U);
             const unsigned pb = wb < sms * MINB ? (wb ? wb : 1u) : sms * MINB;
             const uint32_t *sv_groups = b->dims_dev ? b->dims_dev + 1 : nullptr;
-            if (nstr == 2) sieve_kernel<2, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pl, b->d_bad, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
-            else sieve_kernel<1, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pl, b->d_bad, n_pos, sv_groups, b->d_counters, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink);
+            if (nstr == 2) sieve_kernel<2, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pl, b->d_bad, n_pos, sv_groups, b->d_counters, b->d_smask);
+            else sieve_kernel<1, U, MINB><<<pb, 256, 0, b->st>>>(d, b->d_pl, b->d_bad, n_pos, sv_groups, b->d_counters, b->d_smask);
             if (timed) CK(cudaEventRecord(b->ev[5], b->st));
-            if (lists) queue_lookup_kernel<true><<<sms * 6, 256, 0, b->st>>>(d, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink, b->d_counters);
-            else queue_lookup_kernel<false><<<sms * 6, 256, 0, b->st>>>(d, b->d_qwords, b->d_qslots, b->d_qcount, b->q_cap, sink, b->d_counters);
+            if (lists) queue_lookup_kernel<true><<<sms * SB_MINB, SB_WARPS * 32, 0, b->st>>>(d, b->d_smask, b->d_pl, n_groups, sv_groups, sink, b->d_counters);
+            else queue_lookup_kernel<false><<<sms * SB_MINB, SB_WARPS * 32, 0, b->st>>>(d, b->d_smask, b->d_pl, n_groups, sv_groups, sink, b->d_counters);
             b->launches++;
         } else if (b->db->use_table) {
             if (nstr == 2) lookup_kernel<2, true><<<nb, 256, 0, b->st>>>(d, b->d_pk, b->d_bad, n_pos, b->dims_dev ? b->dims_dev + 1 : nullptr, b->d_hits, b->d_counters);
@@ -3284,7 +3292,7 @@ extern "C" int utb_batch_last_ms(utb_batch *b, float ms[4]) {
     return UTB_OK;
 }
 extern "C" uint64_t utb_batch_launches(const utb_batch *b) { return b ? b->launches : 0; }
-// Two-phase detail of the LAST run (valid after wait): ms[0] filter kernel, ms[1] queue kernel (0/0 when the
+// Two-phase detail of the LAST run (valid after wait): ms[0] filter kernel, ms[1] survivor kernel (0/0 when the
 // single lookup kernel ran); sectors[0] = lookups answered by the filter (one sector per position, both
 // strands), sectors[1] = sectors the exact path touched for the survivors.
 extern "C" int utb_batch_lookup_detail(utb_batch *b, float ms[2], uint64_t sectors[2]) {
