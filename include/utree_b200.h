@@ -316,6 +316,47 @@ int utb_main_shallow(int argc, char **argv);
 enum { UTB_INPUT_FASTA = 0, UTB_INPUT_FASTQ = 1, UTB_INPUT_FASTA_WRAPPED = 2 };
 int utb_searcher_set_input(utb_searcher *s, int format, uint32_t min_qual);
 
+/* ---- sample profile ----------------------------------------------------------- */
+/* The profile of a search maps each distinct taxonomy string (column 2 of the
+ * output lines: label `label` cut to `len` bytes, exactly what the line
+ * prints) to the number of reads whose line carries it.  Reads without a
+ * line are unclassified: unclassified = stats.reads - stats.good_finds, and
+ * the row counts add up to good_finds.
+ *   rows       one per distinct string.  Results that print the same bytes
+ *              with different labels (a cut in the middle of a token, the
+ *              empty cut, a full label that is a prefix of another label)
+ *              are one row, whose label is the smallest id among them.
+ *   order      unsigned byte order of the strings, a string before any
+ *              longer string it is a prefix of (the empty string first).
+ *   errors     after UTB_ERR_FORMAT the profile counts exactly the reads
+ *              whose lines were written before the bad record.
+ * set_profile(s, 1) allocates what the profile needs on every device (nothing
+ * is allocated on a device inside a search); every later search starts from
+ * an empty profile.  With the profile on, utb_search_file accepts
+ * out_path == NULL and utb_search_mem accepts out == NULL && out_len == NULL:
+ * then no output text is built or copied (stats.out_bytes == 0), only the
+ * profile.  With an output given, the lines and the profile come from one
+ * pass.  With the profile off every search behaves as without this call.
+ * The profile is counted on the devices, per batch, and merged on the host
+ * for the batches whose lines are emitted.  It is not available for the
+ * non-GG search: set_profile(s, 1) on a shallow searcher and
+ * utb_searcher_set_shallow(s, 1) on a profiling one fail with UTB_ERR_ARG.
+ * utb_searcher_profile gives the rows of the last search (owned by the
+ * searcher) after it returned UTB_OK or UTB_ERR_FORMAT, until the next
+ * search; otherwise it fails with UTB_ERR_ARG. */
+typedef struct { uint32_t label; uint32_t len; uint64_t reads; } utb_profile_row;
+int utb_searcher_set_profile(utb_searcher *s, int on);
+int utb_searcher_profile(const utb_searcher *s, const utb_profile_row **rows, size_t *n_rows, uint64_t *unclassified);
+/* utree-profile [-r] [-t threads] [-f fasta|fastq|wrapped] [-q min_qual]
+ *               compTree.ctr table.tsv reads1 [reads2 ...]
+ * One searcher profiles every sample in order and writes one TSV table:
+ * "#taxonomy\t<reads1>\t...", "#unclassified\t<n1>\t...", then one line per
+ * string counted in any sample, in row order.  Exit codes: 0 ok; 1 usage,
+ * unreadable CTR or input, unwritable table; 2 a malformed sample (no table
+ * is written); 3 out of memory or a truncated CTR; 4 no sm_100 GPU or a CUDA
+ * error. */
+int utb_profile_main(int argc, char **argv);
+
 /* ---- utree-compress equivalent (XT_cmp32, itree.c:1234-1315; SURVEY 8f-2) -- */
 /* .ubt -> .ctr, byte-identical to the reference compressor (first-bin quirk
  * included).  Host only. */

@@ -41,7 +41,7 @@ def _newer(target, sources):
 
 
 def build(force=False, verbose=False):
-    srcs = [os.path.join(CSRC, f) for f in C_SOURCES + ["kernels.cu", "builder.cu", "utb_internal.h", "main.c", "main_shallow.c", "compress_main.c", "build_main.c"]]
+    srcs = [os.path.join(CSRC, f) for f in C_SOURCES + ["kernels.cu", "builder.cu", "utb_internal.h", "main.c", "main_shallow.c", "main_profile.c", "compress_main.c", "build_main.c"]]
     srcs.append(os.path.join(ROOT, "include", "utree_b200.h"))
     exe = os.path.join(BIN, "utree-search_gg")
     if not force and _newer(LIB, srcs) and _newer(exe, srcs):
@@ -67,6 +67,8 @@ def build(force=False, verbose=False):
     shutil.copyfile(exe, os.path.join(BIN, "utree-searchGG"))
     os.chmod(os.path.join(BIN, "utree-searchGG"), 0o755)
     _run([GCC] + C_FLAGS + [os.path.join(CSRC, "main_shallow.c"), "-o", os.path.join(BIN, "utree-search"), "-L" + CSRC, "-lutree_b200",
+                            "-Wl,-rpath,$ORIGIN/../utree_b200/csrc"], log)
+    _run([GCC] + C_FLAGS + [os.path.join(CSRC, "main_profile.c"), "-o", os.path.join(BIN, "utree-profile"), "-L" + CSRC, "-lutree_b200",
                             "-Wl,-rpath,$ORIGIN/../utree_b200/csrc"], log)
     _run([GCC] + C_FLAGS + [os.path.join(CSRC, "build_main.c"), "-o", os.path.join(BIN, "utree-build_gg"), "-L" + CSRC, "-lutree_b200",
                             "-Wl,-rpath,$ORIGIN/../utree_b200/csrc"], log)

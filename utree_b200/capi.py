@@ -53,7 +53,8 @@ EXPORTS = [
     "utb_batch_submit", "utb_batch_wait", "utb_batch_name_off", "utb_batch_name_len", "utb_batch_rerun_device", "utb_batch_counts", "utb_batch_lookup_detail", "utb_db_clone", "utb_db_device",
     "utb_lookup_words", "utb_pack_sequence", "utb_vote_hits", "utb_vote_hits_sparse", "utb_frame_records", "utb_frame_fastq_records", "utb_frame_wrapped_records", "utb_format_results",
     "utb_searcher_create", "utb_searcher_destroy", "utb_search_file", "utb_search_mem", "utb_free",
-    "utb_main", "utb_main_shallow", "utb_build_ubt", "utb_build_main", "utb_searcher_set_shallow", "utb_searcher_set_input", "utb_measure_rand32", "utb_compress_ubt", "utb_compress_main",
+    "utb_main", "utb_main_shallow", "utb_build_ubt", "utb_build_main", "utb_searcher_set_shallow", "utb_searcher_set_input",
+    "utb_searcher_set_profile", "utb_searcher_profile", "utb_profile_main", "utb_measure_rand32", "utb_compress_ubt", "utb_compress_main",
 ]
 
 _lib = None
@@ -345,6 +346,10 @@ class Batch:
             self.h = C.c_void_p()
 
 
+class ProfileRow(C.Structure):
+    _fields_ = [("label", C.c_uint32), ("len", C.c_uint32), ("reads", C.c_uint64)]
+
+
 class Searcher:
     """Whole search over one or more GPUs (utb_searcher_* / utb_search_*)."""
 
@@ -369,18 +374,38 @@ class Searcher:
         fmt = INPUT_FASTQ if fastq else INPUT_FASTA_WRAPPED if wrapped else INPUT_FASTA
         _ck(lib().utb_searcher_set_input(self.h, fmt, min_qual))
 
+    def set_profile(self, on=True):
+        """Count reads per taxonomy string in the following searches (utb_searcher_set_profile)."""
+        lib().utb_searcher_set_profile.argtypes = [C.c_void_p, C.c_int]
+        _ck(lib().utb_searcher_set_profile(self.h, int(on)))
+
+    def profile(self):
+        """The last search's profile (utb_searcher_profile): ([(taxonomy bytes, reads, label)] in row order,
+        unclassified reads)."""
+        L = lib()
+        L.utb_searcher_profile.argtypes = [C.c_void_p, C.POINTER(C.POINTER(ProfileRow)), C.POINTER(C.c_size_t), C.POINTER(C.c_uint64)]
+        rows, n, uncl = C.POINTER(ProfileRow)(), C.c_size_t(), C.c_uint64()
+        _ck(L.utb_searcher_profile(self.h, C.byref(rows), C.byref(n), C.byref(uncl)))
+        return [(self.ctr.label(rows[i].label)[:rows[i].len], rows[i].reads, rows[i].label) for i in range(n.value)], uncl.value
+
     def search_file(self, fasta, out, do_rc=True):
+        """out=None: no output file (with the profile on: the profile alone)."""
         st, ex = Stats(), C.c_int()
-        rc = lib().utb_search_file(self.h, os.fsencode(fasta), os.fsencode(out), int(do_rc), C.byref(st), C.byref(ex))
+        rc = lib().utb_search_file(self.h, os.fsencode(fasta), None if out is None else os.fsencode(out), int(do_rc),
+                                   C.byref(st), C.byref(ex))
         return rc, ex.value, st.as_dict()
 
-    def search_mem(self, fasta: bytes, do_rc=True, ptr=None, n=None, copy=True):
-        """copy=False: the output text is not copied into Python (returns its length instead)."""
+    def search_mem(self, fasta: bytes, do_rc=True, ptr=None, n=None, copy=True, text=True):
+        """copy=False: the output text is not copied into Python (returns its length instead).  text=False: no output
+        is asked for (NULL out and out_len; with the profile on: the profile alone); returns None for the text."""
         st, ex = Stats(), C.c_int()
         out, out_len = C.c_void_p(), C.c_size_t()
         if ptr is None:
             keep = C.create_string_buffer(fasta, len(fasta))
             ptr, n = C.addressof(keep), len(fasta)
+        if not text:
+            rc = lib().utb_search_mem(self.h, ptr, n, int(do_rc), None, None, C.byref(st), C.byref(ex))
+            return rc, ex.value, None, st.as_dict()
         rc = lib().utb_search_mem(self.h, ptr, n, int(do_rc), C.byref(out), C.byref(out_len), C.byref(st), C.byref(ex))
         data = out_len.value
         if copy:

@@ -2196,6 +2196,79 @@ fmt_write_kernel(DevDB db, const utb_result *__restrict__ res, const uint8_t *__
 }
 
 // ---------------------------------------------------------------------------
+// Sample profile: reads per printed taxonomy string, counted per batch.  The key of a read with a line is
+// (label << 32) | printed length; the host merges keys that print the same bytes.  A few taxa take most reads in a
+// typical sample, so lanes of a warp that share a key are merged first (one atomic per distinct key per warp), into
+// a per-CTA table in shared memory; a key that finds no shared slot within PF_PROBE steps goes to the batch's global
+// table, which holds at least twice the keys a batch can have and so never fills.  The thread that creates a global
+// key appends its slot to the batch's list; profile_compact_kernel gathers (key, count) from the list and clears
+// those slots, so the table is clean for the next batch without a whole-table memset.
+// ---------------------------------------------------------------------------
+#define PF_THREADS 256
+#define PF_SLOTS 2048                                              // per CTA: 16 KiB of keys + 8 KiB of counts
+#define PF_PROBE 16
+#define PF_EMPTY 0xFFFFFFFFFFFFFFFFull                             // no key: label < max_ix < 2^32 - 1
+__device__ __forceinline__ uint32_t pf_hash(unsigned long long key) {
+    return (uint32_t)((key * 0x9E3779B97F4A7C15ull) >> 32);
+}
+__device__ __forceinline__ void pf_global_add(unsigned long long key, uint32_t c, unsigned long long *__restrict__ tkey,
+                                              uint32_t *__restrict__ tcnt, uint32_t tmask, uint32_t *__restrict__ list,
+                                              uint32_t *__restrict__ n_keys) {
+    for (uint32_t s = pf_hash(key) & tmask;; s = (s + 1u) & tmask) {
+        const unsigned long long k = tkey[s];
+        const unsigned long long prev = k == key || k != PF_EMPTY ? k : atomicCAS(tkey + s, PF_EMPTY, key);
+        if (prev == PF_EMPTY) list[atomicAdd(n_keys, 1u)] = s;
+        if (prev == PF_EMPTY || prev == key) { atomicAdd(tcnt + s, c); return; }
+    }
+}
+__global__ void __launch_bounds__(PF_THREADS)
+profile_kernel(DevDB db, const utb_result *__restrict__ res, uint32_t n_reads, const uint32_t *__restrict__ dims,
+               unsigned long long *__restrict__ tkey, uint32_t *__restrict__ tcnt, uint32_t tmask,
+               uint32_t *__restrict__ list, uint32_t *__restrict__ n_keys) {
+    if (dims) n_reads = dims[0];
+    __shared__ unsigned long long s_key[PF_SLOTS];
+    __shared__ uint32_t s_cnt[PF_SLOTS];
+    for (uint32_t i = threadIdx.x; i < PF_SLOTS; i += PF_THREADS) { s_key[i] = PF_EMPTY; s_cnt[i] = 0; }
+    __syncthreads();
+    const uint32_t lane = threadIdx.x & 31u;
+    // the loop bound is uniform per CTA, so every lane of a warp takes part in each __match_any_sync
+    for (uint64_t base = (uint64_t)blockIdx.x * PF_THREADS; base < n_reads; base += (uint64_t)gridDim.x * PF_THREADS) {
+        const uint64_t r = base + threadIdx.x;
+        unsigned long long key = PF_EMPTY;
+        if (r < n_reads) {
+            const utb_result v = res[r];
+            if (v.kind != UTB_NONE) key = ((unsigned long long)v.label << 32) | tax_len_of(db, v);
+        }
+        const uint32_t same = __match_any_sync(0xFFFFFFFFu, key);
+        if (key == PF_EMPTY || lane != (uint32_t)__ffs(same) - 1u) continue;
+        const uint32_t c = (uint32_t)__popc(same);
+        uint32_t s = pf_hash(key) & (PF_SLOTS - 1u);
+        bool done = false;
+        for (int p = 0; p < PF_PROBE && !done; ++p, s = (s + 1u) & (PF_SLOTS - 1u)) {
+            const unsigned long long k = s_key[s];
+            const unsigned long long prev = k == key || k != PF_EMPTY ? k : atomicCAS(s_key + s, PF_EMPTY, key);
+            if (prev == PF_EMPTY || prev == key) { atomicAdd(s_cnt + s, c); done = true; }
+        }
+        if (!done) pf_global_add(key, c, tkey, tcnt, tmask, list, n_keys);
+    }
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < PF_SLOTS; i += PF_THREADS)
+        if (s_key[i] != PF_EMPTY) pf_global_add(s_key[i], s_cnt[i], tkey, tcnt, tmask, list, n_keys);
+}
+__global__ void __launch_bounds__(256)
+profile_compact_kernel(unsigned long long *__restrict__ tkey, uint32_t *__restrict__ tcnt, const uint32_t *__restrict__ list,
+                       const uint32_t *__restrict__ n_keys, unsigned long long *__restrict__ out) {
+    const uint32_t n = *n_keys;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const uint32_t s = list[i];
+        out[2 * i] = tkey[s];
+        out[2 * i + 1] = tcnt[s];
+        tkey[s] = PF_EMPTY;
+        tcnt[s] = 0;
+    }
+}
+
+// ---------------------------------------------------------------------------
 // random-sector gather microbenchmark (roofline denominator, SURVEY 8d)
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
@@ -2645,6 +2718,10 @@ struct utb_batch {
     int wrapped; const uint8_t *d_pack;                            // pack_kernel's input: d_raw, or d_join
     char *h_join; uint8_t *d_join;
     uint32_t *d_wt, *d_wsums, *d_wtotal; uint64_t *d_kmask; size_t wt_cap;
+    // sample profile (utb_batch_set_profile): 0 off, 1 with the text, 2 instead of the text.  Global key table of
+    // pf_mask + 1 slots, list of the slots in use, (key, count) pairs of the last batch on the device and host
+    int profile; uint32_t pf_mask; size_t pf_keys;
+    unsigned long long *d_pf_key, *d_pf_out, *h_pf_out; uint32_t *d_pf_cnt, *d_pf_list, *d_pf_n, *h_pf_n;
 };
 
 extern "C" uint64_t utb_read_slots(uint32_t len) { return ((uint64_t)len + 1 + 31) / 32; }
@@ -2675,6 +2752,8 @@ extern "C" void utb_batch_destroy(utb_batch *b) {
     cudaFree(b->d_frame_info); cudaFree(b->d_dims); cudaFreeHost(b->h_dims);
     cudaFreeHost(b->h_qual_off); cudaFree(b->d_qual_off);
     cudaFreeHost(b->h_join); cudaFree(b->d_join); cudaFree(b->d_wt); cudaFree(b->d_wsums); cudaFree(b->d_wtotal); cudaFree(b->d_kmask);
+    cudaFree(b->d_pf_key); cudaFree(b->d_pf_cnt); cudaFree(b->d_pf_list); cudaFree(b->d_pf_out); cudaFree(b->d_pf_n);
+    cudaFreeHost(b->h_pf_out); cudaFreeHost(b->h_pf_n);
     if (b->done) cudaEventDestroy(b->done);
     for (int i = 0; i < 7; ++i) if (b->ev[i]) cudaEventDestroy(b->ev[i]);
     if (b->st) cudaStreamDestroy(b->st);
@@ -3005,7 +3084,7 @@ static int finish_submit(utb_batch *b) {
         // lines built on the device: lengths -> exclusive scan -> one warp per read writes its line
         const uint32_t n = (uint32_t)n_reads, nt = (n + SCAN_TILE - 1) / SCAN_TILE;
         CK(cudaMemsetAsync(b->d_text_len, 0, 4, b->st));
-        if (n) {
+        if (n && b->profile != 2) {
             fmt_len_kernel<<<gs_grid(b, n, 256, 16), 256, 0, b->st>>>(b->db->d, b->d_results, b->d_name_len, n, b->dims_dev, b->d_line_len);
             scan_sums_kernel<false><<<gs_grid(b, nt, 1, 8), 256, 0, b->st>>>(b->d_line_len, n, b->dims_dev, nt, b->d_scan_sums);
             scan_top_kernel<false><<<1, 1024, 0, b->st>>>(b->d_scan_sums, nt, b->d_text_len);
@@ -3016,6 +3095,19 @@ static int finish_submit(utb_batch *b) {
             CK(cudaGetLastError());
         }
         CK(cudaMemcpyAsync(b->h_text_len, b->d_text_len, 4, cudaMemcpyDeviceToHost, b->st));
+        if (b->profile) {
+            // reads per printed (label, length) key; the pairs stay on the device until the host accepts the batch
+            CK(cudaMemsetAsync(b->d_pf_n, 0, 4, b->st));
+            if (n) {
+                const size_t nk = b->pf_keys < n ? b->pf_keys : n;
+                profile_kernel<<<gs_grid(b, n, PF_THREADS, 2), PF_THREADS, 0, b->st>>>(
+                    b->db->d, b->d_results, n, b->dims_dev, b->d_pf_key, b->d_pf_cnt, b->pf_mask, b->d_pf_list, b->d_pf_n);
+                profile_compact_kernel<<<gs_grid(b, nk, 256, 4), 256, 0, b->st>>>(b->d_pf_key, b->d_pf_cnt, b->d_pf_list, b->d_pf_n, b->d_pf_out);
+                b->launches += 2;
+                CK(cudaGetLastError());
+            }
+            CK(cudaMemcpyAsync(b->h_pf_n, b->d_pf_n, 4, cudaMemcpyDeviceToHost, b->st));
+        }
     } else if (n_reads) CK(cudaMemcpyAsync(b->h_results, b->d_results, n_reads * sizeof(utb_result), cudaMemcpyDeviceToHost, b->st));
     if (b->dims_dev) CK(cudaMemcpyAsync(b->h_dims, b->d_dims, 8, cudaMemcpyDeviceToHost, b->st));
     CK(cudaMemcpyAsync(b->h_counters, b->d_counters, 4 * COUNTER_SLOTS * 8, cudaMemcpyDeviceToHost, b->st));
@@ -3265,6 +3357,50 @@ extern "C" int utb_batch_text_piece(utb_batch *b, size_t off, size_t *len, const
     if (*len) CK(cudaMemcpyAsync(b->h_text, b->d_text + off, *len, cudaMemcpyDeviceToHost, b->st));
     CK(cudaStreamSynchronize(b->st));
     *piece = b->h_text;
+    return UTB_OK;
+}
+// The sample profile of the batch's later submits (mode 0 off, 1 with the text, 2 instead of the text).  The first
+// call with mode != 0 allocates the key table for at most max_keys distinct keys per batch (fewer when the batch has
+// fewer reads): a power of two at least twice that, so a probe always ends.
+extern "C" int utb_batch_set_profile(utb_batch *b, int mode, size_t max_keys) {
+    if (!b || mode < 0 || mode > 2 || (mode && !max_keys)) { utb_set_error("utb_batch_set_profile: bad argument"); return UTB_ERR_ARG; }
+    if (mode && !b->d_pf_key) {
+        CK(cudaSetDevice(b->db->device));
+        const size_t nk = max_keys < b->max_reads ? max_keys : b->max_reads;
+        size_t slots = 1;
+        while (slots < 2 * nk) slots <<= 1;
+        if (slots > ((size_t)1 << 32)) { utb_set_error("utb_batch_set_profile: key table too large"); return UTB_ERR_LIMIT; }
+        void *p[5] = {nullptr, nullptr, nullptr, nullptr, nullptr}, *h[2] = {nullptr, nullptr};
+        cudaError_t e = cudaMalloc(&p[0], slots * 8);
+        if (e == cudaSuccess) e = cudaMalloc(&p[1], slots * 4);
+        if (e == cudaSuccess) e = cudaMalloc(&p[2], nk * 4);
+        if (e == cudaSuccess) e = cudaMalloc(&p[3], nk * 16);
+        if (e == cudaSuccess) e = cudaMalloc(&p[4], 4);
+        if (e == cudaSuccess) e = cudaMallocHost(&h[0], nk * 16);
+        if (e == cudaSuccess) e = cudaMallocHost(&h[1], 4);
+        if (e == cudaSuccess) e = cudaMemset(p[0], 0xFF, slots * 8);
+        if (e == cudaSuccess) e = cudaMemset(p[1], 0, slots * 4);
+        if (e != cudaSuccess) { for (int i = 0; i < 5; ++i) cudaFree(p[i]); cudaFreeHost(h[0]); cudaFreeHost(h[1]); CK(e); }
+        b->d_pf_key = (unsigned long long *)p[0]; b->d_pf_cnt = (uint32_t *)p[1]; b->d_pf_list = (uint32_t *)p[2];
+        b->d_pf_out = (unsigned long long *)p[3]; b->d_pf_n = (uint32_t *)p[4];
+        b->h_pf_out = (unsigned long long *)h[0]; b->h_pf_n = (uint32_t *)h[1];
+        b->pf_mask = (uint32_t)(slots - 1); b->pf_keys = nk;
+    }
+    b->profile = mode;
+    return UTB_OK;
+}
+// After the wait of a profiled batch: its distinct keys as *n (key, count) pairs, copied into page-locked memory of the
+// batch (valid until its next submit); blocks until they are there.
+extern "C" int utb_batch_profile(utb_batch *b, const uint64_t **pairs, size_t *n) {
+    if (!b || !pairs || !n || !b->profile) { utb_set_error("utb_batch_profile: bad argument"); return UTB_ERR_ARG; }
+    const size_t k = *b->h_pf_n;
+    if (k > b->pf_keys) { utb_set_error("profile key list overflow"); return UTB_ERR_LIMIT; }
+    CK(cudaSetDevice(b->db->device));
+    if (k) {
+        CK(cudaMemcpyAsync(b->h_pf_out, b->d_pf_out, k * 16, cudaMemcpyDeviceToHost, b->st));
+        CK(cudaStreamSynchronize(b->st));
+    }
+    *pairs = (const uint64_t *)b->h_pf_out; *n = k;
     return UTB_OK;
 }
 extern "C" int utb_batch_sync(utb_batch *b) {

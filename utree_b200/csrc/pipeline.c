@@ -127,6 +127,13 @@ struct utb_searcher {
     int spread;                    /* more than one physical GPU: page-locked buffers are interleaved over the NUMA nodes */
     int format;                    /* UTB_INPUT_FASTA, _FASTQ (4-line) or _FASTA_WRAPPED (utb_searcher_set_input) */
     uint32_t min_qual;             /* FASTQ: bases with a quality byte below 33 + min_qual count as 'N' (0: off) */
+    /* sample profile (utb_searcher_set_profile): the batches' (label << 32 | printed length, reads) pairs merged in an
+     * open-addressing map, then the canonical rows of the last search */
+    int profile;
+    size_t pf_keys;                /* most distinct keys a batch can have: sum over the labels of strlen + 1 */
+    uint64_t *pm_key, *pm_cnt; size_t pm_cap, pm_n;
+    utb_profile_row *rows; size_t n_rows, rows_cap; uint64_t unclassified;
+    int profile_valid;             /* the last search returned UTB_OK or UTB_ERR_FORMAT with the profile on */
 };
 
 static double now_s(void) {
@@ -178,6 +185,7 @@ static int slots_create(utb_searcher *s) {
         if (!rc) rc = utb_batch_prepare(nb[i], UTB_OUT_TEXT, s->device_frame);
         if (!rc && s->shallow) rc = utb_batch_prepare(nb[i], UTB_OUT_SELECTIONS, s->device_frame);
         if (!rc && s->format != UTB_INPUT_FASTA) rc = utb_batch_set_input(nb[i], s->format, s->min_qual, s->device_frame);
+        if (!rc && s->profile) rc = utb_batch_set_profile(nb[i], 1, s->pf_keys);
         if (s->spread) mem_interleave(0);
     }
     for (int i = 0; i < s->n_slots; ++i) {
@@ -244,6 +252,7 @@ int utb_searcher_create(const utb_ctr *ctr, const int *devices, int n_devices,
  * selects; the order-dependent vote and the "%f" column are done by the formatter thread, read by read. */
 int utb_searcher_set_shallow(utb_searcher *s, int on) {
     if (!s) { utb_set_error("utb_searcher_set_shallow: null searcher"); return UTB_ERR_ARG; }
+    if (on && s->profile) { utb_set_error("utb_searcher_set_shallow: the profile is not available for the non-GG search"); return UTB_ERR_ARG; }
     s->shallow = on ? 1 : 0;
     if (!on) return UTB_OK;
     if (!s->tally) s->tally = (uint32_t *)calloc(s->ctr->max_ix ? s->ctr->max_ix : 1, sizeof(uint32_t));
@@ -285,8 +294,100 @@ int utb_searcher_set_input(utb_searcher *s, int format, uint32_t min_qual) {
     return UTB_OK;
 }
 
+#define PM_EMPTY UINT64_MAX                                      /* no key: label < max_ix < 2^32 - 1 */
+static int pm_alloc(utb_searcher *s, size_t cap) {
+    uint64_t *k = (uint64_t *)malloc(cap * sizeof(uint64_t)), *c = (uint64_t *)malloc(cap * sizeof(uint64_t));
+    if (!k || !c) { free(k); free(c); utb_set_error("out of memory (profile)"); return UTB_ERR_NOMEM; }
+    memset(k, 0xFF, cap * sizeof(uint64_t));
+    free(s->pm_key); free(s->pm_cnt);
+    s->pm_key = k; s->pm_cnt = c; s->pm_cap = cap; s->pm_n = 0;
+    return UTB_OK;
+}
+static inline size_t pm_home(uint64_t key, size_t cap) { return (size_t)((key * 0x9E3779B97F4A7C15ull) >> 32) & (cap - 1); }
+/* adds c reads to key; the map doubles when half full */
+static int pm_add(utb_searcher *s, uint64_t key, uint64_t c) {
+    if (2 * (s->pm_n + 1) > s->pm_cap) {
+        uint64_t *ok = s->pm_key, *oc = s->pm_cnt;
+        const size_t ocap = s->pm_cap;
+        s->pm_key = s->pm_cnt = NULL;
+        if (pm_alloc(s, 2 * ocap)) { s->pm_key = ok; s->pm_cnt = oc; s->pm_cap = ocap; return UTB_ERR_NOMEM; }
+        for (size_t i = 0; i < ocap; ++i) if (ok[i] != PM_EMPTY) {
+            size_t h = pm_home(ok[i], s->pm_cap);
+            while (s->pm_key[h] != PM_EMPTY) h = (h + 1) & (s->pm_cap - 1);
+            s->pm_key[h] = ok[i]; s->pm_cnt[h] = oc[i]; ++s->pm_n;
+        }
+        free(ok); free(oc);
+    }
+    size_t h = pm_home(key, s->pm_cap);
+    while (s->pm_key[h] != PM_EMPTY && s->pm_key[h] != key) h = (h + 1) & (s->pm_cap - 1);
+    if (s->pm_key[h] == PM_EMPTY) { s->pm_key[h] = key; s->pm_cnt[h] = 0; ++s->pm_n; }
+    s->pm_cnt[h] += c;
+    return UTB_OK;
+}
+
+int utb_searcher_set_profile(utb_searcher *s, int on) {
+    if (!s) { utb_set_error("utb_searcher_set_profile: null searcher"); return UTB_ERR_ARG; }
+    s->profile_valid = 0;
+    if (!on) { s->profile = 0; return UTB_OK; }
+    if (s->shallow) { utb_set_error("utb_searcher_set_profile: the profile is not available for the non-GG search"); return UTB_ERR_ARG; }
+    size_t keys = 0;
+    for (uint32_t i = 0; i < s->ctr->max_ix; ++i) keys += strlen(s->ctr->blob + s->ctr->off[i]) + 1;
+    if (!keys) keys = 1;
+    s->pf_keys = keys;
+    if (!s->pm_key) { int rc = pm_alloc(s, 1024); if (rc) return rc; }
+    for (int i = 0; i < s->n_slots; ++i) {
+        int rc = utb_batch_set_profile(s->slots[i].b, 1, keys);
+        if (rc) { for (int j = 0; j < i; ++j) (void)utb_batch_set_profile(s->slots[j].b, 0, keys); return rc; }
+    }
+    s->profile = 1;
+    return UTB_OK;
+}
+
+/* rows in byte order of the printed strings, a prefix first; equal strings tie on the label id */
+static int row_cmp(const void *a_, const void *b_, void *c_) {
+    const utb_profile_row *a = (const utb_profile_row *)a_, *b = (const utb_profile_row *)b_;
+    const utb_ctr *c = (const utb_ctr *)c_;
+    const int d = memcmp(c->blob + c->off[a->label], c->blob + c->off[b->label], a->len < b->len ? a->len : b->len);
+    if (d) return d;
+    if (a->len != b->len) return a->len < b->len ? -1 : 1;
+    return a->label < b->label ? -1 : a->label > b->label;
+}
+/* the map -> the canonical rows: sorted by their strings, equal strings merged under the smallest label id */
+static int profile_rows(utb_searcher *s, uint64_t reads, uint64_t good) {
+    if (s->pm_n > s->rows_cap) {
+        utb_profile_row *r = (utb_profile_row *)malloc(s->pm_n * sizeof *r);
+        if (!r) { utb_set_error("out of memory (profile)"); return UTB_ERR_NOMEM; }
+        free(s->rows);
+        s->rows = r; s->rows_cap = s->pm_n;
+    }
+    size_t n = 0;
+    for (size_t i = 0; i < s->pm_cap; ++i) if (s->pm_key[i] != PM_EMPTY) {
+        utb_profile_row *r = &s->rows[n++];
+        r->label = (uint32_t)(s->pm_key[i] >> 32); r->len = (uint32_t)s->pm_key[i]; r->reads = s->pm_cnt[i];
+    }
+    qsort_r(s->rows, n, sizeof *s->rows, row_cmp, (void *)s->ctr);
+    size_t m = 0;
+    for (size_t i = 0; i < n; ++i) {
+        if (m && s->rows[m - 1].len == s->rows[i].len &&
+            !memcmp(s->ctr->blob + s->ctr->off[s->rows[m - 1].label], s->ctr->blob + s->ctr->off[s->rows[i].label], s->rows[i].len))
+            s->rows[m - 1].reads += s->rows[i].reads;
+        else s->rows[m++] = s->rows[i];
+    }
+    s->n_rows = m;
+    s->unclassified = reads - good;
+    return UTB_OK;
+}
+
+int utb_searcher_profile(const utb_searcher *s, const utb_profile_row **rows, size_t *n_rows, uint64_t *unclassified) {
+    if (!s || !rows || !n_rows || !unclassified) { utb_set_error("utb_searcher_profile: null argument"); return UTB_ERR_ARG; }
+    if (!s->profile_valid) { utb_set_error("utb_searcher_profile: no profile (the profile is off, or the last search failed)"); return UTB_ERR_ARG; }
+    *rows = s->rows; *n_rows = s->n_rows; *unclassified = s->unclassified;
+    return UTB_OK;
+}
+
 void utb_searcher_destroy(utb_searcher *s) {
     if (!s) return;
+    free(s->pm_key); free(s->pm_cnt); free(s->rows);
     if (s->slots) for (int i = 0; i < s->n_slots; ++i) utb_batch_destroy(s->slots[i].b);
     if (s->dbs) for (int d = 0; d < s->n_devices; ++d) {
         int shared = 0;
@@ -358,6 +459,7 @@ typedef struct {
      * lock (~2.7 GB/s whatever the thread count), page faults of a mapping do not.  Otherwise parallel pwrite. */
     int stream, mapped;
     char *map; size_t map_lo, map_hi, file_len;
+    int none;               /* no output text (profile only): the devices build no lines */
 } sink_t;
 #define SINK_WINDOW ((size_t)256 << 20)
 
@@ -620,6 +722,13 @@ static void *formatter_main(void *arg) {
             R->st.good_finds += good;
             R->st.fm_emit += now_s() - tf;
             R->st.d2h_bytes += text_len + 4 * 1024 * 8 + 16;
+            if (s->profile) {                                      /* the only place the profile is counted: batches dropped above never are */
+                const uint64_t *pairs = NULL; size_t n_pairs = 0;
+                int r2 = utb_batch_profile(sl->b, &pairs, &n_pairs);
+                for (size_t i = 0; i < n_pairs && !r2; ++i) r2 = pm_add(s, pairs[2 * i], pairs[2 * i + 1]);
+                if (r2 && !R->error) { R->error = r2; snprintf(R->errmsg, sizeof R->errmsg, "%s", utb_last_error()); }
+                R->st.d2h_bytes += 4 + 16 * n_pairs;
+            }
         }
         if (!rc) {
             uint64_t lk = 0, ht = 0; float ms[4] = {0, 0, 0, 0};
@@ -1224,6 +1333,12 @@ static int run_search(utb_searcher *s, source_t *src, sink_t *sink, int do_rc, u
     uint64_t launches0 = 0;
     for (int i = 0; i < s->n_slots; ++i) { s->slots[i].state = 0; launches0 += utb_batch_launches(s->slots[i].b); }
     if (s->shallow && s->horses) memset(s->horses, 0, s->horses_cap * sizeof(uint32_t));   /* every search starts like a fresh process */
+    if (s->profile) {                                              /* an empty profile */
+        memset(s->pm_key, 0xFF, s->pm_cap * sizeof(uint64_t));
+        s->pm_n = 0;
+    }
+    for (int i = 0; i < s->n_slots; ++i)                          /* no text when there is nowhere to put it */
+        (void)utb_batch_set_profile(s->slots[i].b, !s->profile ? 0 : sink->none ? 2 : 1, s->pf_keys);
     /* split the host threads between the two teams */
     /* with the lines built on the device the formatter only moves finished text: most threads frame */
     int T = s->host_threads, n_fm = T >= 4 ? T / 2 : 1, n_rd = T >= 4 ? T - n_fm : 1;
@@ -1468,6 +1583,10 @@ read_loop:
     }
     R.st.rd_wait_slot = rd_t[0]; R.st.rd_fill = rd_t[1]; R.st.rd_frame = rd_t[2]; R.st.rd_submit = rd_t[3];
     if (stats) *stats = R.st;
+    if (s->profile && !rc) {
+        rc = profile_rows(s, R.st.reads, R.st.good_finds);
+        s->profile_valid = !rc;
+    }
     if (!rc && fmt_err) {
         utb_set_error("%s", fmt_msg);
         if (ref_exit) *ref_exit = 2;                               /* itree.c:872-888 */
@@ -1478,38 +1597,61 @@ read_loop:
 
 int utb_search_file(utb_searcher *s, const char *fasta_path, const char *out_path,
                     int do_rc, utb_stats *stats, int *ref_exit) {
-    if (!s || !fasta_path || !out_path) { utb_set_error("utb_search_file: null argument"); return UTB_ERR_ARG; }
+    if (s) s->profile_valid = 0;
+    if (!s || !fasta_path || (!out_path && !s->profile)) { utb_set_error("utb_search_file: null argument"); return UTB_ERR_ARG; }
     if (ref_exit) *ref_exit = 0;
     int fd = open(fasta_path, O_RDONLY);
     if (fd < 0) { utb_set_error("Invalid input files"); if (ref_exit) *ref_exit = 1; return UTB_ERR_IO; }   /* itree.c:835 */
-    int fo = open(out_path, O_RDWR | O_CREAT | O_TRUNC, 0644);   /* read access only for the shared mapping of sink_reserve */
-    if (fo < 0) fo = open(out_path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
-    if (fo < 0) { close(fd); utb_set_error("cannot open output file %s", out_path); if (ref_exit) *ref_exit = 1; return UTB_ERR_IO; }
+    int fo = -1;
+    if (out_path) {
+        fo = open(out_path, O_RDWR | O_CREAT | O_TRUNC, 0644);     /* read access only for the shared mapping of sink_reserve */
+        if (fo < 0) fo = open(out_path, O_WRONLY | O_CREAT | O_TRUNC, 0644);
+        if (fo < 0) { close(fd); utb_set_error("cannot open output file %s", out_path); if (ref_exit) *ref_exit = 1; return UTB_ERR_IO; }
+    }
     source_t src; memset(&src, 0, sizeof src); src.fd = fd;
     struct stat st;
     if (!fstat(fd, &st) && S_ISREG(st.st_mode)) { src.seekable = 1; src.file_size = st.st_size; if (!st.st_size) src.eof = 1; }
-    sink_t sink; memset(&sink, 0, sizeof sink); sink.fd = fo; sink.s = s;
-    sink_open_file(&sink);
+    sink_t sink; memset(&sink, 0, sizeof sink); sink.fd = fo; sink.s = s; sink.none = !out_path;
+    if (out_path) sink_open_file(&sink);
     int rc = run_search(s, &src, &sink, do_rc, stats, ref_exit);
-    int bad = sink_close_file(&sink);
-    if ((close(fo) || bad) && !rc) { rc = UTB_ERR_IO; utb_set_error("write error on output"); }
+    if (out_path) {
+        int bad = sink_close_file(&sink);
+        if ((close(fo) || bad) && !rc) { rc = UTB_ERR_IO; utb_set_error("write error on output"); }
+    }
     close(fd);
     return rc;
 }
 
 int utb_search_mem(utb_searcher *s, const char *fasta, size_t n, int do_rc,
                    char **out, size_t *out_len, utb_stats *stats, int *ref_exit) {
-    if (!s || (!fasta && n) || !out || !out_len) { utb_set_error("utb_search_mem: null argument"); return UTB_ERR_ARG; }
+    if (s) s->profile_valid = 0;
+    const int none = s && s->profile && !out && !out_len;          /* the profile alone */
+    if (!s || (!fasta && n) || ((!out || !out_len) && !none)) { utb_set_error("utb_search_mem: null argument"); return UTB_ERR_ARG; }
     source_t src; memset(&src, 0, sizeof src); src.fd = -1; src.mem = fasta; src.mem_len = n; src.eof = n == 0;
-    sink_t sink; memset(&sink, 0, sizeof sink); sink.fd = -1; sink.s = s;
+    sink_t sink; memset(&sink, 0, sizeof sink); sink.fd = -1; sink.s = s; sink.none = none;
     sink.hint = n / 2 + n / 4 + ((size_t)1 << 20);                 /* typical output: about half the FASTA */
     int rc = run_search(s, &src, &sink, do_rc, stats, ref_exit);
-    *out = sink.off ? s->arena : NULL; *out_len = sink.off;
+    if (!none) { *out = sink.off ? s->arena : NULL; *out_len = sink.off; }
     return rc;
 }
 
 /* ---- CLI (itree.c:1357-1377; stdout lines of SURVEY App. C) -------------------------------------- */
 static const char *TYPEARR[9] = {"NA", "uint8_t", "uint16_t", "NA", "uint32_t", "NA", "NA", "NA", "uint64_t"};
+
+/* The CLIs' searcher over the GPUs in UTB_DEVICES (e.g. "0,1,2,3"; default: all visible); *n: how many. */
+static int cli_searcher(const utb_ctr *ctr, int threads, utb_searcher **s, int *n) {
+    int ndev = 0, devs[64];
+    int rc = utb_device_count(&ndev);
+    if (rc) return rc;
+    *n = 0;
+    const char *e = getenv("UTB_DEVICES");
+    if (e && *e) {
+        char *dup = strdup(e), *save = NULL;
+        for (char *t = strtok_r(dup, ",", &save); t && *n < 64; t = strtok_r(NULL, ",", &save)) devs[(*n)++] = atoi(t);
+        free(dup);
+    } else for (; *n < ndev && *n < 64; ++*n) devs[*n] = *n;
+    return utb_searcher_create(ctr, devs, *n, threads, s);
+}
 
 static int main_impl(int argc, char **argv, int gg);
 int utb_main(int argc, char **argv) { return main_impl(argc, argv, 1); }
@@ -1555,18 +1697,9 @@ static int main_impl(int argc, char **argv, int gg) {
     if (ctr->last_bin != ctr->num_nodes)                           /* itree.c:792-793 */
         printf("Warning: detected nodes %u != %u\n", (unsigned)ctr->last_bin, (unsigned)ctr->num_nodes);
 
-    int ndev = 0, devs[64];
-    rc = utb_device_count(&ndev);
-    if (rc) { fprintf(stderr, "utree-b200: %s\n", utb_last_error()); utb_ctr_close(ctr); return 4; }
     int n = 0;
-    const char *e = getenv("UTB_DEVICES");                         /* e.g. "0,1,2,3"; default: all visible */
-    if (e && *e) {
-        char *dup = strdup(e), *save = NULL;
-        for (char *t = strtok_r(dup, ",", &save); t && n < 64; t = strtok_r(NULL, ",", &save)) devs[n++] = atoi(t);
-        free(dup);
-    } else for (; n < ndev && n < 64; ++n) devs[n] = n;
     utb_searcher *s = NULL;
-    rc = utb_searcher_create(ctr, devs, n, threads, &s);
+    rc = cli_searcher(ctr, threads, &s, &n);
     if (rc) { fprintf(stderr, "utree-b200: %s\n", utb_last_error()); utb_ctr_close(ctr); return rc == UTB_ERR_NOMEM ? 3 : 4; }
     if (!gg) rc = utb_searcher_set_shallow(s, 1);
     if (rc) { fprintf(stderr, "utree-b200: %s\n", utb_last_error()); utb_searcher_destroy(s); utb_ctr_close(ctr); return rc == UTB_ERR_NOMEM ? 3 : 4; }
@@ -1593,4 +1726,109 @@ static int main_impl(int argc, char **argv, int gg) {
     utb_searcher_destroy(s);
     utb_ctr_close(ctr);
     return 0;
+}
+
+/* ---- utree-profile: per-sample read counts per taxonomy string, as one TSV table ---------------------------------- */
+typedef struct { const char *str; uint32_t len; int sample; uint64_t reads; } pf_cell;
+static int pf_cell_cmp(const void *a_, const void *b_) {
+    const pf_cell *a = (const pf_cell *)a_, *b = (const pf_cell *)b_;
+    const int d = memcmp(a->str, b->str, a->len < b->len ? a->len : b->len);
+    if (d) return d;
+    if (a->len != b->len) return a->len < b->len ? -1 : 1;
+    return (a->sample > b->sample) - (a->sample < b->sample);
+}
+static int pf_usage(void) {
+    fprintf(stderr, "usage: utree-profile [-r] [-t threads] [-f fasta|fastq|wrapped] [-q min_qual] compTree.ctr table.tsv reads1 [reads2 ...]\n");
+    return 1;
+}
+static int pf_exit(int rc) { return rc == UTB_ERR_NOMEM ? 3 : 4; }
+
+int utb_profile_main(int argc, char **argv) {
+    int do_rc = 0, format = UTB_INPUT_FASTA, i = 1;
+    long ncpu = sysconf(_SC_NPROCESSORS_ONLN), threads = ncpu > 0 ? ncpu : 1, q = 0;
+    for (; i < argc && argv[i][0] == '-' && argv[i][1]; ++i) {
+        const char *a = argv[i];
+        if (!strcmp(a, "-r")) { do_rc = 1; continue; }
+        if (strlen(a) != 2 || !strchr("tfq", a[1]) || i + 1 >= argc) return pf_usage();
+        const char *v = argv[++i];
+        char *end = NULL;
+        if (a[1] == 't') { threads = strtol(v, &end, 10); if (!*v || *end || threads < 1 || threads > 4096) return pf_usage(); }
+        else if (a[1] == 'q') { q = strtol(v, &end, 10); if (!*v || *end || q < 0 || q > 222) return pf_usage(); }
+        else if (!strcmp(v, "fasta")) format = UTB_INPUT_FASTA;
+        else if (!strcmp(v, "fastq")) format = UTB_INPUT_FASTQ;
+        else if (!strcmp(v, "wrapped")) format = UTB_INPUT_FASTA_WRAPPED;
+        else return pf_usage();
+    }
+    if (argc - i < 3 || (q && format != UTB_INPUT_FASTQ)) return pf_usage();
+    const char *ctr_path = argv[i], *table = argv[i + 1];
+    char **samples = argv + i + 2;
+    const int n_samples = argc - i - 2;
+
+    utb_ctr *ctr = NULL;
+    int rc = utb_ctr_open(ctr_path, &ctr);
+    if (rc) {
+        fprintf(stderr, "utree-profile: %s: %s\n", ctr_path, utb_last_error());
+        return rc == UTB_ERR_NOMEM || (rc == UTB_ERR_FORMAT && !strcmp(utb_last_error(), "Error in reading tree.")) ? 3 : 1;
+    }
+    for (int k = 0; k < n_samples; ++k) {                          /* before any GPU work */
+        int fd = open(samples[k], O_RDONLY);
+        if (fd < 0) { fprintf(stderr, "utree-profile: cannot read %s: %s\n", samples[k], strerror(errno)); utb_ctr_close(ctr); return 1; }
+        close(fd);
+    }
+    int n_dev = 0, code = 0;
+    utb_searcher *s = NULL;
+    pf_cell *cells = NULL; size_t n_cells = 0, cap = 0;
+    uint64_t *uncl = (uint64_t *)calloc((size_t)n_samples, sizeof(uint64_t));
+    rc = uncl ? cli_searcher(ctr, (int)threads, &s, &n_dev) : UTB_ERR_NOMEM;
+    if (!rc) rc = utb_searcher_set_input(s, format, (uint32_t)q);
+    if (!rc) rc = utb_searcher_set_profile(s, 1);
+    if (rc) { fprintf(stderr, "utree-profile: %s\n", rc == UTB_ERR_NOMEM && !uncl ? "out of memory" : utb_last_error()); code = pf_exit(rc); goto done; }
+    for (int k = 0; k < n_samples; ++k) {
+        utb_stats st; int ref_exit = 0;
+        rc = utb_search_file(s, samples[k], NULL, do_rc, &st, &ref_exit);
+        if (rc == UTB_ERR_IO && ref_exit == 1) { fprintf(stderr, "utree-profile: cannot read %s\n", samples[k]); code = 1; goto done; }
+        if (rc == UTB_ERR_FORMAT) { fprintf(stderr, "utree-profile: %s: %s\n", samples[k], utb_last_error()); code = 2; goto done; }
+        if (rc) { fprintf(stderr, "utree-profile: %s: %s\n", samples[k], utb_last_error()); code = pf_exit(rc); goto done; }
+        printf("Searched %llu queries\n", (unsigned long long)st.reads);
+        printf("Good finds: %llu\n", (unsigned long long)st.good_finds);
+        fflush(stdout);
+        const utb_profile_row *rows; size_t n_rows;
+        utb_searcher_profile(s, &rows, &n_rows, &uncl[k]);
+        if (n_cells + n_rows > cap) {
+            size_t nc = 2 * cap + n_rows;
+            pf_cell *c = (pf_cell *)realloc(cells, nc * sizeof *c);
+            if (!c) { fprintf(stderr, "utree-profile: out of memory\n"); code = 3; goto done; }
+            cells = c; cap = nc;
+        }
+        for (size_t r = 0; r < n_rows; ++r) {
+            pf_cell *c = &cells[n_cells++];
+            c->str = ctr->blob + ctr->off[rows[r].label]; c->len = rows[r].len; c->sample = k; c->reads = rows[r].reads;
+        }
+    }
+    qsort(cells, n_cells, sizeof *cells, pf_cell_cmp);
+    FILE *f = fopen(table, "w");
+    if (!f) { fprintf(stderr, "utree-profile: cannot write %s: %s\n", table, strerror(errno)); code = 1; goto done; }
+    fputs("#taxonomy", f);
+    for (int k = 0; k < n_samples; ++k) fprintf(f, "\t%s", samples[k]);
+    fputs("\n#unclassified", f);
+    for (int k = 0; k < n_samples; ++k) fprintf(f, "\t%llu", (unsigned long long)uncl[k]);
+    fputc('\n', f);
+    for (size_t a = 0; a < n_cells;) {                             /* one line per string: its cells are adjacent, by sample */
+        size_t b = a;
+        fwrite(cells[a].str, 1, cells[a].len, f);
+        for (int k = 0; k < n_samples; ++k) {
+            uint64_t v = 0;
+            if (b < n_cells && cells[b].sample == k && cells[b].len == cells[a].len && !memcmp(cells[b].str, cells[a].str, cells[a].len))
+                v = cells[b++].reads;
+            fprintf(f, "\t%llu", (unsigned long long)v);
+        }
+        fputc('\n', f);
+        a = b;
+    }
+    if (fclose(f)) { fprintf(stderr, "utree-profile: cannot write %s\n", table); code = 1; }
+done:
+    free(cells); free(uncl);
+    utb_searcher_destroy(s);
+    utb_ctr_close(ctr);
+    return code;
 }

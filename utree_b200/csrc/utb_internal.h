@@ -59,6 +59,11 @@ int utb_batch_text_piece(utb_batch *b, size_t off, size_t *len, const char **pie
 int utb_batch_wait_shallow(utb_batch *b, const uint32_t **sel_cnt, const uint32_t **sel, size_t *sel_total,
                            const uint32_t **name_off, const uint32_t **name_len);
 int utb_batch_sync(utb_batch *b);
+/* Sample profile of the later submits of a text batch: mode 0 off, 1 with the text, 2 instead of it (the format
+ * kernels do not run).  The first mode != 0 allocates a key table for max_keys distinct keys per batch. */
+int utb_batch_set_profile(utb_batch *b, int mode, size_t max_keys);
+/* After utb_batch_wait_len: the batch's (key = label << 32 | printed length, reads) pairs, *n of them. */
+int utb_batch_profile(utb_batch *b, const uint64_t **pairs, size_t *n);
 /* The most reads per batch, at most max_reads, for which the worst-case output text of a batch of max_bytes raw
  * bytes (every read printing its name and the longest label, max_label bytes with the NUL) fits the 32-bit offsets
  * of the format kernels; 0 if none does. */
